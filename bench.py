@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched by torchrun, one rank per GPU)
   python bench.py --impl reference --gpus N --steps K --warmup W
+  python bench.py ... --dump-outputs DIR                   (what the last timed step computed, as DIR/*.npy)
 
 Workload (config.workload): synthetic 3.1 Gbp human-scale genome (24 chromosomes + 170 scaffolds,
 5 % N, 50 % soft-masked) resident on the GPU as two strand planes of 0.5 B/base each, and a GTF-shaped annotation of 200k
@@ -586,6 +587,29 @@ class Workload(object):
 
 STEP_MODE = os.environ.get("MAGOT_STEP", "streams3")     # streams3 | fused | multi  (see Workload.step)
 STEP_DEFER = os.environ.get("MAGOT_STEP_DEFER", "1") != "0" and STEP_MODE == "streams3"   # record pass of K1 off the critical path
+DUMP_SAMPLE = 4 << 20      # bytes kept per text over all ranks: 3 texts x 4 Mi x 4 B (float32) = 48 MiB in all
+
+
+def dump_outputs(wl, out_dir, rank, world):
+    """The three texts the last timed step left in HBM, as .npy files in out_dir, so that two builds can be compared output
+    for output.  Each rank writes lengths<sfx>.npy (float64: bytes of its CDS nucleotide, CDS protein and exon transcript
+    texts) and one float32 file per text with its bytes -- all of them when the text has at most DUMP_SAMPLE // world bytes,
+    else the bytes at that many positions drawn with a fixed seed (ascending, repeats possible).  <sfx> is empty on one GPU
+    and _rank<r> otherwise; the ranks split DUMP_SAMPLE, so a dump stays within 48 MiB whatever the number of GPUs."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = "_rank%d" % rank if world > 1 else ""
+    cap = DUMP_SAMPLE // world
+    texts = (("cds_nuc", "cds_n", wl.sizes["cds"][0]), ("cds_prot", "cds_p", wl.sizes["cds"][1]),
+             ("exon_nuc", "exon_n", wl.sizes["exon"][0]))
+    np.save(os.path.join(out_dir, "lengths%s.npy" % suffix), np.array([n for _, _, n in texts], dtype=np.float64))
+    for name, key, n in texts:
+        text = wl.out[key][:n]
+        if n > cap:
+            pos = np.sort(np.random.default_rng(SEED).integers(0, n, size=cap))
+            text = text[torch.from_numpy(pos).to(text.device)]
+        np.save(os.path.join(out_dir, "%s%s.npy" % (name, suffix)), text.cpu().numpy().astype(np.float32))
 
 
 def profile_traffic():
@@ -690,6 +714,8 @@ def gpu_arm(args):
     clocks.start()
     dev_ms, launches = timed_loop(wl, args.warmup, args.steps)
     wl.check_totals()
+    if args.dump_outputs:
+        dump_outputs(wl, args.dump_outputs, rank, world)
     kt = wl.kernel_times(max(3, min(args.steps, 10)))
     ft = wl.fused_times(max(3, min(args.steps, 10))) if world == 1 else None
 
@@ -1063,7 +1089,12 @@ def main():
     ap.add_argument("--impl", default="magot_b200", choices=["magot_b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sixframe", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the texts of the last timed step to DIR/*.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path only")
     if args.impl == "reference":
         reference_arm(args)
     else:

@@ -10,6 +10,8 @@ Writes
                        so the GPU box -- which has no /root/reference -- can run the same cases
   manifest.json        POSIX cksum + byte count of the reference's stdout for every whole-file
                        case (plus the three cksums hard-coded in test_data/test_suite.py)
+  obiroi_gff2fasta_protein.fa.gz
+                       the whole stdout of gff2fasta seq_type=protein on the O.biroi pair, gzipped
   kat.json             known-answer vectors for Sequence.reverse_compliment / translate /
                        get_orfs / BaseAnnotation.get_seq clamping produced by the reference
 """
@@ -62,7 +64,10 @@ def whole_file_cases(tmp):
 
     # --- BASELINE config 1: O.biroi FASTA + GFF3
     put("obiroi:gff2fasta", ref_runner.gff2fasta(ob_fa, ob_gff))
-    put("obiroi:gff2fasta_protein", ref_runner.gff2fasta(ob_fa, ob_gff, seq_type="protein"))
+    prot = ref_runner.gff2fasta(ob_fa, ob_gff, seq_type="protein")
+    put("obiroi:gff2fasta_protein", prot)
+    with open(os.path.join(HERE, "obiroi_gff2fasta_protein.fa.gz"), "wb") as fh:
+        fh.write(gzip.compress(prot.encode("latin-1"), 9, mtime=0))
     put("obiroi:gff2fasta_from_exons", ref_runner.gff2fasta(ob_fa, ob_gff, from_exons="True"))
     my = ref_runner.load_genome(ob_fa, ob_gff, base_features=['exon', 'match_part', 'similarity', 'region'],
                                 features_to_ignore=['CDS'])
