@@ -135,6 +135,11 @@ int mg_plan_totals(mg_plan *p, int64_t *nuc_total, int64_t *prot_total, void *st
  * nuc_len[r] = spliced bases; aa_len[r] = amino acids, or -1 where the reference's translate
  * returns None (spliced length <= 2, genome.py:810).  Either pointer may be NULL.           */
 int mg_plan_lengths(mg_plan *p, int64_t *nuc_len, int64_t *aa_len, void *stream);
+/* Genetic code of the plan's protein text (K3, K23, mg_emit_products_*, every _host variant): codon64[16*b0 + 4*b1 + b2]
+ * (A=0 C=1 G=2 T=3) is the residue of codon b0 b1 b2, '*' a stop; no entry may be 'X' (a codon with a base outside ACGT is 'X'
+ * whatever the code, which is what trimX tests).  The table is uploaded by this call, so emits captured in a CUDA graph
+ * afterwards stay valid.  codon64 == NULL restores the genome's standard code (NCBI table 1).                                 */
+int mg_plan_set_codon_table(mg_plan *p, const uint8_t *codon64);
 
 /* ---- K2: spliced nucleotides (+ per-segment reverse complement, + literal framing) ---------
  * replaces ParentAnnotation.get_fasta seq_type="nucleotide" (genome.py:687-710) and
@@ -204,6 +209,15 @@ int mg_sixframe_count(mg_genome *g, int64_t contig_lo, int64_t contig_hi, int64_
  * contig in list order.                                                                        */
 int mg_sixframe_count_list(mg_genome *g, int64_t n_list, const int64_t *contig_ids, int64_t min_aa,
                            int64_t *n_orf, int64_t *n_bytes, void *stream);
+/* The same two scans under another genetic code: codon64 as in mg_plan_set_codon_table.  A codon is a stop iff the table maps it
+ * to '*' (any number of stop codons, 0..64); the following mg_sixframe_emit* writes residues from this table.  codon64 == NULL
+ * is exactly mg_sixframe_count / mg_sixframe_count_list.  With the stop-codon index (mg_tune "six" = 2), a code whose stops
+ * differ from TAA/TAG/TGA builds a second index (0.25 B/base, counted in mg_genome_bytes) next to the standard one; one such
+ * index is kept, and pack / finalize / mask drop both.                                                                      */
+int mg_sixframe_count_table(mg_genome *g, int64_t contig_lo, int64_t contig_hi, int64_t min_aa, const uint8_t *codon64,
+                            int64_t *n_orf, int64_t *n_bytes, void *stream);
+int mg_sixframe_count_list_table(mg_genome *g, int64_t n_list, const int64_t *contig_ids, int64_t min_aa, const uint8_t *codon64,
+                                 int64_t *n_orf, int64_t *n_bytes, void *stream);
 /* Emits the result of the preceding mg_sixframe_count on this genome handle.  aa_out_host gets
  * n_bytes residues (ORFs back to back, no separators), recs_host n_orf records.  Either may
  * be NULL.  *_device variant leaves the residues in `aa_out_dev` (16-byte aligned, n_bytes

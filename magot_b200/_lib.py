@@ -63,6 +63,7 @@ SIGNATURES = {
     "mg_plan_prepare_prot_async": (_i32, [_vp, _vp]),
     "mg_plan_totals": (_i32, [_vp, _pi64, _pi64, _vp]),
     "mg_plan_lengths": (_i32, [_vp, _vp, _vp, _vp]),
+    "mg_plan_set_codon_table": (_i32, [_vp, _vp]),
     "mg_emit_nuc_device": (_i32, [_vp, _vp, _vp]),
     "mg_emit_prot_device": (_i32, [_vp, _vp, _vp]),
     "mg_emit_nuc_prot_device": (_i32, [_vp, _vp, _vp, _vp]),
@@ -76,6 +77,8 @@ SIGNATURES = {
     "mg_translate_ascii_table": (_i32, [_i32, _vp, _vp, _vp, _i64, _i32, _i32, _i32, _vp, _i64, _vp, _vp, _vp]),
     "mg_sixframe_count": (_i32, [_vp, _i64, _i64, _i64, _pi64, _pi64, _vp]),
     "mg_sixframe_count_list": (_i32, [_vp, _i64, _vp, _i64, _pi64, _pi64, _vp]),
+    "mg_sixframe_count_table": (_i32, [_vp, _i64, _i64, _i64, _vp, _pi64, _pi64, _vp]),
+    "mg_sixframe_count_list_table": (_i32, [_vp, _i64, _vp, _i64, _vp, _pi64, _pi64, _vp]),
     "mg_sixframe_emit": (_i32, [_vp, _vp, _vp, _vp]),
     "mg_sixframe_emit_device": (_i32, [_vp, _vp, _vp, _vp]),
     "mg_stream_sync": (_i32, [_i32, _vp]),

@@ -92,6 +92,9 @@ struct mg_genome {
     uint32_t *d_stops = nullptr;              // stop-codon index (K4): one bit per base and strand, [0, stop_words) plus, [stop_words, 2 stop_words) minus
     int64_t stop_words = 0;
     bool stops_valid = false;                 // false after pack / mask: rebuilt by the next ORF scan
+    uint32_t *d_stops_alt = nullptr;          // the same for ONE other stop set (a non-standard genetic code), same layout
+    uint64_t stops_alt_key = 0;               // its stop codons: bit 16*b0 + 4*b1 + b2 (A=0 C=1 G=2 T=3)
+    bool stops_alt_valid = false;             // false after pack / mask, like stops_valid
     mg_sixframe_state *six = nullptr;
     int64_t device_bytes = 0;
 };
@@ -142,6 +145,8 @@ struct mg_plan {
     int64_t order_cap = 0;
     uint8_t *d_out = nullptr;                 // library-owned output buffer for *_host emits
     int64_t out_cap = 0;
+    uint8_t *d_aa8192 = nullptr;              // the plan's own translation tables (mg_plan_set_codon_table): plain | mg_aa_slot order
+    bool own_code = false;                    // true: K3 / K23 / the one-launch emit read d_aa8192 instead of the genome's tables
     std::vector<void *> owned;                // everything to free
 };
 
@@ -159,6 +164,7 @@ struct mg_plan {
 #endif
 
 // internal cross-file helpers
+void build_aa4096(uint8_t *t, const uint8_t *codon64);   // nibble-triplet -> residue table from a codon64 table (NULL = standard code)
 int mg_scan_i32(const int32_t *d_in, int64_t *d_out, int64_t n, int64_t *d_tmp, int64_t tmp_cap, cudaStream_t st);
 int64_t mg_scan_tmp_elems(int64_t n);
 int mg_ensure_stage(mg_genome *g, int64_t bytes);

@@ -814,7 +814,9 @@ static ProtArgs prot_args(const mg_plan *p, uint8_t *out_dev) {
     a.packed = g->d_packed; a.piece_off = p->d_piece_off; a.piece_src = p->d_piece_src; a.rec_seg_off = p->d_rec_seg_off;
     a.prot_off = p->d_prot_off; a.rec_aa = p->d_rec_aa; a.rec_skip = p->d_rec_skip; a.rec_pre = p->d_rec_pre; a.rec_suf = p->d_rec_suf;
     a.rec_lit_off = p->d_rec_lit_off; a.lit = p->n_lit > 0 ? p->d_lit : nullptr; a.n_rec = p->n_rec; a.tile_first = p->d_prot_tile;
-    a.total_dev = p->d_totals + 1; a.cap = p->prot_total; a.aa4096 = g->d_aa4096; a.aa4096h = g->d_aa4096h; a.out = out_dev;
+    a.total_dev = p->d_totals + 1; a.cap = p->prot_total; a.out = out_dev;
+    a.aa4096 = p->own_code ? p->d_aa8192 : g->d_aa4096;             // mg_plan_set_codon_table
+    a.aa4096h = p->own_code ? p->d_aa8192 + 4096 : g->d_aa4096h;
     return a;
 }
 

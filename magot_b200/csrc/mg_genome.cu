@@ -100,8 +100,9 @@ extern "C" int mg_stream_wait_stream(int device, void *waiter, void *signaller) 
 // ---- 4096-entry translation table -----------------------------------------------------------------
 // index = n0 | n1<<4 | n2<<8 (n0 = first base of the codon, nibble codes as above).  Any nibble >= 8
 // (N, n, '-', IUPAC, exception) gives 'X' (genome.py:816-817); case bit 2 is ignored, which is the
-// `.upper()` of genome.py:812.  Amino acids follow the reference's table (genome.py:795-802).
-static void build_aa4096(uint8_t *t) {
+// `.upper()` of genome.py:812.  Amino acids come from codon64[16*b0 + 4*b1 + b2] (A=0 C=1 G=2 T=3), or with
+// codon64 == NULL from the reference's table (genome.py:795-802, NCBI table 1).
+void build_aa4096(uint8_t *t, const uint8_t *codon64) {
     // reference table is indexed T,C,A,G; our base codes are A=0,C=1,G=2,T=3
     static const char *tcag = "FFLLSSSSYY**CC*WLLLLPPPPHHQQRRRRIIIMTTTTNNKKSSRRVVVVAAAADDEEGGGG";
     static const int to_tcag[4] = {2, 1, 3, 0};
@@ -109,6 +110,8 @@ static void build_aa4096(uint8_t *t) {
         const int n0 = i & 15, n1 = (i >> 4) & 15, n2 = (i >> 8) & 15;
         if (n0 >= 8 || n1 >= 8 || n2 >= 8) {
             t[i] = 'X';
+        } else if (codon64) {
+            t[i] = codon64[(n0 & 3) * 16 + (n1 & 3) * 4 + (n2 & 3)];
         } else {
             t[i] = (uint8_t)tcag[to_tcag[n0 & 3] * 16 + to_tcag[n1 & 3] * 4 + to_tcag[n2 & 3]];
         }
@@ -153,7 +156,7 @@ extern "C" int mg_genome_create(int device, int64_t n_contigs, const int64_t *co
     MG_CUDA(cudaMalloc(&g->d_exc_pos, g->exc_cap * sizeof(int64_t)));
     MG_CUDA(cudaMalloc(&g->d_exc_byte, g->exc_cap));
     uint8_t tbl[4096];
-    build_aa4096(tbl);
+    build_aa4096(tbl, nullptr);
     MG_CUDA(cudaMalloc(&g->d_aa4096, 4096));
     MG_CUDA(cudaMemcpy(g->d_aa4096, tbl, 4096, cudaMemcpyHostToDevice));
     uint8_t tblh[4096];
@@ -189,6 +192,7 @@ extern "C" int mg_genome_destroy(mg_genome *g) {
     cudaFree(g->d_aa4096);
     cudaFree(g->d_aa4096h);
     cudaFree(g->d_stops);
+    cudaFree(g->d_stops_alt);
     if (g->h_pin) cudaFreeHost(g->h_pin);
     delete g;
     return MG_OK;
@@ -306,7 +310,7 @@ extern "C" int mg_genome_pack_device(mg_genome *g, int64_t contig, int64_t offse
     MG_REQUIRE(((uintptr_t)ascii_dev & 15) == 0, "device text must be 16-byte aligned");
     MG_CUDA(cudaSetDevice(g->device));
     g->finalized = false;
-    g->stops_valid = false;
+    g->stops_valid = g->stops_alt_valid = false;
     if (n == 0) return MG_OK;
     return pack_device_chunk(g, g->h_contig_base[contig] + offset, ascii_dev, n, (cudaStream_t)stream);
 }
@@ -316,7 +320,7 @@ extern "C" int mg_genome_pack(mg_genome *g, int64_t contig, int64_t offset, cons
     if (rc) return rc;
     MG_CUDA(cudaSetDevice(g->device));
     g->finalized = false;
-    g->stops_valid = false;
+    g->stops_valid = g->stops_alt_valid = false;
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t STAGE = 64ll << 20;
     rc = mg_ensure_stage(g, std::min<int64_t>(STAGE, (n + 255) / 256 * 256));
@@ -436,7 +440,7 @@ extern "C" int mg_genome_pack_fasta(mg_genome *g, int64_t contig, const uint8_t 
     MG_REQUIRE(n_raw >= 0 && (n_raw == 0 || raw != nullptr), "bad FASTA body");
     MG_CUDA(cudaSetDevice(g->device));
     g->finalized = false;
-    g->stops_valid = false;
+    g->stops_valid = g->stops_alt_valid = false;
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t RAW = 64ll << 20;                   // raw bytes per trip (multiple of the tile)
     const int64_t clen = g->h_contig_len[contig];
@@ -535,7 +539,7 @@ extern "C" int mg_genome_finalize(mg_genome *g, int64_t *n_exceptions_out) {
     g->h_exc_pos.swap(pos);
     g->h_exc_byte.swap(byt);
     g->finalized = true;
-    g->stops_valid = false;
+    g->stops_valid = g->stops_alt_valid = false;
     if (n_exceptions_out) *n_exceptions_out = g->n_exc;
     return MG_OK;
 }

@@ -109,7 +109,7 @@ extern "C" int mg_genome_mask(mg_genome *g, int64_t n_iv, const int32_t *contig,
     MG_REQUIRE(n_iv >= 0 && (n_iv == 0 || (contig && lo && hi)), "bad interval table");
     MG_CUDA(cudaSetDevice(g->device));
     cudaStream_t st = (cudaStream_t)stream;
-    g->stops_valid = false;                          // the stop-codon index of the ORF scan is rebuilt on its next use
+    g->stops_valid = g->stops_alt_valid = false;                          // the stop-codon index of the ORF scan is rebuilt on its next use
     // host: intervals in global base indices
     std::vector<int64_t> glo(n_iv), ghi(n_iv);
     for (int64_t i = 0; i < n_iv; i++) {

@@ -535,6 +535,28 @@ extern "C" int mg_plan_destroy(mg_plan *p) {
     return MG_OK;
 }
 
+// The plan's protein emits read their own translation table from here on.  It is built and uploaded now, so an emit queued or
+// captured in a graph later reads a table that is already on the device; codon64 == NULL goes back to the genome's table.
+extern "C" int mg_plan_set_codon_table(mg_plan *p, const uint8_t *codon64) {
+    MG_REQUIRE(p != nullptr, "plan handle is NULL");
+    if (!codon64) { p->own_code = false; return MG_OK; }
+    // the record pass drops a leading codon for trimX when it holds a base outside ACGT, i.e. where the table gives 'X'
+    for (int c = 0; c < 64; c++) MG_REQUIRE(codon64[c] != 'X', "codon64 maps an A/C/G/T codon to 'X'");
+    MG_CUDA(cudaSetDevice(p->device));
+    uint8_t t[8192];
+    build_aa4096(t, codon64);
+    for (uint32_t c = 0; c < 4096; c++) t[4096 + mg_aa_slot(c)] = t[c];
+    cudaStream_t st = p->last_stream;                 // after the emits already queued with the previous table
+    if (!p->d_aa8192) {
+        int rc = dalloc(p, &p->d_aa8192, 8192, st);
+        if (rc) return rc;
+    }
+    MG_CUDA(cudaMemcpyAsync(p->d_aa8192, t, 8192, cudaMemcpyHostToDevice, st));
+    MG_CUDA(cudaStreamSynchronize(st));
+    p->own_code = true;
+    return MG_OK;
+}
+
 // K1, first half: clamp + lengths + offsets of every piece and record; the two text sizes land in p->d_totals
 static int plan_alloc_tiles(mg_plan *p, int64_t cap_nuc, int64_t cap_prot, cudaStream_t st);
 

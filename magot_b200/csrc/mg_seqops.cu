@@ -192,10 +192,7 @@ extern "C" int mg_translate_ascii_table(int device, const uint8_t *codon64, cons
     MG_CUDA(cudaMallocAsync((void **)&d, b_in + 2 * b_off + b_len + b_l32 + b_drop + b_tmp + b_out + 4096, st));
     if (codon64 != nullptr) {                         // caller's codon table (Sequence.translate(library=...), genome.py:795)
         uint8_t t[4096];
-        for (int i = 0; i < 4096; i++) {
-            const int n0 = i & 15, n1 = (i >> 4) & 15, n2 = (i >> 8) & 15;
-            t[i] = (n0 >= 8 || n1 >= 8 || n2 >= 8) ? 'X' : codon64[(n0 & 3) * 16 + (n1 & 3) * 4 + (n2 & 3)];
-        }
+        build_aa4096(t, codon64);
         aa = d + b_in + 2 * b_off + b_len + b_l32 + b_drop + b_tmp + b_out;
         MG_CUDA(cudaMemcpyAsync(aa, t, 4096, cudaMemcpyHostToDevice, st));   // pageable source: staged before the call returns
     }

@@ -15,6 +15,11 @@
 // (plus strands ascend, minus strands descend; k_six_place), and the residues are produced by a flat
 // 16-residue-per-thread gather like K3 (k_six_aa).  Only when the kept ORFs do not fit the hit list
 // (tiny min_aa: an ORF every few bases) a second genome pass writes them (k_six_orfs<true>).
+//
+// Genetic codes: the stop test is a compile-time expression for the standard code's TAA/TAG/TGA (GEN = false, the default
+// kernels) or, for any other code, a loop over the code's stop codons passed as a kernel argument (GEN = true, SixStops).
+// The residues come from the call's 4096-entry table.  A code whose stops are the standard three (e.g. table 11) runs the
+// default kernels.
 #include <algorithm>
 #include <cstdlib>
 #include <cstring>
@@ -74,6 +79,8 @@ struct mg_sixframe_state {
     int64_t n_aa_tile = 0;
     uint8_t *d_aa = nullptr;                         // library-owned residue buffer for the host variant
     int64_t aa_cap = 0;
+    uint8_t *d_aa4096 = nullptr;                     // residue table of a caller's genetic code (NULL: the genome's standard table)
+    uint8_t h_aa4096[4096];                          // its host copy (source of the asynchronous upload)
     std::vector<void *> owned;
     bool counted = false;
     bool force_single = false;
@@ -118,11 +125,25 @@ struct SixMasks {
     uint64_t pm[3], mm[3];                           // plus / minus stop flags, bit 4k of group g = position 16g+k
 };
 
+// Stop codons of a non-standard genetic code, codon index 16*b0 + 4*b1 + b2 (A=0 C=1 G=2 T=3).  Passed by value as a
+// __grid_constant__ kernel argument: the loop over the codons reads the constant bank.
+struct SixStops {
+    int32_t n;                                       // 0..64
+    uint8_t fwd[64];                                 // the stops, read on the plus strand
+    uint8_t rev[64];                                 // their reverse complements: the minus-strand stops as read forward
+};
+#define SIX_STD_STOPS ((1ull << 48) | (1ull << 50) | (1ull << 56))   // TAA TAG TGA: the stop set of the GEN = false kernels
+
+__device__ __forceinline__ uint64_t pick_plane(int b, uint64_t a, uint64_t c, uint64_t g, uint64_t t) {
+    return (b & 2) ? ((b & 1) ? t : g) : ((b & 1) ? c : a);
+}
+
 // x0 = contig offset of the thread's first position (multiple of 48); gb = contig's global base index
 // WHICH: 0 = both strands, 1 = plus only (s.mm undefined), 2 = minus only (s.pm undefined)
-template <int WHICH>
+// GEN: stops from `ss` instead of TAA/TAG/TGA (ss is not read when GEN is false)
+template <int WHICH, bool GEN>
 __device__ __forceinline__ void six_masks_t(const uint32_t *__restrict__ packed, int64_t gb, int64_t L, int64_t x0,
-                                            const int32_t *cs6, SixMasks &s) {
+                                            const int32_t *cs6, const SixStops &ss, SixMasks &s) {
     uint64_t v[4];
     const uint2 *p = reinterpret_cast<const uint2 *>(packed + ((gb + x0) >> 3));
 #pragma unroll
@@ -146,8 +167,29 @@ __device__ __forceinline__ void six_masks_t(const uint32_t *__restrict__ packed,
         const uint64_t G1 = (G[g] >> 4) | (G[g + 1] << 60), G2 = (G[g] >> 8) | (G[g + 1] << 56);
         const uint64_t T1 = (T[g] >> 4) | (T[g + 1] << 60);
         const uint64_t C1 = (C[g] >> 4) | (C[g + 1] << 60);
-        if (WHICH != 2) s.pm[g] = T[g] & ((A1 & (A2 | G2)) | (G1 & A2));              // TAA TAG TGA
-        if (WHICH != 1) s.mm[g] = A2 & ((T1 & (T[g] | C[g])) | (C1 & T[g]));          // TTA CTA TCA = rc of the above
+        if (!GEN) {
+            if (WHICH != 2) s.pm[g] = T[g] & ((A1 & (A2 | G2)) | (G1 & A2));          // TAA TAG TGA
+            if (WHICH != 1) s.mm[g] = A2 & ((T1 & (T[g] | C[g])) | (C1 & T[g]));      // TTA CTA TCA = rc of the above
+        } else {
+            // every stop codon b0 b1 b2: the AND of the planes of b0, b1, b2 at offsets 0, 1, 2
+            const uint64_t T2 = (T[g] >> 8) | (T[g + 1] << 56), C2 = (C[g] >> 8) | (C[g + 1] << 56);
+            uint64_t pm = 0, mm = 0;
+#pragma unroll 1
+            for (int i = 0; i < ss.n; i++) {
+                if (WHICH != 2) {
+                    const int c = ss.fwd[i];
+                    pm |= pick_plane(c >> 4, A[g], C[g], G[g], T[g]) & pick_plane((c >> 2) & 3, A1, C1, G1, T1) &
+                          pick_plane(c & 3, A2, C2, G2, T2);
+                }
+                if (WHICH != 1) {
+                    const int c = ss.rev[i];
+                    mm |= pick_plane(c >> 4, A[g], C[g], G[g], T[g]) & pick_plane((c >> 2) & 3, A1, C1, G1, T1) &
+                          pick_plane(c & 3, A2, C2, G2, T2);
+                }
+            }
+            if (WHICH != 2) s.pm[g] = pm;
+            if (WHICH != 1) s.mm[g] = mm;
+        }
     }
     // ---- validity at the contig ends
     const int64_t lim = L - 2 - x0;                  // positions t >= lim have no full codon
@@ -172,9 +214,10 @@ __device__ __forceinline__ void six_masks_t(const uint32_t *__restrict__ packed,
     }
 }
 
+template <bool GEN>
 __device__ __forceinline__ void six_masks(const uint32_t *__restrict__ packed, int64_t gb, int64_t L, int64_t x0,
-                                          const int32_t *cs6, SixMasks &s) {
-    six_masks_t<0>(packed, gb, L, x0, cs6, s);
+                                          const int32_t *cs6, const SixStops &ss, SixMasks &s) {
+    six_masks_t<0, GEN>(packed, gb, L, x0, cs6, ss, s);
 }
 
 // residue (t % 3) selected by stream sidx: plus frame f -> rho_f, minus -> (L%3 - rho_f) % 3
@@ -227,7 +270,6 @@ __device__ __forceinline__ void stops_first_last(const uint64_t x[SIX_HALVES], i
 }
 
 struct TileInfo;
-__device__ __forceinline__ void thread_stops(const uint32_t *__restrict__ packed, const TileInfo &ti, int64_t x0, ThreadStops &ts);
 
 struct TileInfo {
     int64_t c, ci, k, gb, L, Tc;                     // contig, its index in the scanned list, tile index in contig, global base, length, tiles in contig
@@ -299,13 +341,15 @@ __device__ __forceinline__ void tile_info_at(int64_t tile, int64_t lo, const int
     }
 }
 
-__device__ __forceinline__ void thread_stops(const uint32_t *__restrict__ packed, const TileInfo &ti, int64_t x0, ThreadStops &ts) {
+template <bool GEN>
+__device__ __forceinline__ void thread_stops(const uint32_t *__restrict__ packed, const TileInfo &ti, int64_t x0, const SixStops &ss,
+                                             ThreadStops &ts) {
 #pragma unroll
     for (int h = 0; h < SIX_HALVES; h++) {
         const int64_t xh = x0 + SIX_HALF * h;
         if (xh < ti.L) {
             SixMasks sm;
-            six_masks(packed, ti.gb, ti.L, xh, ti.cs, sm);
+            six_masks<GEN>(packed, ti.gb, ti.L, xh, ti.cs, ss, sm);
             ts.p[h] = pos48(sm.pm);
             ts.m[h] = pos48(sm.mm);
         } else {
@@ -441,13 +485,13 @@ __device__ __forceinline__ int64_t block_incl_sum(int64_t v, int64_t *s_warp, in
     return v + off;
 }
 
-template <bool EMIT>
+template <bool EMIT, bool GEN>
 __global__ void __launch_bounds__(SIX_THREADS) k_six_orfs(
     const uint32_t *__restrict__ packed, const int64_t *__restrict__ tile_base, int64_t nc, const int32_t *__restrict__ cid,
     const int64_t *__restrict__ contig_len, const int64_t *__restrict__ contig_base, const int32_t *__restrict__ cs,
     const int64_t *__restrict__ m, int64_t n_tiles, const int64_t *__restrict__ carry, int64_t min_aa, int64_t two_T,
     int32_t *__restrict__ cnt, const int64_t *__restrict__ cnt_off, mg_orf *__restrict__ recs, int32_t *__restrict__ lens,
-    int64_t *__restrict__ srcs) {
+    int64_t *__restrict__ srcs, const __grid_constant__ SixStops ss) {
     __shared__ TileInfo ti;
     __shared__ int s_cnt[6];
     __shared__ int64_t s_warp[SIX_THREADS / 32];
@@ -460,7 +504,7 @@ __global__ void __launch_bounds__(SIX_THREADS) k_six_orfs(
     const bool active = x0 < ti.L;
     const bool is_end_thread = active && (x0 + SIX_BPT >= ti.L);       // owns the virtual high-end stops
     ThreadStops sm;                                   // the thread's stops, one bit per position
-    if (active) thread_stops(packed, ti, x0, sm);
+    if (active) thread_stops<GEN>(packed, ti, x0, ss, sm);
     else { for (int h = 0; h < SIX_HALVES; h++) { sm.p[h] = 0; sm.m[h] = 0; } }
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
 
@@ -548,11 +592,13 @@ __global__ void __launch_bounds__(SIX_THREADS) k_six_orfs(
 #define SIX_LOOK_PREFIX (2ull << 62)                 // value = 1 + last stop at or before the end of this tile (0 = none)
 #define SIX_LOOK_MASK (3ull << 62)
 
+template <bool GEN>
 __global__ void __launch_bounds__(SIX_THREADS, SIX_SCAN_MINB) k_six_scan(
     const uint32_t *__restrict__ packed, const int64_t *__restrict__ tile_base, int64_t nc, const int32_t *__restrict__ cid,
     const int64_t *__restrict__ contig_len, const int64_t *__restrict__ contig_base, const int32_t *__restrict__ cs,
     const int64_t *__restrict__ m, const int32_t *__restrict__ tile_contig, int64_t n_tiles, unsigned long long *look, int64_t *__restrict__ carry_out, int64_t min_aa,
-    int64_t two_T, int32_t *__restrict__ cnt, SixHit *__restrict__ hits, int64_t hit_cap, unsigned long long *hit_count) {
+    int64_t two_T, int32_t *__restrict__ cnt, SixHit *__restrict__ hits, int64_t hit_cap, unsigned long long *hit_count,
+    const __grid_constant__ SixStops ss) {
     __shared__ TileInfo ti;
     __shared__ int64_t s_warp[SIX_THREADS / 32];
     __shared__ int s_wlast[6][SIX_THREADS / 32];     // per-warp max of `last stop in thread`
@@ -571,7 +617,7 @@ __global__ void __launch_bounds__(SIX_THREADS, SIX_SCAN_MINB) k_six_scan(
     const bool active = x0 < ti.L;
     const bool is_end_thread = active && (x0 + SIX_BPT >= ti.L);       // owns the virtual high-end stops
     ThreadStops sm;                                   // the thread's stops, one bit per position
-    if (active) thread_stops(packed, ti, x0, sm);
+    if (active) thread_stops<GEN>(packed, ti, x0, ss, sm);
     else { for (int h = 0; h < SIX_HALVES; h++) { sm.p[h] = 0; sm.m[h] = 0; } }
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
 
@@ -753,7 +799,9 @@ __global__ void __launch_bounds__(SIX_THREADS, SIX_SCAN_MINB) k_six_scan(
 static_assert(SIX_TILE % (SIX_WIN * 32) == 0, "a tile must hold a whole number of bitmap words");
 
 // stops of stream s inside window w of the contig (two 48-base halves), one bit per position
-__device__ __forceinline__ void window_stream_stops(const uint32_t *__restrict__ packed, const TileInfo &ti, int64_t w, int s, uint64_t x[2]) {
+template <bool GEN>
+__device__ __forceinline__ void window_stream_stops(const uint32_t *__restrict__ packed, const TileInfo &ti, int64_t w, int s,
+                                                    const SixStops &ss, uint64_t x[2]) {
     const uint64_t rm = 0x0000249249249249ull << stream_res(s, ti.Lm3);
 #pragma unroll
     for (int h = 0; h < 2; h++) {
@@ -762,21 +810,23 @@ __device__ __forceinline__ void window_stream_stops(const uint32_t *__restrict__
         if (xh < ti.L) {
             SixMasks sm;
             if (s & 1) {                                   // one strand only: half the mask logic (s is uniform across the warp)
-                six_masks_t<1>(packed, ti.gb, ti.L, xh, ti.cs, sm);
+                six_masks_t<1, GEN>(packed, ti.gb, ti.L, xh, ti.cs, ss, sm);
                 x[h] = pos48(sm.pm) & rm;
             } else {
-                six_masks_t<2>(packed, ti.gb, ti.L, xh, ti.cs, sm);
+                six_masks_t<2, GEN>(packed, ti.gb, ti.L, xh, ti.cs, ss, sm);
                 x[h] = pos48(sm.mm) & rm;
             }
         }
     }
 }
 
+template <bool GEN>
 __global__ void __launch_bounds__(256) k_six_bits(const uint32_t *__restrict__ packed, const int64_t *__restrict__ tile_base,
                                                   const int32_t *__restrict__ cid, const int64_t *__restrict__ contig_len,
                                                   const int64_t *__restrict__ contig_base, const int32_t *__restrict__ cs,
                                                   const int64_t *__restrict__ m, const int32_t *__restrict__ tile_contig,
-                                                  uint32_t *__restrict__ bits, int32_t *__restrict__ last_set) {
+                                                  uint32_t *__restrict__ bits, int32_t *__restrict__ last_set,
+                                                  const __grid_constant__ SixStops ss) {
     __shared__ TileInfo ti;
     const int64_t tile = blockIdx.x / 3;
     const int part = blockIdx.x % 3;
@@ -794,7 +844,7 @@ __global__ void __launch_bounds__(256) k_six_bits(const uint32_t *__restrict__ p
         const int64_t xh = x0 + SIX_HALF * h;
         if (xh < ti.L) {
             SixMasks sm;
-            six_masks(packed, ti.gb, ti.L, xh, ti.cs, sm);
+            six_masks<GEN>(packed, ti.gb, ti.L, xh, ti.cs, ss, sm);
 #pragma unroll
             for (int r = 0; r < 3; r++) {
                 hp[r] |= (sm.pm[0] & res_mask(r)) | (sm.pm[1] & res_mask((r + 2) % 3)) | (sm.pm[2] & res_mask((r + 1) % 3));
@@ -833,9 +883,11 @@ __device__ __forceinline__ int64_t six_span3(const TileInfo &ti, int s, int64_t 
 // bases instead of ~8 per base on the codon logic (k_six_bits: 790 M warp instructions, 1.08 ms on config 5).  Built lazily by
 // the first ORF scan after mg_genome_finalize / mg_genome_mask (k_stop_index, one thread per 96-base window, six_masks as in the
 // scan kernels, so the validity rules at contig ends are the same code).
+template <bool GEN>
 __global__ void __launch_bounds__(256) k_stop_index(const uint32_t *__restrict__ packed, const int64_t *__restrict__ contig_len,
                                                     const int64_t *__restrict__ contig_base, const int64_t *__restrict__ win_base, int64_t nc,
-                                                    const int32_t *__restrict__ cs, uint32_t *__restrict__ sp, uint32_t *__restrict__ sm_) {
+                                                    const int32_t *__restrict__ cs, uint32_t *__restrict__ sp, uint32_t *__restrict__ sm_,
+                                                    const __grid_constant__ SixStops ss) {
     const int64_t flat = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (flat >= win_base[nc]) return;
     int64_t lo = 0, hi = nc;                          // largest c with win_base[c] <= flat
@@ -853,7 +905,7 @@ __global__ void __launch_bounds__(256) k_stop_index(const uint32_t *__restrict__
         const int64_t xh = w * SIX_WIN + SIX_HALF * h;
         if (xh < L) {
             SixMasks s;
-            six_masks(packed, gb, L, xh, cs6, s);
+            six_masks<GEN>(packed, gb, L, xh, cs6, ss, s);
             P[h] = pos48(s.pm);
             M[h] = pos48(s.mm);
         }
@@ -932,7 +984,8 @@ __global__ void __launch_bounds__(256) k_six_bits_ix(const uint32_t *__restrict_
 // list order is the window order, so the rank of a kept ORF inside the row is a running count + a ballot prefix.
 #define CAND_WARPS 8
 #define CAND_LIST (SIX_WPT / 3 + 2)                  // a candidate needs two stop-free windows in front of it
-template <bool IX>                                   // IX: exact stop positions from the stop-codon index instead of the packed bases
+// IX: exact stop positions from the stop-codon index instead of the packed bases; GEN: as in six_masks_t (IX == false only)
+template <bool IX, bool GEN>
 __global__ void __launch_bounds__(32 * CAND_WARPS) k_six_cand(const uint32_t *__restrict__ packed, const uint32_t *__restrict__ stops,
                                                   int64_t stop_words, const int64_t *__restrict__ tile_base,
                                                   const int32_t *__restrict__ cid, const int64_t *__restrict__ contig_len,
@@ -940,7 +993,7 @@ __global__ void __launch_bounds__(32 * CAND_WARPS) k_six_cand(const uint32_t *__
                                                   const int64_t *__restrict__ m, const int32_t *__restrict__ tile_contig, int64_t n_tiles,
                                                   const uint32_t *__restrict__ bits, const int32_t *__restrict__ last_set, int64_t min_aa,
                                                   int32_t *__restrict__ cnt, SixHit *__restrict__ hits, int64_t hit_cap,
-                                                  unsigned long long *hit_count) {
+                                                  unsigned long long *hit_count, const __grid_constant__ SixStops ss) {
     // per warp: the row's candidates (window, previous window with a stop), overwritten in place by the bounding stops (xl, xh)
     __shared__ int32_t s_w[CAND_WARPS][CAND_LIST], s_pw[CAND_WARPS][CAND_LIST];
     __shared__ uint8_t s_f[CAND_WARPS][CAND_LIST];          // bit 0 xl_real, bit 1 xh_real, bit 2 kept
@@ -1034,11 +1087,11 @@ __global__ void __launch_bounds__(32 * CAND_WARPS) k_six_cand(const uint32_t *__
                 } else {
                     uint64_t x[2];
                     if (xh_real) {
-                        window_stream_stops(packed, ti, w, s, x);
+                        window_stream_stops<GEN>(packed, ti, w, s, ss, x);
                         xh = w * SIX_WIN + (x[0] ? __ffsll((long long)x[0]) - 1 : SIX_HALF + __ffsll((long long)x[1]) - 1);
                     }
                     if (xl_real) {
-                        window_stream_stops(packed, ti, pw, s, x);
+                        window_stream_stops<GEN>(packed, ti, pw, s, ss, x);
                         xl = pw * SIX_WIN + (x[1] ? SIX_HALF + 63 - __clzll((long long)x[1]) : 63 - __clzll((long long)x[0]));
                     }
                 }
@@ -1286,23 +1339,27 @@ static int six_alloc(mg_sixframe_state *s, T **p, int64_t n) {
     return MG_OK;
 }
 
-// contigs given as a LIST (any order, e.g. the LPT share of one GPU): ORFs come out contig by contig in list order
-// stop-codon index of the whole genome (see k_stop_index); st-ordered, no host wait
-static int six_build_stops(mg_genome *g, cudaStream_t st) {
-    if (g->stops_valid) return MG_OK;
+// stop-codon index of the whole genome (see k_stop_index) for the stop set `key` (bit 16*b0 + 4*b1 + b2 per stop codon);
+// st-ordered, no host wait.  The standard set has its own index; ONE other set is kept next to it (0.25 B/base more), so
+// that scans with another genetic code neither rebuild nor overwrite the standard one.  *out = the index to scan.
+static int six_build_stops(mg_genome *g, cudaStream_t st, uint64_t key, const SixStops &ss, const uint32_t **out) {
+    const bool gen = key != SIX_STD_STOPS;
+    uint32_t *&buf = gen ? g->d_stops_alt : g->d_stops;
+    *out = buf;
+    if (gen ? (g->stops_alt_valid && g->stops_alt_key == key) : g->stops_valid) return MG_OK;
     const int64_t W = g->total_bases / 32 + 8, nc = g->n_contigs;
-    if (!g->d_stops || g->stop_words != W) {
-        if (g->d_stops) { MG_CUDA(cudaFree(g->d_stops)); g->device_bytes -= 2 * g->stop_words * 4; }
-        g->d_stops = nullptr;
-        MG_CUDA(cudaMalloc((void **)&g->d_stops, 2 * W * sizeof(uint32_t)));
+    if (!buf) {                                              // W only depends on the genome's size, fixed at mg_genome_create
+        MG_CUDA(cudaMalloc((void **)&buf, 2 * W * sizeof(uint32_t)));
         g->stop_words = W;
         g->device_bytes += 2 * W * 4;
     }
-    MG_CUDA(cudaMemsetAsync(g->d_stops, 0, 2 * W * sizeof(uint32_t), st));
+    *out = buf;
+    if (gen) { g->stops_alt_valid = false; g->stops_alt_key = key; }
+    MG_CUDA(cudaMemsetAsync(buf, 0, 2 * W * sizeof(uint32_t), st));
     std::vector<int64_t> wb(nc + 1, 0);
     std::vector<int32_t> ident(nc);
     for (int64_t c = 0; c < nc; c++) { wb[c + 1] = wb[c] + (g->h_contig_len[c] + SIX_WIN - 1) / SIX_WIN; ident[c] = (int32_t)c; }
-    if (wb[nc] == 0) { g->stops_valid = true; return MG_OK; }
+    if (wb[nc] == 0) { (gen ? g->stops_alt_valid : g->stops_valid) = true; return MG_OK; }
     char *tmp = nullptr;                                     // win_base | cs | m | ident
     const size_t o_cs = (nc + 1) * 8, o_m = o_cs + nc * 6 * 4 + 8, o_id = o_m + nc * 6 * 8, bytes = o_id + nc * 4;
     MG_CUDA(cudaMallocAsync((void **)&tmp, bytes, st));
@@ -1312,22 +1369,40 @@ static int six_build_stops(mg_genome *g, cudaStream_t st) {
     MG_CUDA(cudaMemcpyAsync(d_id, ident.data(), nc * 4, cudaMemcpyHostToDevice, st));
     k_six_streams<<<(unsigned)((nc * 6 + 127) / 128), 128, 0, st>>>(g->d_packed, g->d_contig_len, g->d_contig_base, d_id, nc, d_cs, d_m);
     MG_LAUNCH_CHECK();
-    k_stop_index<<<(unsigned)((wb[nc] + 255) / 256), 256, 0, st>>>(g->d_packed, g->d_contig_len, g->d_contig_base, d_wb, nc, d_cs, g->d_stops,
-                                                                   g->d_stops + W);
+    (gen ? k_stop_index<true> : k_stop_index<false>)<<<(unsigned)((wb[nc] + 255) / 256), 256, 0, st>>>(
+        g->d_packed, g->d_contig_len, g->d_contig_base, d_wb, nc, d_cs, buf, buf + W, ss);
     MG_LAUNCH_CHECK();
     MG_CUDA(cudaStreamSynchronize(st));                      // wb / ident are host vectors of this frame
     MG_CUDA(cudaFreeAsync(tmp, st));
-    g->stops_valid = true;
+    (gen ? g->stops_alt_valid : g->stops_valid) = true;
     return MG_OK;
 }
 
-extern "C" int mg_sixframe_count_list(mg_genome *g, int64_t n_list, const int64_t *contig_ids, int64_t min_aa, int64_t *n_orf,
-                                      int64_t *n_bytes, void *stream) {
+// contigs given as a LIST (any order, e.g. the LPT share of one GPU): ORFs come out contig by contig in list order
+extern "C" int mg_sixframe_count_list_table(mg_genome *g, int64_t n_list, const int64_t *contig_ids, int64_t min_aa,
+                                            const uint8_t *codon64, int64_t *n_orf, int64_t *n_bytes, void *stream) {
     MG_REQUIRE(g != nullptr, "genome handle is NULL");
     MG_REQUIRE(g->finalized, "mg_genome_finalize has not been called");
     MG_REQUIRE(n_list >= 0 && (n_list == 0 || contig_ids != nullptr), "bad contig list");
     MG_REQUIRE(min_aa >= 0, "min_aa must be >= 0");
     for (int64_t i = 0; i < n_list; i++) MG_REQUIRE(contig_ids[i] >= 0 && contig_ids[i] < g->n_contigs, "contig index out of range");
+    // the genetic code: its stop set selects the scan kernels, its table the residues
+    uint64_t key = SIX_STD_STOPS;
+    SixStops ss;
+    memset(&ss, 0, sizeof(ss));
+    if (codon64) {
+        // k_six_streams drops a leading codon for trimX when it holds a base outside ACGT, i.e. where the table gives 'X'
+        for (int c = 0; c < 64; c++) MG_REQUIRE(codon64[c] != 'X', "codon64 maps an A/C/G/T codon to 'X'");
+        key = 0;
+        for (int c = 0; c < 64; c++) {
+            if (codon64[c] != '*') continue;
+            key |= 1ull << c;
+            ss.fwd[ss.n] = (uint8_t)c;
+            ss.rev[ss.n] = (uint8_t)(16 * (3 - (c & 3)) + 4 * (3 - ((c >> 2) & 3)) + (3 - (c >> 4)));
+            ss.n++;
+        }
+    }
+    const bool gen = key != SIX_STD_STOPS;
     MG_CUDA(cudaSetDevice(g->device));
     cudaStream_t st = (cudaStream_t)stream;
     mg_sixframe_free(g);
@@ -1355,6 +1430,11 @@ extern "C" int mg_sixframe_count_list(mg_genome *g, int64_t n_list, const int64_
     if (s->n_tiles == 0) return MG_OK;
     int rc;
 #define TRY(x) do { rc = (x); if (rc) return rc; } while (0)
+    if (codon64) {
+        build_aa4096(s->h_aa4096, codon64);
+        TRY(six_alloc(s, &s->d_aa4096, 4096));
+        MG_CUDA(cudaMemcpyAsync(s->d_aa4096, s->h_aa4096, 4096, cudaMemcpyHostToDevice, st));
+    }
     TRY(six_alloc(s, &s->d_cid, nc));
     MG_CUDA(cudaMemcpyAsync(s->d_cid, h_cid.data(), nc * sizeof(int32_t), cudaMemcpyHostToDevice, st));
     TRY(six_alloc(s, &s->d_tile_base, nc + 1));
@@ -1388,27 +1468,29 @@ extern "C" int mg_sixframe_count_list(mg_genome *g, int64_t n_list, const int64_
         MG_CUDA(cudaMemsetAsync(d_last, 0xFF, s->n_tiles * 6 * sizeof(int32_t), st));
         const unsigned cand_grid = (unsigned)((s->n_tiles * 6 + CAND_WARPS - 1) / CAND_WARPS);
         if (two_level == 2) {
-            TRY(six_build_stops(g, st));
-            k_six_bits_ix<<<(unsigned)s->n_tiles, 256, 0, st>>>(g->d_stops, g->stop_words, s->d_tile_base, s->d_cid, g->d_contig_len,
+            const uint32_t *stops = nullptr;
+            TRY(six_build_stops(g, st, key, ss, &stops));
+            k_six_bits_ix<<<(unsigned)s->n_tiles, 256, 0, st>>>(stops, g->stop_words, s->d_tile_base, s->d_cid, g->d_contig_len,
                                                                      g->d_contig_base, s->d_cs, s->d_m, s->d_tile_contig, d_bits, d_last);
             MG_LAUNCH_CHECK();
-            k_six_cand<true><<<cand_grid, 32 * CAND_WARPS, 0, st>>>(g->d_packed, g->d_stops, g->stop_words, s->d_tile_base, s->d_cid, g->d_contig_len,
-                                                                     g->d_contig_base, s->d_cs, s->d_m, s->d_tile_contig, s->n_tiles, d_bits,
-                                                                     d_last, min_aa, s->d_cnt, s->d_hits, s->hit_cap, s->d_hit_count);
+            k_six_cand<true, false><<<cand_grid, 32 * CAND_WARPS, 0, st>>>(g->d_packed, stops, g->stop_words, s->d_tile_base, s->d_cid,
+                                                                            g->d_contig_len, g->d_contig_base, s->d_cs, s->d_m, s->d_tile_contig,
+                                                                            s->n_tiles, d_bits, d_last, min_aa, s->d_cnt, s->d_hits, s->hit_cap,
+                                                                            s->d_hit_count, ss);
             MG_LAUNCH_CHECK();
         } else {
-            k_six_bits<<<(unsigned)(s->n_tiles * 3), 256, 0, st>>>(g->d_packed, s->d_tile_base, s->d_cid, g->d_contig_len, g->d_contig_base, s->d_cs,
-                                                                  s->d_m, s->d_tile_contig, d_bits, d_last);
+            (gen ? k_six_bits<true> : k_six_bits<false>)<<<(unsigned)(s->n_tiles * 3), 256, 0, st>>>(
+                g->d_packed, s->d_tile_base, s->d_cid, g->d_contig_len, g->d_contig_base, s->d_cs, s->d_m, s->d_tile_contig, d_bits, d_last, ss);
             MG_LAUNCH_CHECK();
-            k_six_cand<false><<<cand_grid, 32 * CAND_WARPS, 0, st>>>(g->d_packed, nullptr, 0, s->d_tile_base, s->d_cid, g->d_contig_len,
-                                                                      g->d_contig_base, s->d_cs, s->d_m, s->d_tile_contig, s->n_tiles, d_bits,
-                                                                      d_last, min_aa, s->d_cnt, s->d_hits, s->hit_cap, s->d_hit_count);
+            (gen ? k_six_cand<false, true> : k_six_cand<false, false>)<<<cand_grid, 32 * CAND_WARPS, 0, st>>>(
+                g->d_packed, nullptr, 0, s->d_tile_base, s->d_cid, g->d_contig_len, g->d_contig_base, s->d_cs, s->d_m, s->d_tile_contig,
+                s->n_tiles, d_bits, d_last, min_aa, s->d_cnt, s->d_hits, s->hit_cap, s->d_hit_count, ss);
             MG_LAUNCH_CHECK();
         }
     } else {
-        k_six_scan<<<(unsigned)s->n_tiles, SIX_THREADS, 0, st>>>(g->d_packed, s->d_tile_base, nc, s->d_cid, g->d_contig_len, g->d_contig_base,
-                                                                  s->d_cs, s->d_m, s->d_tile_contig, s->n_tiles, s->d_look, s->d_carry, min_aa, 2 * g->total_bases,
-                                                                  s->d_cnt, s->d_hits, s->hit_cap, s->d_hit_count);
+        (gen ? k_six_scan<true> : k_six_scan<false>)<<<(unsigned)s->n_tiles, SIX_THREADS, 0, st>>>(
+            g->d_packed, s->d_tile_base, nc, s->d_cid, g->d_contig_len, g->d_contig_base, s->d_cs, s->d_m, s->d_tile_contig, s->n_tiles,
+            s->d_look, s->d_carry, min_aa, 2 * g->total_bases, s->d_cnt, s->d_hits, s->hit_cap, s->d_hit_count, ss);
         MG_LAUNCH_CHECK();
     }
     s->scan_tmp_cap = mg_scan_tmp_elems(s->n_tiles * 6) + 2;
@@ -1421,7 +1503,7 @@ extern "C" int mg_sixframe_count_list(mg_genome *g, int64_t n_list, const int64_
         std::vector<int64_t> ids(contig_ids, contig_ids + n_list);
         mg_sixframe_free(g);
         g_six_force_single = true;
-        const int rc2 = mg_sixframe_count_list(g, n_list, ids.data(), min_aa, n_orf, n_bytes, stream);
+        const int rc2 = mg_sixframe_count_list_table(g, n_list, ids.data(), min_aa, codon64, n_orf, n_bytes, stream);
         g_six_force_single = false;
         return rc2;
 #define TRY(x) do { rc = (x); if (rc) return rc; } while (0)
@@ -1436,9 +1518,9 @@ extern "C" int mg_sixframe_count_list(mg_genome *g, int64_t n_list, const int64_
                                                                             g->d_contig_base, s->d_cs, s->d_m, s->d_cnt_off, 2 * g->total_bases,
                                                                             s->d_recs, s->d_len, s->d_src);
         } else {                                     // dense output (tiny min_aa): second pass over the genome
-            k_six_orfs<true><<<(unsigned)s->n_tiles, SIX_THREADS, 0, st>>>(g->d_packed, s->d_tile_base, nc, s->d_cid, g->d_contig_len,
-                                                                          g->d_contig_base, s->d_cs, s->d_m, s->n_tiles, s->d_carry, min_aa,
-                                                                          2 * g->total_bases, nullptr, s->d_cnt_off, s->d_recs, s->d_len, s->d_src);
+            (gen ? k_six_orfs<true, true> : k_six_orfs<true, false>)<<<(unsigned)s->n_tiles, SIX_THREADS, 0, st>>>(
+                g->d_packed, s->d_tile_base, nc, s->d_cid, g->d_contig_len, g->d_contig_base, s->d_cs, s->d_m, s->n_tiles, s->d_carry,
+                min_aa, 2 * g->total_bases, nullptr, s->d_cnt_off, s->d_recs, s->d_len, s->d_src, ss);
         }
         MG_LAUNCH_CHECK();
         const int64_t need = mg_scan_tmp_elems(s->n_orf) + 2;
@@ -1462,13 +1544,23 @@ extern "C" int mg_sixframe_count_list(mg_genome *g, int64_t n_list, const int64_
     return MG_OK;
 }
 
-extern "C" int mg_sixframe_count(mg_genome *g, int64_t contig_lo, int64_t contig_hi, int64_t min_aa, int64_t *n_orf,
-                                 int64_t *n_bytes, void *stream) {
+extern "C" int mg_sixframe_count_list(mg_genome *g, int64_t n_list, const int64_t *contig_ids, int64_t min_aa, int64_t *n_orf,
+                                      int64_t *n_bytes, void *stream) {
+    return mg_sixframe_count_list_table(g, n_list, contig_ids, min_aa, nullptr, n_orf, n_bytes, stream);
+}
+
+extern "C" int mg_sixframe_count_table(mg_genome *g, int64_t contig_lo, int64_t contig_hi, int64_t min_aa, const uint8_t *codon64,
+                                       int64_t *n_orf, int64_t *n_bytes, void *stream) {
     MG_REQUIRE(g != nullptr, "genome handle is NULL");
     MG_REQUIRE(contig_lo >= 0 && contig_lo <= contig_hi && contig_hi <= g->n_contigs, "contig range out of bounds");
     std::vector<int64_t> ids(contig_hi - contig_lo);
     for (int64_t i = 0; i < (int64_t)ids.size(); i++) ids[i] = contig_lo + i;
-    return mg_sixframe_count_list(g, (int64_t)ids.size(), ids.data(), min_aa, n_orf, n_bytes, stream);
+    return mg_sixframe_count_list_table(g, (int64_t)ids.size(), ids.data(), min_aa, codon64, n_orf, n_bytes, stream);
+}
+
+extern "C" int mg_sixframe_count(mg_genome *g, int64_t contig_lo, int64_t contig_hi, int64_t min_aa, int64_t *n_orf,
+                                 int64_t *n_bytes, void *stream) {
+    return mg_sixframe_count_table(g, contig_lo, contig_hi, min_aa, nullptr, n_orf, n_bytes, stream);
 }
 
 extern "C" int mg_sixframe_emit_device(mg_genome *g, uint8_t *aa_out_dev, mg_orf *recs_dev, void *stream) {
@@ -1480,7 +1572,7 @@ extern "C" int mg_sixframe_emit_device(mg_genome *g, uint8_t *aa_out_dev, mg_orf
     if (aa_out_dev && s->n_bytes > 0) {
         MG_REQUIRE(((uintptr_t)aa_out_dev & 15) == 0, "aa_out_dev must be 16-byte aligned");
         k_six_aa<<<(unsigned)s->n_aa_tile, AA_THREADS, 0, st>>>(g->d_packed, s->d_aa_off, s->d_src, s->n_orf, s->d_aa_tile, s->n_bytes,
-                                                                g->d_aa4096, aa_out_dev);
+                                                                s->d_aa4096 ? s->d_aa4096 : g->d_aa4096, aa_out_dev);
         MG_LAUNCH_CHECK();
     }
     if (recs_dev && s->n_orf > 0)

@@ -147,6 +147,15 @@ class Plan(object):
         self.nuc_total = None
         self.prot_total = None
 
+    def set_codon_table(self, codon64):
+        """Genetic code of this plan's protein text (mg_plan_set_codon_table): codon64 = 64 bytes as gencode.codon64(n),
+        None = the standard code.  Takes effect for every emit queued after the call."""
+        if codon64 is not None:
+            codon64 = bytes(codon64)
+            if len(codon64) != 64:
+                raise ValueError("codon64 must hold 64 bytes")
+        check(lib.mg_plan_set_codon_table(self.handle, codon64))
+
     def prepare(self, trimx=True, use_phase=False):
         flags = (_lib.MG_PROT_TRIMX if trimx else 0) | (_lib.MG_PROT_USE_PHASE if use_phase else 0)
         a, b = ctypes.c_int64(0), ctypes.c_int64(0)
@@ -239,10 +248,13 @@ class Plan(object):
             pass
 
 
-def run_table(genome, table, protein=False, trimx=True, use_phase=False, want_lengths=False):
-    """One pass of the hot path over one batch on one GPU. Returns (text bytes, (nuc_len, aa_len) | None)."""
+def run_table(genome, table, protein=False, trimx=True, use_phase=False, want_lengths=False, codon64=None):
+    """One pass of the hot path over one batch on one GPU. Returns (text bytes, (nuc_len, aa_len) | None).
+    codon64: genetic code of the protein text (gencode.codon64), None = the standard code."""
     plan = Plan(genome, table)
     try:
+        if codon64 is not None:
+            plan.set_codon_table(codon64)
         plan.prepare(trimx=trimx, use_phase=use_phase)
         lens = plan.lengths() if want_lengths else None
         text = plan.emit_bytes(protein=protein)
@@ -251,10 +263,12 @@ def run_table(genome, table, protein=False, trimx=True, use_phase=False, want_le
     return text, lens
 
 
-def run_table_both(genome, table, trimx=True, use_phase=False, async_prepare=False):
+def run_table_both(genome, table, trimx=True, use_phase=False, async_prepare=False, codon64=None):
     """Nucleotide AND protein text of one batch from one fused pass (K23). Returns (nuc bytes, prot bytes)."""
     plan = Plan(genome, table)
     try:
+        if codon64 is not None:
+            plan.set_codon_table(codon64)
         if async_prepare:
             plan.prepare_async(trimx=trimx, use_phase=use_phase)
             plan.totals()
@@ -266,11 +280,13 @@ def run_table_both(genome, table, trimx=True, use_phase=False, async_prepare=Fal
     return nuc.tobytes(), prot.tobytes()
 
 
-def run_products(genome, table_a, table_b, protein_b=True, trimx=True, use_phase=False):
+def run_products(genome, table_a, table_b, protein_b=True, trimx=True, use_phase=False, codon64=None):
     """mg_emit_products_host: nucleotide text of table_a, nucleotide (+ protein) text of table_b from one launch.
     Returns (text_a, nuc_b, prot_b) as bytes (prot_b is b"" without protein_b)."""
     pa, pb = Plan(genome, table_a), Plan(genome, table_b)
     try:
+        if codon64 is not None:
+            pb.set_codon_table(codon64)
         pa.prepare(trimx=trimx, use_phase=use_phase)
         pb.prepare(trimx=trimx, use_phase=use_phase)
         oa = np.empty(pa.nuc_total, dtype=np.uint8)
@@ -309,9 +325,9 @@ class ShardedGenome(object):
     def primary(self):
         return self.replicas[0]
 
-    def run_table(self, table, protein=False, trimx=True, use_phase=False, want_lengths=False):
+    def run_table(self, table, protein=False, trimx=True, use_phase=False, want_lengths=False, codon64=None):
         if len(self.replicas) == 1 or table.n_rec < 2 * len(self.replicas):
-            return run_table(self.primary, table, protein, trimx, use_phase, want_lengths)
+            return run_table(self.primary, table, protein, trimx, use_phase, want_lengths, codon64)
         bounds = shard_bounds(table.approx_bytes_per_record(), len(self.replicas))
         results = [None] * len(self.replicas)
         errors = []
@@ -320,7 +336,7 @@ class ShardedGenome(object):
             try:
                 r0, r1 = bounds[k], bounds[k + 1]
                 if r1 > r0:
-                    results[k] = run_table(self.replicas[k], table.slice(r0, r1), protein, trimx, use_phase, want_lengths)
+                    results[k] = run_table(self.replicas[k], table.slice(r0, r1), protein, trimx, use_phase, want_lengths, codon64)
                 else:
                     results[k] = (b"", (np.empty(0, np.int64), np.empty(0, np.int64)) if want_lengths else None)
             except Exception as e:      # re-raised on the caller's thread

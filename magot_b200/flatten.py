@@ -164,7 +164,7 @@ class Flattener(object):
                                   se[src] if total else se[:0], st[src] if total else st[:0], lit_off, pre_len,
                                   suf_len, lit, np.where(valid, ph[safe] if ph.size else 0, 0).astype(np.int8))
 
-    def run(self, seq_type):
+    def run(self, seq_type, codon64=None):
         if seq_type not in ("nucleotide", "protein"):
             if any(t.entries for t in self.tops if not t.genomic):
                 print(seq_type + ' is not valid seq_type. Please specify "protein" or "nucleotide".')
@@ -209,7 +209,7 @@ class Flattener(object):
                 pre.append(b">" + self.names[rid].encode("latin-1") + b"\n")
                 suf.append(b"\n\n" if top.genomic else b"\n")
         tbl = self._table(rec_ids, pre, suf)
-        text, l2 = eng.run_table(tbl, protein=protein, want_lengths=protein)
+        text, l2 = eng.run_table(tbl, protein=protein, want_lengths=protein, codon64=codon64)
         if protein and l2 is not None and (l2[1] < 0)[np.asarray(rec_ids) >= 0].any():
             # Sequence.translate returned None (spliced length <= 2): '>' + name + '\n' + None (genome.py:710)
             raise TypeError("cannot concatenate 'str' and 'NoneType' objects")

@@ -25,6 +25,7 @@ import numpy as np
 
 from . import _lib
 from . import engine
+from . import gencode
 from .py2dict import py2_order, py2_order_after_deepcopy, py2_instance_attr_order
 import weakref
 
@@ -162,6 +163,12 @@ def _codon_table(library):
     return bytes(table)
 
 
+def _codon64_of(genetic_code):
+    """The 64-byte device table of an NCBI code id, None for the standard code (the default kernels' own table)."""
+    code = gencode.check(genetic_code)
+    return None if code == 1 else gencode.codon64(code)
+
+
 _RC_SMALL = {'a': 't', 't': 'a', 'g': 'c', 'c': 'g', 'A': 'T', 'T': 'A', 'G': 'C', 'C': 'G', 'n': 'n', 'N': 'N', '-': '-'}
 
 
@@ -228,20 +235,29 @@ class Sequence(str):
         _lib.check(_lib.lib.mg_revcomp(_device(), ctypes.c_void_p(src.ctypes.data), n, ctypes.c_void_p(out.ctypes.data), None))
         return Sequence(out.tobytes().decode("latin-1"))
 
-    def translate(self, library=None, frame=0, strand='+', trimX=True):
+    def translate(self, library=None, frame=0, strand='+', trimX=True, genetic_code=1):
         """genome.py:795-822 with the reference's frame quirk; returns None when len <= 2 + frame.
-        `library` = a codon -> residue dict (default: the reference's table, NCBI table 1), see _codon_table."""
+        `library` = a codon -> residue dict (default: the reference's table, NCBI table 1), see _codon_table.
+        `genetic_code` = an NCBI table id (magot_b200.gencode); a code other than 1 cannot be combined with `library`."""
+        code = gencode.check(genetic_code)
+        if code != 1:
+            if library is not None:
+                raise ValueError("pass either library= or genetic_code=, not both")
+            library = gencode.library(code)
         return _translate_many([self.encode("latin-1")], frame=frame, strand=strand, trimX=trimX, library=library)[0]
 
-    def get_orfs(self, longest=False, strand='both', from_atg=False):
-        """genome.py:824-851 (the `strand` argument is shadowed in the reference and ignored)."""
+    def get_orfs(self, longest=False, strand='both', from_atg=False, genetic_code=1):
+        """genome.py:824-851 (the `strand` argument is shadowed in the reference and ignored).  `genetic_code`: NCBI table
+        id of the translations, and so of the stops the ORFs are split on; start codons stay the reference's 'M' rule."""
+        code = gencode.check(genetic_code)
+        library = gencode.library(code) if code != 1 else None
         orflist = []
         candidate_list = []
         longest_orf_len = 0
         raw = self.encode("latin-1")
         for frame in (0, 1, 2):
             for st in ('-', '+'):
-                translated_seq = _translate_many([raw], frame=frame, strand=st)[0]
+                translated_seq = _translate_many([raw], frame=frame, strand=st, library=library)[0]
                 if translated_seq:
                     for orf in translated_seq.split('*'):
                         output_orf = ('M' + ''.join(orf.split('M')[1:])) if from_atg else orf
@@ -586,8 +602,10 @@ class ParentAnnotation(object):
             out = [ln for ln, c in zip(physical, is_cds) if not c] + [ln for ln, c in zip(physical, is_cds) if c]
         return '\n'.join(out)
 
-    def get_fasta(self, seq_type="nucleotide", longest=False, genomic=False, name_from='ID'):
-        """genome.py:677-731.  One device pass for this annotation and all its descendants."""
+    def get_fasta(self, seq_type="nucleotide", longest=False, genomic=False, name_from='ID', genetic_code=1):
+        """genome.py:677-731.  One device pass for this annotation and all its descendants.  `genetic_code` (NCBI table id)
+        translates seq_type="protein"; it changes no length, so longest= picks the same records."""
+        codon64 = _codon64_of(genetic_code)
         if genomic is not True and not (len(self.child_list) > 0 and self.annotation_set is not None):
             return ""
         if self.annotation_set is None or self.annotation_set.genome is None:
@@ -595,7 +613,7 @@ class ParentAnnotation(object):
         from .flatten import Flattener
         fl = Flattener(self.annotation_set)
         fl.add_top(self, seq_type=seq_type, longest=longest, genomic=genomic, name_from=name_from)
-        return fl.run(seq_type)
+        return fl.run(seq_type, codon64=codon64)
 
 
 class AnnotationSet(object):
@@ -688,13 +706,15 @@ class AnnotationSet(object):
         read_blast_csv(blast_csv, annotation_set_to_modify=self, hierarchy=hierarchy, source=source,
                        find_truncated_locname=find_truncated_locname)
 
-    def get_fasta(self, feature, seq_type="nucleotide", longest=False, genomic=False):
+    def get_fasta(self, feature, seq_type="nucleotide", longest=False, genomic=False, genetic_code=1):
         """genome.py:578-582: '\\n'.join of every <feature> annotation's fasta, in dict order
         (empty results stay in the list -> blank lines).  All records go through ONE device plan.  A set that still holds
-        the native model of its read_gff call is flattened there (no Python object per feature)."""
+        the native model of its read_gff call is flattened there (no Python object per feature).  `genetic_code` (NCBI
+        table id) translates seq_type="protein"."""
+        codon64 = _codon64_of(genetic_code)
         model = _PENDING.get(self) if _PENDING else None
         if model is not None:
-            text = _native_get_fasta(self, model, feature, seq_type, longest, genomic)
+            text = _native_get_fasta(self, model, feature, seq_type, longest, genomic, codon64)
             if text is not None:
                 return text
         table = getattr(self, feature)
@@ -705,7 +725,7 @@ class AnnotationSet(object):
             if not hasattr(obj, "get_fasta"):
                 raise AttributeError("%s instance has no attribute 'get_fasta'" % obj.__class__.__name__)
             fl.add_top(obj, seq_type=seq_type, longest=longest, genomic=genomic, name_from='ID')
-        return fl.run(seq_type)
+        return fl.run(seq_type, codon64=codon64)
 
 
 _ASET_CLASS_NAMES = frozenset(dir(AnnotationSet))
@@ -727,7 +747,7 @@ def _materialise(annotation_set):
     model.close()
 
 
-def _native_get_fasta(annotation_set, model, feature, seq_type, longest, genomic):
+def _native_get_fasta(annotation_set, model, feature, seq_type, longest, genomic, codon64=None):
     """AnnotationSet.get_fasta on the native model: tops in the set's (Python-2.7 dict, after deepcopy) order, children chosen
     and ordered by mg_gff_flatten, one device plan.  Returns None when the call needs the object model (genomic spans,
     longest=, an unknown table, a model the flattener refuses: the object path then prints / raises like the reference)."""
@@ -758,7 +778,7 @@ def _native_get_fasta(annotation_set, model, feature, seq_type, longest, genomic
         return None
     protein = seq_type == "protein"
     t1 = _time.perf_counter()
-    text, lens = gs._engine().run_table(tbl, protein=protein, want_lengths=protein)
+    text, lens = gs._engine().run_table(tbl, protein=protein, want_lengths=protein, codon64=codon64)
     t2 = _time.perf_counter()
     if protein and lens is not None and ((lens[1] < 0) & (rec_name >= 0)).any():
         # Sequence.translate returned None (spliced length <= 2): '>' + name + '\n' + None (genome.py:710)

@@ -19,6 +19,7 @@ import numpy as np
 
 from . import genome
 from . import engine
+from . import gencode
 
 
 def _truth(s):
@@ -30,8 +31,11 @@ def _truth(s):
     raise NameError("name %r is not defined" % (s,))
 
 
-def gff2fasta(genome_sequence, gff, from_exons="False", seq_type="nucleotide", longest="False", genomic="False"):
-    """genome_tools.py:324-330."""
+def gff2fasta(genome_sequence, gff, from_exons="False", seq_type="nucleotide", longest="False", genomic="False",
+              genetic_code="1"):
+    """genome_tools.py:324-330.  genetic_code=<NCBI table id> (new; default 1, the reference's table) translates
+    seq_type=protein, e.g. genetic_code=5 for insect mitochondria."""
+    code = gencode.check(genetic_code)
     my_genome = genome.Genome(genome_sequence)
     if from_exons == "True":
         # the reference passes features_to_ignore as the *string* "CDS" (substring test) after renaming
@@ -39,7 +43,8 @@ def gff2fasta(genome_sequence, gff, from_exons="False", seq_type="nucleotide", l
         my_genome.read_gff(gff, features_to_ignore="CDS", features_to_replace=[('exon', 'CDS')])
     else:
         my_genome.read_gff(gff)
-    print(my_genome.annotations.get_fasta('gene', seq_type=seq_type, longest=_truth(longest), genomic=_truth(genomic)))
+    print(my_genome.annotations.get_fasta('gene', seq_type=seq_type, longest=_truth(longest), genomic=_truth(genomic),
+                                          genetic_code=code))
 
 
 def convert_gff(gff, input_format, output_format):
@@ -142,8 +147,10 @@ def mask_from_gff(genome_sequence, gff, mask_type="soft", overwrite_softmask="Tr
         g.close()
 
 
-def cds2pep(fasta_file):
-    """genome_tools.py:664-675 -- all records are translated in ONE device launch."""
+def cds2pep(fasta_file, genetic_code="1"):
+    """genome_tools.py:664-675 -- all records are translated in ONE device launch.  genetic_code=<NCBI table id> (new;
+    default 1, the reference's table)."""
+    code = gencode.check(genetic_code)
     headers = []
     seqs = []
     working = []
@@ -166,7 +173,7 @@ def cds2pep(fasta_file):
                     have = True
     seqs.append("".join(working).encode("latin-1"))
     order.append(('s', len(seqs) - 1))
-    peps = genome._translate_many(seqs)
+    peps = genome._translate_many(seqs, library=gencode.library(code) if code != 1 else None)
     out = []
     for kind, idx in order:
         out.append(headers[idx] if kind == 'h' else str(peps[idx]))
@@ -249,18 +256,20 @@ def extract_upstream_downstream(genome_sequence, gff, sequence_length, stream, f
     print("\n".join(output_seqs))
 
 
-def dna2orfs(fasta_location, output_file, from_atg=False, longest=False, min_orf="0"):
+def dna2orfs(fasta_location, output_file, from_atg=False, longest=False, min_orf="0", genetic_code="1"):
     """What genome_tools.py:145-180 intended (the reference's own version raises TypeError because
     GenomeSequence values are plain str): six-frame translation of every contig, split on stops,
     written as '>{seqid}-pos:{orf_start}' records, or one '>{seqid}_longestORF' record per contig.
-    `min_orf` (residues, new) filters short ORFs on the device; "0" reproduces the reference list."""
+    `min_orf` (residues, new) filters short ORFs on the device; "0" reproduces the reference list.
+    `genetic_code` (NCBI table id, new; default 1) sets the residues and the stops, e.g. genetic_code=6 for ciliates."""
+    code = gencode.check(genetic_code)
     from .orfs import contig_orfs
     dna = genome.Genome(fasta_location)
     gs = dna.genome_sequence
     with open(output_file, 'w', encoding="latin-1", newline="\n") as out:
         for seq in gs:
             L = len(gs[seq])
-            recs, aa = contig_orfs(gs, seq, int(min_orf))
+            recs, aa = contig_orfs(gs, seq, int(min_orf), genetic_code=code)
             candidate = None
             longest_orf_len = 0
             for r, orf in zip(recs, aa):

@@ -8,6 +8,7 @@ import ctypes
 import numpy as np
 
 from . import _lib
+from . import gencode
 from ._lib import lib, check
 
 ORF_DTYPE = np.dtype([("contig", np.int32), ("frame", np.int8), ("minus", np.int8), ("pad", np.int16),
@@ -15,12 +16,18 @@ ORF_DTYPE = np.dtype([("contig", np.int32), ("frame", np.int8), ("minus", np.int
 assert ORF_DTYPE.itemsize == ctypes.sizeof(_lib.MgOrf)
 
 
-def sixframe(device_genome, contig_lo, contig_hi, min_aa=0, stream=None):
-    """ORFs of contigs [contig_lo, contig_hi) in reference order.
-    Returns (records: structured array ORF_DTYPE, residues: bytes with the ORFs back to back)."""
+def _codon64(genetic_code):
+    code = gencode.check(genetic_code)
+    return None if code == 1 else gencode.codon64(code)
+
+
+def sixframe(device_genome, contig_lo, contig_hi, min_aa=0, stream=None, genetic_code=1):
+    """ORFs of contigs [contig_lo, contig_hi) in reference order, translated with NCBI table `genetic_code` and split
+    on its stops.  Returns (records: structured array ORF_DTYPE, residues: bytes with the ORFs back to back)."""
+    table = _codon64(genetic_code)
     n_orf, n_bytes = ctypes.c_int64(0), ctypes.c_int64(0)
-    check(lib.mg_sixframe_count(device_genome.handle, contig_lo, contig_hi, int(min_aa),
-                                ctypes.byref(n_orf), ctypes.byref(n_bytes), stream))
+    check(lib.mg_sixframe_count_table(device_genome.handle, contig_lo, contig_hi, int(min_aa), table,
+                                      ctypes.byref(n_orf), ctypes.byref(n_bytes), stream))
     recs = np.zeros(n_orf.value, dtype=ORF_DTYPE)
     aa = np.empty(max(n_bytes.value, 1), dtype=np.uint8)
     check(lib.mg_sixframe_emit(device_genome.handle, ctypes.c_void_p(aa.ctypes.data),
@@ -29,12 +36,13 @@ def sixframe(device_genome, contig_lo, contig_hi, min_aa=0, stream=None):
     return recs, aa[:n_bytes.value].tobytes()
 
 
-def sixframe_list(device_genome, contig_ids, min_aa=0, stream=None):
-    """ORFs of the listed contigs (any order), contig by contig in list order; same return as sixframe()."""
+def sixframe_list(device_genome, contig_ids, min_aa=0, stream=None, genetic_code=1):
+    """ORFs of the listed contigs (any order), contig by contig in list order; same arguments and return as sixframe()."""
+    table = _codon64(genetic_code)
     ids = np.ascontiguousarray(contig_ids, dtype=np.int64)
     n_orf, n_bytes = ctypes.c_int64(0), ctypes.c_int64(0)
-    check(lib.mg_sixframe_count_list(device_genome.handle, ids.size, ctypes.c_void_p(ids.ctypes.data), int(min_aa),
-                                     ctypes.byref(n_orf), ctypes.byref(n_bytes), stream))
+    check(lib.mg_sixframe_count_list_table(device_genome.handle, ids.size, ctypes.c_void_p(ids.ctypes.data), int(min_aa),
+                                           table, ctypes.byref(n_orf), ctypes.byref(n_bytes), stream))
     recs = np.zeros(n_orf.value, dtype=ORF_DTYPE)
     aa = np.empty(max(n_bytes.value, 1), dtype=np.uint8)
     check(lib.mg_sixframe_emit(device_genome.handle, ctypes.c_void_p(aa.ctypes.data),
@@ -55,10 +63,10 @@ def lpt_shards(lengths, n_shards):
     return [sorted(x) for x in shards]
 
 
-def contig_orfs(genome_sequence, seqid, min_aa=0):
+def contig_orfs(genome_sequence, seqid, min_aa=0, genetic_code=1):
     """(records, list of ORF strings) for one contig of a magot_b200.genome.GenomeSequence."""
     ci = genome_sequence.contig_index(seqid)
-    recs, aa = sixframe(genome_sequence._engine().primary, ci, ci + 1, min_aa)
+    recs, aa = sixframe(genome_sequence._engine().primary, ci, ci + 1, min_aa, genetic_code=genetic_code)
     text = aa.decode("latin-1")
     out = [text[int(r["aa_off"]):int(r["aa_off"]) + int(r["len"])] for r in recs]
     return recs, out
