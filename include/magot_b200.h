@@ -225,6 +225,36 @@ int mg_sixframe_count_list_table(mg_genome *g, int64_t n_list, const int64_t *co
 int mg_sixframe_emit(mg_genome *g, uint8_t *aa_out_host, mg_orf *recs_host, void *stream);
 int mg_sixframe_emit_device(mg_genome *g, uint8_t *aa_out_dev, mg_orf *recs_dev, void *stream);
 
+/* ---- start-to-stop ORF calling (ORFfinder / getorf style) on whole contigs, both strands, three TRUE phases.
+ * Phase p reads codons at offsets p, p+3, ... of the strand's 5'->3' sequence (the minus strand is the reverse complement,
+ * phase counted from the contig's end); no frame quirk, no trimX.  Lower case is upper case; a codon with a base outside
+ * A/C/G/T is neither a start nor a stop.  A stop is a codon that codon64 maps to '*'.  Each stop-bounded segment gives at most
+ * one ORF: from its FIRST codon flagged in start64 through the stop that ends it (nested starts are not reported).  A segment
+ * that runs to the contig end without a stop gives a 3' partial ORF, kept only when `partial` != 0.  The protein is the
+ * translation of the start codon up to, not including, the stop, with the first residue always 'M'; ORFs of fewer than
+ * min_aa residues are dropped.
+ * Order: contig in list order, then stream in the order (phase 0 '-'), (0 '+'), (2 '-'), (2 '+'), (1 '-'), (1 '+') -- K4's
+ * stream order, whose frames 1 and 2 read residue classes 2 and 1 -- then position (plus ascending, minus descending).
+ * The count / emit state is the one mg_sixframe_count* uses: a count of either kind replaces the other, and an emit after the
+ * other kind of count fails with MG_ESTATE.                                                                              */
+typedef struct {
+    int32_t contig;
+    int8_t  minus;                /* 1 = minus strand                                                  */
+    int8_t  phase;                /* 0..2, offset of the first codon in the strand's 5'->3' read       */
+    int8_t  flags;                /* bit 0: no stop codon (3' partial)                                 */
+    int8_t  start_codon;          /* 16*b0 + 4*b1 + b2, A=0 C=1 G=2 T=3                                */
+    int64_t lo, hi;               /* 0-based half-open forward-contig interval, stop codon included    */
+    int64_t len;                  /* residues, M included, stop excluded                               */
+    int64_t aa_off;               /* offset of the residues in the emitted buffer                      */
+} mg_orfcall;
+/* codon64: as in mg_sixframe_count_table (NULL = table 1).  start64: 64 flags, byte 16*b0 + 4*b1 + b2 non-zero = start codon
+ * (NULL = ATG only); at least one codon must be flagged and none may be a stop of codon64.  partial: report 3' partials.  */
+int mg_orfcall_count(mg_genome *g, int64_t n_list, const int64_t *contig_ids, int64_t min_aa, const uint8_t *codon64,
+                     const uint8_t *start64, int partial, int64_t *n_orf, int64_t *n_bytes, void *stream);
+/* As mg_sixframe_emit / mg_sixframe_emit_device, for the preceding mg_orfcall_count.                                      */
+int mg_orfcall_emit(mg_genome *g, uint8_t *aa_out_host, mg_orfcall *recs_host, void *stream);
+int mg_orfcall_emit_device(mg_genome *g, uint8_t *aa_out_dev, mg_orfcall *recs_dev, void *stream);
+
 /* ---- host side: native GFF3 / GTF reader + flattener (no GPU work; csrc/mg_gff.cu) ------------------------------------------
  * mg_gff_parse replaces read_gff (genome.py:242-415: line filter, version detection, attribute parsing, ID naming, de-dup,
  * implicit parents, child lists) on interned integer ids; `opts` is the option blob magot_b200/gffnative.py packs (format

@@ -26,6 +26,13 @@ class MgOrf(ctypes.Structure):
                 ("aa_off", ctypes.c_int64)]
 
 
+class MgOrfCall(ctypes.Structure):
+    """mg_orfcall (include/magot_b200.h)."""
+    _fields_ = [("contig", ctypes.c_int32), ("minus", ctypes.c_int8), ("phase", ctypes.c_int8),
+                ("flags", ctypes.c_int8), ("start_codon", ctypes.c_int8), ("lo", ctypes.c_int64),
+                ("hi", ctypes.c_int64), ("len", ctypes.c_int64), ("aa_off", ctypes.c_int64)]
+
+
 if not os.path.isfile(LIB_PATH):
     raise ImportError(
         "magot_b200: %s is missing -- build it with `python -c 'import __graft_entry__ as g; g.build()'` "
@@ -81,6 +88,9 @@ SIGNATURES = {
     "mg_sixframe_count_list_table": (_i32, [_vp, _i64, _vp, _i64, _vp, _pi64, _pi64, _vp]),
     "mg_sixframe_emit": (_i32, [_vp, _vp, _vp, _vp]),
     "mg_sixframe_emit_device": (_i32, [_vp, _vp, _vp, _vp]),
+    "mg_orfcall_count": (_i32, [_vp, _i64, _vp, _i64, _vp, _vp, _i32, _pi64, _pi64, _vp]),
+    "mg_orfcall_emit": (_i32, [_vp, _vp, _vp, _vp]),
+    "mg_orfcall_emit_device": (_i32, [_vp, _vp, _vp, _vp]),
     "mg_stream_sync": (_i32, [_i32, _vp]),
     "mg_copy_d2h_async": (_i32, [_i32, _vp, _vp, _i64, _vp]),
     "mg_tune": (_i32, [ctypes.c_char_p, _i32]),

@@ -81,6 +81,10 @@ struct mg_sixframe_state {
     int64_t aa_cap = 0;
     uint8_t *d_aa4096 = nullptr;                     // residue table of a caller's genetic code (NULL: the genome's standard table)
     uint8_t h_aa4096[4096];                          // its host copy (source of the asynchronous upload)
+    bool orfcall = false;                            // counted by mg_orfcall_count (records in d_calls) instead of mg_sixframe_count*
+    mg_orfcall *d_calls = nullptr;
+    uint8_t *d_start4096 = nullptr;                  // start-codon table of an ORF call (see build_start4096)
+    uint8_t h_start4096[4096];
     std::vector<void *> owned;
     bool counted = false;
     bool force_single = false;
@@ -113,6 +117,18 @@ __global__ void k_six_streams(const uint32_t *__restrict__ packed, const int64_t
     }
     cs_out[i] = cs;
     m_out[i] = m;
+}
+
+// The same for ORF calling: true phases, no trimX.  Stream sidx reads residue class stream_res(sidx), so frame f = sidx >> 1
+// is phase 0, 2, 1 for f = 0, 1, 2 (the quirk's offsets 0, 2, 4 modulo 3).
+__global__ void k_orf_streams(const int64_t *__restrict__ contig_len, const int32_t *__restrict__ cid, int64_t nc,
+                              int32_t *__restrict__ cs_out, int64_t *__restrict__ m_out) {
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i >= nc * 6) return;
+    const int f = (int)(i % 6) >> 1, phase = f == 0 ? 0 : (f == 1 ? 2 : 1);
+    const int64_t L = contig_len[cid[i / 6]];
+    cs_out[i] = phase;
+    m_out[i] = L > phase ? (L - phase) / 3 : 0;
 }
 
 // ---- stop masks of one thread's 48 positions ---------------------------------------------------------
@@ -1313,6 +1329,117 @@ __global__ void __launch_bounds__(AA_THREADS) k_six_aa(const uint32_t *__restric
     }
 }
 
+// ---- ORF calling (mg_orfcall_count): start codon of each stop-bounded segment -----------------------------------------
+// The scan kernels above, run on the true-phase geometry (k_orf_streams) with min_aa as the segment threshold, place every
+// segment of >= min_aa codons (an ORF never outruns its segment).  k_orf_start finds each segment's first start codon,
+// mg_scan_i32 compacts the kept ones, k_orf_place writes their records, and k_six_aa + k_orf_first_m their residues.
+#define ORF_WARPS 8
+#define ORF_SPAN 512                                  // codons a warp tests per step: 16 per lane, one 48-nibble window each
+
+// One WARP per segment, ORF_SPAN codons per step from the segment's first base (srcs: a forward read of either plane), until
+// the first start codon: a segment of n codons costs ceil(n_to_first_start / 512) steps, so a stop-free stretch of any length
+// never holds one lane for long.  kpos = codon offset of the start (-1: none); keep = start found, len - kpos >= min_aa and a
+// real stop ends the segment (or partial).
+__global__ void __launch_bounds__(32 * ORF_WARPS) k_orf_start(const uint32_t *__restrict__ packed, const mg_orf *__restrict__ segs,
+                                                              const int64_t *__restrict__ srcs, int64_t n_seg,
+                                                              const int64_t *__restrict__ contig_len, const uint8_t *__restrict__ start4096,
+                                                              int64_t min_aa, int partial, int32_t *__restrict__ kpos,
+                                                              int32_t *__restrict__ keep) {
+    __shared__ __align__(16) uint8_t s_st[4096];
+    for (int k = threadIdx.x; k < 256; k += blockDim.x)
+        reinterpret_cast<uint4 *>(s_st)[k] = __ldg(reinterpret_cast<const uint4 *>(start4096) + k);
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    const int64_t i = blockIdx.x * (int64_t)ORF_WARPS + (threadIdx.x >> 5);
+    if (i >= n_seg) return;                           // whole warp
+    const int64_t len = segs[i].len, src = srcs[i];
+    int64_t found = -1;
+    for (int64_t base = 0; base < len && found < 0; base += ORF_SPAN) {
+        const int64_t c0 = base + 16 * lane;
+        uint32_t hits = 0;
+        if (c0 < len) {
+            const int64_t g0 = src + 3 * c0;
+            const uint32_t *pp = packed + (g0 >> 3);
+            const uint32_t sh0 = ((uint32_t)g0 & 7u) << 2;
+            uint32_t v[7], n[6];
+#pragma unroll
+            for (int k = 0; k < 7; k++) v[k] = __ldg(pp + k);
+#pragma unroll
+            for (int k = 0; k < 6; k++) n[k] = __funnelshift_r(v[k], v[k + 1], sh0);
+#pragma unroll
+            for (int k = 0; k < 16; k++) {            // codon k = nibbles 3k..3k+2 = bits 12k.. of n[5]:..:n[0]
+                const int bit = 12 * k, ww = bit >> 5, sh = bit & 31;
+                uint32_t idx = n[ww] >> sh;
+                if (sh > 20) idx |= n[ww + 1] << (32 - sh);
+                hits |= (s_st[idx & 0xFFFu] != 0 ? 1u : 0u) << k;
+            }
+            if (len - c0 < 16) hits &= (1u << (len - c0)) - 1u;
+        }
+        const unsigned int any = __ballot_sync(0xffffffffu, hits != 0);
+        if (any) {
+            const int l = __ffs(any) - 1;
+            found = base + 16 * l + __ffs(__shfl_sync(0xffffffffu, hits, l)) - 1;
+        }
+    }
+    if (lane == 0) {
+        const mg_orf o = segs[i];
+        const int f = o.frame, phase = f == 0 ? 0 : (f == 1 ? 2 : 1);
+        const int64_t L = contig_len[o.contig], m = L > phase ? (L - phase) / 3 : 0;
+        const bool stop = o.start + len < m;          // else the segment ends at the contig end
+        kpos[i] = (int32_t)found;
+        keep[i] = found >= 0 && len - found >= min_aa && (stop || partial);
+    }
+}
+
+// thread per segment: the kept ones' records, residue counts and first bases, compacted in segment order
+__global__ void __launch_bounds__(256) k_orf_place(const uint32_t *__restrict__ packed, const mg_orf *__restrict__ segs,
+                                                   const int64_t *__restrict__ srcs, int64_t n_seg, const int64_t *__restrict__ contig_len,
+                                                   const uint8_t *__restrict__ start4096, const int32_t *__restrict__ kpos,
+                                                   const int32_t *__restrict__ keep, const int64_t *__restrict__ slot,
+                                                   mg_orfcall *__restrict__ calls, int32_t *__restrict__ lens, int64_t *__restrict__ srcs_out) {
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i >= n_seg || !keep[i]) return;
+    const mg_orf o = segs[i];
+    const int64_t j = slot[i], k = kpos[i];
+    const int f = o.frame, phase = f == 0 ? 0 : (f == 1 ? 2 : 1);
+    const int64_t L = contig_len[o.contig], m = L > phase ? (L - phase) / 3 : 0;
+    const bool stop = o.start + o.len < m;
+    const int64_t len = o.len - k, g = srcs[i] + 3 * k;
+    const int64_t q = phase + 3 * (o.start + k);      // oriented offset of the start codon
+    const int64_t span = 3 * len + (stop ? 3 : 0);
+    mg_orfcall c;
+    c.contig = o.contig; c.minus = o.minus; c.phase = (int8_t)phase; c.flags = stop ? 0 : 1;
+    c.start_codon = (int8_t)(start4096[mg_ld_nib16(packed, g) & 0xFFFu] - 1);
+    c.lo = o.minus ? L - q - span : q;
+    c.hi = c.lo + span;
+    c.len = len;
+    c.aa_off = 0;
+    calls[j] = c;
+    lens[j] = (int32_t)len;
+    srcs_out[j] = g;
+}
+
+__global__ void __launch_bounds__(256) k_orf_fill_off(int64_t n, const int64_t *__restrict__ aa_off, mg_orfcall *__restrict__ calls) {
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i < n) calls[i].aa_off = aa_off[i];
+}
+
+// after k_six_aa: every ORF's first residue is M, whatever its start codon
+__global__ void __launch_bounds__(256) k_orf_first_m(int64_t n, const int64_t *__restrict__ aa_off, uint8_t *__restrict__ out) {
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i < n) out[aa_off[i]] = 'M';
+}
+
+// Start flags indexed like build_aa4096's residue table (12-bit nibble triplet), by the same decoding: 1 + codon index for a
+// start codon, 0 for any other triplet (a base outside ACGT included).
+static void build_start4096(uint8_t *t, const uint8_t *start64) {
+    uint8_t c64[64];
+    for (int c = 0; c < 64; c++) c64[c] = start64[c] ? (uint8_t)(1 + c) : 0;
+    build_aa4096(t, c64);
+    for (int i = 0; i < 4096; i++)
+        if (t[i] == 'X') t[i] = 0;                   // 'X' (88) is no 1 + codon index (1..64)
+}
+
 // ---- host API -------------------------------------------------------------------------------------------------
 static void six_release(mg_sixframe_state *s) {
     for (void *d : s->owned) cudaFreeAsync(d, s->stream);
@@ -1378,21 +1505,73 @@ static int six_build_stops(mg_genome *g, cudaStream_t st, uint64_t key, const Si
     return MG_OK;
 }
 
-// contigs given as a LIST (any order, e.g. the LPT share of one GPU): ORFs come out contig by contig in list order
-extern "C" int mg_sixframe_count_list_table(mg_genome *g, int64_t n_list, const int64_t *contig_ids, int64_t min_aa,
-                                            const uint8_t *codon64, int64_t *n_orf, int64_t *n_bytes, void *stream) {
+// ORF calling after the scan placed the n_orf segments: their start codons, the kept ones compacted into d_calls / d_len / d_src
+// (which then describe the ORFs, not the segments), s->n_orf = their number.
+static int orf_select(mg_genome *g, mg_sixframe_state *s, const uint8_t *start64, int partial, int64_t min_aa) {
+    cudaStream_t st = s->stream;
+    const int64_t n_seg = s->n_orf;
+    int rc;
+#define TRY(x) do { rc = (x); if (rc) return rc; } while (0)
+    build_start4096(s->h_start4096, start64);
+    TRY(six_alloc(s, &s->d_start4096, 4096));
+    MG_CUDA(cudaMemcpyAsync(s->d_start4096, s->h_start4096, 4096, cudaMemcpyHostToDevice, st));
+    int32_t *d_k = nullptr, *d_keep = nullptr, *d_len = nullptr;
+    int64_t *d_slot = nullptr, *d_src = nullptr;
+    TRY(six_alloc(s, &d_k, n_seg));
+    TRY(six_alloc(s, &d_keep, n_seg));
+    TRY(six_alloc(s, &d_slot, n_seg + 1));
+    k_orf_start<<<(unsigned)((n_seg + ORF_WARPS - 1) / ORF_WARPS), 32 * ORF_WARPS, 0, st>>>(
+        g->d_packed, s->d_recs, s->d_src, n_seg, g->d_contig_len, s->d_start4096, min_aa, partial, d_k, d_keep);
+    MG_LAUNCH_CHECK();
+    const int64_t need = mg_scan_tmp_elems(n_seg) + 2;
+    if (need > s->scan_tmp_cap) {
+        TRY(six_alloc(s, &s->d_scan_tmp, need));
+        s->scan_tmp_cap = need;
+    }
+    TRY(mg_scan_i32(d_keep, d_slot, n_seg, s->d_scan_tmp, s->scan_tmp_cap, st));
+    // records for up to n_seg ORFs, so that k_orf_place runs before the host knows how many are kept
+    TRY(six_alloc(s, &s->d_calls, n_seg));
+    TRY(six_alloc(s, &d_len, n_seg));
+    TRY(six_alloc(s, &d_src, n_seg));
+    k_orf_place<<<(unsigned)((n_seg + 255) / 256), 256, 0, st>>>(g->d_packed, s->d_recs, s->d_src, n_seg, g->d_contig_len, s->d_start4096,
+                                                                  d_k, d_keep, d_slot, s->d_calls, d_len, d_src);
+    MG_LAUNCH_CHECK();
+    MG_CUDA(cudaMemcpyAsync(&s->n_orf, d_slot + n_seg, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    MG_CUDA(cudaStreamSynchronize(st));
+    s->d_len = d_len;
+    s->d_src = d_src;
+#undef TRY
+    return MG_OK;
+}
+
+// the arguments of mg_orfcall_count that the scan does not use (orf == NULL in six_count: the six-frame scan)
+struct OrfSel {
+    const uint8_t *start64;
+    int partial;
+};
+
+static int six_validate(mg_genome *g, int64_t n_list, const int64_t *contig_ids, int64_t min_aa, const uint8_t *codon64) {
     MG_REQUIRE(g != nullptr, "genome handle is NULL");
     MG_REQUIRE(g->finalized, "mg_genome_finalize has not been called");
     MG_REQUIRE(n_list >= 0 && (n_list == 0 || contig_ids != nullptr), "bad contig list");
     MG_REQUIRE(min_aa >= 0, "min_aa must be >= 0");
     for (int64_t i = 0; i < n_list; i++) MG_REQUIRE(contig_ids[i] >= 0 && contig_ids[i] < g->n_contigs, "contig index out of range");
+    // k_six_streams drops a leading codon for trimX when it holds a base outside ACGT, i.e. where the table gives 'X'
+    if (codon64)
+        for (int c = 0; c < 64; c++) MG_REQUIRE(codon64[c] != 'X', "codon64 maps an A/C/G/T codon to 'X'");
+    return MG_OK;
+}
+
+// Both scans.  orf == NULL: the six-frame ORF list (the reference's geometry).  Otherwise ORF calling: the true-phase geometry,
+// then the start-codon selection of the placed segments.  The stop-codon index serves both geometries unchanged: six_masks
+// reads the geometry only to clear the first codon of a trimmed stream, and a codon with a base outside ACGT is never a stop.
+static int six_count(mg_genome *g, int64_t n_list, const int64_t *contig_ids, int64_t min_aa, const uint8_t *codon64,
+                     const OrfSel *orf, int64_t *n_orf, int64_t *n_bytes, void *stream) {
     // the genetic code: its stop set selects the scan kernels, its table the residues
     uint64_t key = SIX_STD_STOPS;
     SixStops ss;
     memset(&ss, 0, sizeof(ss));
     if (codon64) {
-        // k_six_streams drops a leading codon for trimX when it holds a base outside ACGT, i.e. where the table gives 'X'
-        for (int c = 0; c < 64; c++) MG_REQUIRE(codon64[c] != 'X', "codon64 maps an A/C/G/T codon to 'X'");
         key = 0;
         for (int c = 0; c < 64; c++) {
             if (codon64[c] != '*') continue;
@@ -1411,6 +1590,7 @@ extern "C" int mg_sixframe_count_list_table(mg_genome *g, int64_t n_list, const 
     s->stream = st;
     s->min_aa = min_aa;
     s->force_single = g_six_force_single;
+    s->orfcall = orf != nullptr;
     const int64_t nc = n_list;
     std::vector<int32_t> &h_cid = s->h_cid;
     h_cid.resize(nc);
@@ -1450,7 +1630,8 @@ extern "C" int mg_sixframe_count_list_table(mg_genome *g, int64_t n_list, const 
     if (const char *e = getenv("MG_SIX_HIT_CAP")) s->hit_cap = std::max<int64_t>(1, atoll(e));   // tests force the second pass
     TRY(six_alloc(s, &s->d_hits, s->hit_cap));
     MG_CUDA(cudaMemsetAsync(s->d_look, 0, (6 * s->n_tiles + 2) * sizeof(unsigned long long), st));
-    k_six_streams<<<(unsigned)((nc * 6 + 127) / 128), 128, 0, st>>>(g->d_packed, g->d_contig_len, g->d_contig_base, s->d_cid, nc, s->d_cs, s->d_m);
+    if (orf) k_orf_streams<<<(unsigned)((nc * 6 + 127) / 128), 128, 0, st>>>(g->d_contig_len, s->d_cid, nc, s->d_cs, s->d_m);
+    else k_six_streams<<<(unsigned)((nc * 6 + 127) / 128), 128, 0, st>>>(g->d_packed, g->d_contig_len, g->d_contig_base, s->d_cid, nc, s->d_cs, s->d_m);
     MG_LAUNCH_CHECK();
     TRY(six_alloc(s, &s->d_tile_contig, s->n_tiles));
     k_six_tile_contig<<<(unsigned)((s->n_tiles + 255) / 256), 256, 0, st>>>(s->d_tile_base, nc, s->n_tiles, s->d_tile_contig);
@@ -1503,7 +1684,7 @@ extern "C" int mg_sixframe_count_list_table(mg_genome *g, int64_t n_list, const 
         std::vector<int64_t> ids(contig_ids, contig_ids + n_list);
         mg_sixframe_free(g);
         g_six_force_single = true;
-        const int rc2 = mg_sixframe_count_list_table(g, n_list, ids.data(), min_aa, codon64, n_orf, n_bytes, stream);
+        const int rc2 = six_count(g, n_list, ids.data(), min_aa, codon64, orf, n_orf, n_bytes, stream);
         g_six_force_single = false;
         return rc2;
 #define TRY(x) do { rc = (x); if (rc) return rc; } while (0)
@@ -1523,11 +1704,15 @@ extern "C" int mg_sixframe_count_list_table(mg_genome *g, int64_t n_list, const 
                 min_aa, 2 * g->total_bases, nullptr, s->d_cnt_off, s->d_recs, s->d_len, s->d_src, ss);
         }
         MG_LAUNCH_CHECK();
+        if (orf) TRY(orf_select(g, s, orf->start64, orf->partial, min_aa));          // the segments -> the ORFs (s->n_orf may drop to 0)
+    }
+    if (s->n_orf > 0) {
         const int64_t need = mg_scan_tmp_elems(s->n_orf) + 2;
         int64_t *tmp = s->d_scan_tmp;
         if (need > s->scan_tmp_cap) TRY(six_alloc(s, &tmp, need));
         TRY(mg_scan_i32(s->d_len, s->d_aa_off, s->n_orf, tmp, std::max(need, s->scan_tmp_cap), st));
-        k_six_fill_off<<<(unsigned)((s->n_orf + 255) / 256), 256, 0, st>>>(s->n_orf, s->d_aa_off, s->d_recs);
+        if (orf) k_orf_fill_off<<<(unsigned)((s->n_orf + 255) / 256), 256, 0, st>>>(s->n_orf, s->d_aa_off, s->d_calls);
+        else k_six_fill_off<<<(unsigned)((s->n_orf + 255) / 256), 256, 0, st>>>(s->n_orf, s->d_aa_off, s->d_recs);
         MG_LAUNCH_CHECK();
         MG_CUDA(cudaMemcpyAsync(&s->n_bytes, s->d_aa_off + s->n_orf, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
         MG_CUDA(cudaStreamSynchronize(st));
@@ -1542,6 +1727,41 @@ extern "C" int mg_sixframe_count_list_table(mg_genome *g, int64_t n_list, const 
     if (n_orf) *n_orf = s->n_orf;
     if (n_bytes) *n_bytes = s->n_bytes;
     return MG_OK;
+}
+
+// contigs given as a LIST (any order, e.g. the LPT share of one GPU): ORFs come out contig by contig in list order
+extern "C" int mg_sixframe_count_list_table(mg_genome *g, int64_t n_list, const int64_t *contig_ids, int64_t min_aa,
+                                            const uint8_t *codon64, int64_t *n_orf, int64_t *n_bytes, void *stream) {
+    const int rc = six_validate(g, n_list, contig_ids, min_aa, codon64);
+    if (rc) return rc;
+    return six_count(g, n_list, contig_ids, min_aa, codon64, nullptr, n_orf, n_bytes, stream);
+}
+
+extern "C" int mg_orfcall_count(mg_genome *g, int64_t n_list, const int64_t *contig_ids, int64_t min_aa, const uint8_t *codon64,
+                                const uint8_t *start64, int partial, int64_t *n_orf, int64_t *n_bytes, void *stream) {
+    const int rc = six_validate(g, n_list, contig_ids, min_aa, codon64);
+    if (rc) return rc;
+    uint8_t atg[64] = {0};
+    atg[14] = 1;                                                // ATG: 16*0 + 4*3 + 2 (A=0 C=1 G=2 T=3)
+    if (!start64) start64 = atg;
+    uint8_t std64[64];
+    if (!codon64) {                                             // the standard code's stops: TAA TAG TGA
+        memset(std64, 'X', 64);
+        std64[48] = std64[50] = std64[56] = '*';
+    }
+    const uint8_t *stops = codon64 ? codon64 : std64;
+    bool any = false;
+    for (int c = 0; c < 64; c++) {
+        if (!start64[c]) continue;
+        any = true;
+        if (stops[c] == '*') {
+            mg_set_error("start codon %c%c%c is a stop codon of this genetic code", "ACGT"[c >> 4], "ACGT"[(c >> 2) & 3], "ACGT"[c & 3]);
+            return MG_EINVAL;
+        }
+    }
+    MG_REQUIRE(any, "start64 flags no start codon");
+    const OrfSel sel = {start64, partial != 0};
+    return six_count(g, n_list, contig_ids, min_aa, codon64, &sel, n_orf, n_bytes, stream);
 }
 
 extern "C" int mg_sixframe_count_list(mg_genome *g, int64_t n_list, const int64_t *contig_ids, int64_t min_aa, int64_t *n_orf,
@@ -1563,26 +1783,44 @@ extern "C" int mg_sixframe_count(mg_genome *g, int64_t contig_lo, int64_t contig
     return mg_sixframe_count_table(g, contig_lo, contig_hi, min_aa, nullptr, n_orf, n_bytes, stream);
 }
 
-extern "C" int mg_sixframe_emit_device(mg_genome *g, uint8_t *aa_out_dev, mg_orf *recs_dev, void *stream) {
-    MG_REQUIRE(g != nullptr, "genome handle is NULL");
-    if (!g->six || !g->six->counted) { mg_set_error("mg_sixframe_count has not been called"); return MG_ESTATE; }
-    MG_CUDA(cudaSetDevice(g->device));
-    cudaStream_t st = (cudaStream_t)stream;
+// residues of the counted ORFs into out_dev (16-byte aligned); ORF calls get their first residue set to M
+static int six_residues(mg_genome *g, uint8_t *out_dev, cudaStream_t st) {
     mg_sixframe_state *s = g->six;
-    if (aa_out_dev && s->n_bytes > 0) {
-        MG_REQUIRE(((uintptr_t)aa_out_dev & 15) == 0, "aa_out_dev must be 16-byte aligned");
-        k_six_aa<<<(unsigned)s->n_aa_tile, AA_THREADS, 0, st>>>(g->d_packed, s->d_aa_off, s->d_src, s->n_orf, s->d_aa_tile, s->n_bytes,
-                                                                s->d_aa4096 ? s->d_aa4096 : g->d_aa4096, aa_out_dev);
+    if (!out_dev || s->n_bytes <= 0) return MG_OK;
+    MG_REQUIRE(((uintptr_t)out_dev & 15) == 0, "aa_out_dev must be 16-byte aligned");
+    k_six_aa<<<(unsigned)s->n_aa_tile, AA_THREADS, 0, st>>>(g->d_packed, s->d_aa_off, s->d_src, s->n_orf, s->d_aa_tile, s->n_bytes,
+                                                            s->d_aa4096 ? s->d_aa4096 : g->d_aa4096, out_dev);
+    MG_LAUNCH_CHECK();
+    if (s->orfcall) {
+        k_orf_first_m<<<(unsigned)((s->n_orf + 255) / 256), 256, 0, st>>>(s->n_orf, s->d_aa_off, out_dev);
         MG_LAUNCH_CHECK();
     }
-    if (recs_dev && s->n_orf > 0)
-        MG_CUDA(cudaMemcpyAsync(recs_dev, s->d_recs, s->n_orf * sizeof(mg_orf), cudaMemcpyDeviceToDevice, st));
     return MG_OK;
 }
 
-extern "C" int mg_sixframe_emit(mg_genome *g, uint8_t *aa_out_host, mg_orf *recs_host, void *stream) {
+static int six_emit_device(mg_genome *g, bool orfcall, uint8_t *aa_out_dev, void *recs_dev, void *stream) {
     MG_REQUIRE(g != nullptr, "genome handle is NULL");
-    if (!g->six || !g->six->counted) { mg_set_error("mg_sixframe_count has not been called"); return MG_ESTATE; }
+    if (!g->six || !g->six->counted || g->six->orfcall != orfcall) {
+        mg_set_error(orfcall ? "mg_orfcall_count has not been called" : "mg_sixframe_count has not been called");
+        return MG_ESTATE;
+    }
+    MG_CUDA(cudaSetDevice(g->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    mg_sixframe_state *s = g->six;
+    const int rc = six_residues(g, aa_out_dev, st);
+    if (rc) return rc;
+    if (recs_dev && s->n_orf > 0)
+        MG_CUDA(cudaMemcpyAsync(recs_dev, orfcall ? (void *)s->d_calls : (void *)s->d_recs,
+                                s->n_orf * (orfcall ? sizeof(mg_orfcall) : sizeof(mg_orf)), cudaMemcpyDeviceToDevice, st));
+    return MG_OK;
+}
+
+static int six_emit_host(mg_genome *g, bool orfcall, uint8_t *aa_out_host, void *recs_host, void *stream) {
+    MG_REQUIRE(g != nullptr, "genome handle is NULL");
+    if (!g->six || !g->six->counted || g->six->orfcall != orfcall) {
+        mg_set_error(orfcall ? "mg_orfcall_count has not been called" : "mg_sixframe_count has not been called");
+        return MG_ESTATE;
+    }
     MG_CUDA(cudaSetDevice(g->device));
     cudaStream_t st = (cudaStream_t)stream;
     mg_sixframe_state *s = g->six;
@@ -1595,12 +1833,29 @@ extern "C" int mg_sixframe_emit(mg_genome *g, uint8_t *aa_out_host, mg_orf *recs
             MG_CUDA(cudaMalloc(&s->d_aa, need));
             s->aa_cap = need;
         }
-        int rc = mg_sixframe_emit_device(g, s->d_aa, nullptr, stream);
+        int rc = six_residues(g, s->d_aa, st);
         if (rc) return rc;
         MG_CUDA(cudaMemcpyAsync(aa_out_host, s->d_aa, s->n_bytes, cudaMemcpyDeviceToHost, st));
     }
     if (recs_host && s->n_orf > 0)
-        MG_CUDA(cudaMemcpyAsync(recs_host, s->d_recs, s->n_orf * sizeof(mg_orf), cudaMemcpyDeviceToHost, st));
+        MG_CUDA(cudaMemcpyAsync(recs_host, orfcall ? (void *)s->d_calls : (void *)s->d_recs,
+                                s->n_orf * (orfcall ? sizeof(mg_orfcall) : sizeof(mg_orf)), cudaMemcpyDeviceToHost, st));
     MG_CUDA(cudaStreamSynchronize(st));
     return MG_OK;
+}
+
+extern "C" int mg_sixframe_emit_device(mg_genome *g, uint8_t *aa_out_dev, mg_orf *recs_dev, void *stream) {
+    return six_emit_device(g, false, aa_out_dev, recs_dev, stream);
+}
+
+extern "C" int mg_sixframe_emit(mg_genome *g, uint8_t *aa_out_host, mg_orf *recs_host, void *stream) {
+    return six_emit_host(g, false, aa_out_host, recs_host, stream);
+}
+
+extern "C" int mg_orfcall_emit_device(mg_genome *g, uint8_t *aa_out_dev, mg_orfcall *recs_dev, void *stream) {
+    return six_emit_device(g, true, aa_out_dev, recs_dev, stream);
+}
+
+extern "C" int mg_orfcall_emit(mg_genome *g, uint8_t *aa_out_host, mg_orfcall *recs_host, void *stream) {
+    return six_emit_host(g, true, aa_out_host, recs_host, stream);
 }

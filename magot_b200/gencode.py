@@ -3,6 +3,7 @@
 `codon64(n)` is the 64-byte table the C ABI takes (mg_plan_set_codon_table, mg_sixframe_count_table,
 mg_translate_ascii_table): byte 16*b0 + 4*b1 + b2 (A=0 C=1 G=2 T=3) is the residue of codon b0 b1 b2, '*' a stop.
 `library(n)` is the same code as a reference-style codon dict, for Sequence.translate(library=...).
+`start64(codons, n)` is the 64-byte start-codon flag table mg_orfcall_count takes.
 
 Tables 27, 28 and 31 read TAA/TAG/TGA as stop or sense depending on context, which a codon table cannot
 express; they, 32 and the unassigned ids are refused.
@@ -69,3 +70,24 @@ def codon64(genetic_code):
 def stops(genetic_code):
     """The code's stop codons, sorted."""
     return sorted(c for c, a in library(genetic_code).items() if a == "*")
+
+
+def start64(codons, genetic_code=1):
+    """Start codons (e.g. ("ATG", "GTG")) as the C ABI's 64 flags, byte 16*b0 + 4*b1 + b2 (A=0 C=1 G=2 T=3) = 1 for a start.
+    ValueError for an empty list, a codon that is not three letters of A/C/G/T (either case) or a stop of the code."""
+    code = check(genetic_code)
+    if isinstance(codons, str):
+        codons = [codons]
+    codons = list(codons)
+    if not codons:
+        raise ValueError("no start codon given")
+    lib = library(code)
+    flags = bytearray(64)
+    for c in codons:
+        u = str(c).upper()
+        if len(u) != 3 or any(b not in "ACGT" for b in u):
+            raise ValueError("start codon %r is not three letters of A/C/G/T" % (c,))
+        if lib[u] == "*":
+            raise ValueError("start codon %s is a stop codon of genetic code %d" % (u, code))
+        flags["ACGT".index(u[0]) * 16 + "ACGT".index(u[1]) * 4 + "ACGT".index(u[2])] = 1
+    return bytes(flags)

@@ -10,7 +10,8 @@ Kept (file:line in genome_tools.py): gff2fasta :324, cds2pep :664, coords2fasta 
 get_seq_from_fasta :483, exclude_from_fasta :377, extract_upstream_downstream :457,
 blast_csv2fasta :265, exonerate2fasta :274, mask_from_gff :394, convert_gff :527,
 dna2orfs :145 (the reference's version cannot run -- it calls str.translate with keyword
-arguments -- this one does what it intended, on the device).  The dispatcher (main :25-45)
+arguments -- this one does what it intended, on the device).  New: call_orfs, start-to-stop
+ORF calling with genome coordinates (GFF3, protein or CDS nucleotide output).  The dispatcher (main :25-45)
 keeps the grammar but looks the function up in a table instead of eval()-ing a string.
 """
 import sys
@@ -290,9 +291,79 @@ def dna2orfs(fasta_location, output_file, from_atg=False, longest=False, min_orf
                 out.write(candidate)        # TypeError when the contig has no ORF at all (IndexError in the reference)
 
 
+ORF_FORMATS = ("gff3", "protein", "nucleotide")
+
+
+def _orf_order(contig_order, recs):
+    """Permutation of mg_orfcall records into call_orfs' order: contigs as listed in contig_order, then lo, '+' before '-',
+    then phase (stable)."""
+    rank = {int(c): i for i, c in enumerate(contig_order)}
+    key = np.array([rank[int(c)] for c in recs["contig"]], dtype=np.int64)
+    return np.lexsort((recs["phase"], recs["minus"], recs["lo"], key))
+
+
+def _orf_lines(names, recs, out_format, seqs=None):
+    """Output lines of call_orfs for records already in its order.  names[contig] = seqid; seqs[i] = the protein or
+    nucleotide text of recs[i] (not read for gff3).  ORF n (1-based) of a contig is <seqid>_orf<n>."""
+    lines = ["##gff-version 3"] if out_format == "gff3" else []
+    count = {}
+    for i, r in enumerate(recs):
+        c = int(r["contig"])
+        count[c] = count.get(c, 0) + 1
+        seqid = names[c]
+        oid = "%s_orf%d" % (seqid, count[c])
+        strand = "-" if r["minus"] else "+"
+        lo, hi = int(r["lo"]), int(r["hi"])
+        if out_format == "gff3":
+            sc = int(r["start_codon"])
+            attrs = "ID=%s;start_codon=%s" % (oid, "ACGT"[sc >> 4] + "ACGT"[(sc >> 2) & 3] + "ACGT"[sc & 3])
+            if int(r["flags"]) & 1:
+                attrs += ";partial=3prime"
+            lines.append("\t".join((seqid, "magot_b200", "ORF", str(lo + 1), str(hi), ".", strand, ".", attrs)))
+        else:
+            lines.append(">%s %s:%d-%d(%s)" % (oid, seqid, lo + 1, hi, strand))
+            lines.append(seqs[i])
+    return lines
+
+
+def call_orfs(fasta, min_orf="100", genetic_code="1", start_codons="ATG", partial="False", out_format="gff3"):
+    """Start-to-stop ORFs of every contig (new; NCBI ORFfinder / EMBOSS getorf style): both strands, the three true phases,
+    from the first start codon of each stop-bounded stretch through the stop, at least `min_orf` residues (M included, stop
+    excluded).  start_codons: comma-separated codons (default ATG); partial=True adds ORFs that run off the contig end
+    without a stop (partial=3prime).  out_format: gff3 (1-based inclusive coordinates), protein (first residue M) or
+    nucleotide (start through stop codon, reverse-complemented on '-').  Contigs in the order dna2orfs visits them; within a
+    contig by start coordinate, '+' before '-', then phase; IDs <seqid>_orf<n>."""
+    from . import orfs
+    code = gencode.check(genetic_code)
+    if out_format not in ORF_FORMATS:
+        raise ValueError("out_format %r is not one of %s" % (out_format, ", ".join(ORF_FORMATS)))
+    codons = start_codons.split(",") if isinstance(start_codons, str) else list(start_codons)
+    gencode.start64(codons, code)                            # ValueError before any device work
+    gs = genome.Genome(fasta).genome_sequence
+    order = [gs.contig_index(seq) for seq in gs]
+    names = {ci: seq for ci, seq in zip(order, gs)}
+    recs, aa = orfs.call_orfs(gs._engine().primary, order, int(min_orf), genetic_code=code, start_codons=codons,
+                              partial=_truth(partial))
+    recs = recs[_orf_order(order, recs)]
+    seqs = None
+    if out_format == "protein":
+        text = aa.decode("latin-1")
+        seqs = [text[int(r["aa_off"]):int(r["aa_off"]) + int(r["len"])] for r in recs]
+    elif out_format == "nucleotide" and recs.size:
+        R = recs.size
+        zero = np.zeros(R, dtype=np.int32)
+        tbl = engine.RecordTable(np.arange(R + 1), recs["contig"].astype(np.int32), recs["lo"] + 1, recs["hi"],
+                                 recs["minus"].astype(np.int8), np.zeros(R, dtype=np.int64), zero, zero, np.zeros(0, dtype=np.uint8))
+        text, (nuc_len, _) = gs._engine().run_table(tbl, want_lengths=True)
+        off = np.concatenate(([0], np.cumsum(nuc_len)))
+        seqs = [text[off[k]:off[k + 1]].decode("latin-1") for k in range(R)]
+    lines = _orf_lines(names, recs, out_format, seqs)
+    sys.stdout.write("\n".join(lines) + "\n" if lines else "")
+
+
 FUNCTIONS = {f.__name__: f for f in (gff2fasta, cds2pep, coords2fasta, get_seq_from_fasta, exclude_from_fasta,
                                      extract_upstream_downstream, dna2orfs, blast_csv2fasta, exonerate2fasta, mask_from_gff,
-                                     convert_gff)}
+                                     convert_gff, call_orfs)}
 
 
 def help_func():

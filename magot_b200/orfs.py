@@ -2,6 +2,7 @@
 
 Replaces Sequence.get_orfs (genome.py:824-851) applied to whole contigs -- what dna2orfs
 (genome_tools.py:145-180) intended -- with an optional minimum length (0 == reference).
+call_orfs() is start-to-stop ORF calling on the same scan (mg_orfcall_count): true phases, genome coordinates.
 """
 import ctypes
 
@@ -14,6 +15,11 @@ from ._lib import lib, check
 ORF_DTYPE = np.dtype([("contig", np.int32), ("frame", np.int8), ("minus", np.int8), ("pad", np.int16),
                       ("start", np.int64), ("len", np.int64), ("aa_off", np.int64)])
 assert ORF_DTYPE.itemsize == ctypes.sizeof(_lib.MgOrf)
+
+ORFCALL_DTYPE = np.dtype([("contig", np.int32), ("minus", np.int8), ("phase", np.int8), ("flags", np.int8),
+                          ("start_codon", np.int8), ("lo", np.int64), ("hi", np.int64), ("len", np.int64),
+                          ("aa_off", np.int64)])
+assert ORFCALL_DTYPE.itemsize == ctypes.sizeof(_lib.MgOrfCall)
 
 
 def _codon64(genetic_code):
@@ -47,6 +53,25 @@ def sixframe_list(device_genome, contig_ids, min_aa=0, stream=None, genetic_code
     aa = np.empty(max(n_bytes.value, 1), dtype=np.uint8)
     check(lib.mg_sixframe_emit(device_genome.handle, ctypes.c_void_p(aa.ctypes.data),
                                ctypes.c_void_p(recs.ctypes.data) if n_orf.value else None, stream))
+    check(lib.mg_stream_sync(device_genome.device, stream))
+    return recs, aa[:n_bytes.value].tobytes()
+
+
+def call_orfs(device_genome, contig_ids, min_aa=100, genetic_code=1, start_codons=("ATG",), partial=False, stream=None):
+    """Start-to-stop ORFs of the listed contigs on both strands and all three phases (include/magot_b200.h, mg_orfcall):
+    each stop-bounded stretch gives the ORF from its first start codon through the stop, of >= min_aa residues ('M'
+    included, stop excluded); partial=True adds those that reach the contig end without a stop (flags bit 0).
+    Returns (records: structured array ORFCALL_DTYPE in the ABI's order, residues: bytes with the proteins back to back)."""
+    table = _codon64(genetic_code)
+    starts = gencode.start64(start_codons, genetic_code)
+    ids = np.ascontiguousarray(contig_ids, dtype=np.int64)
+    n_orf, n_bytes = ctypes.c_int64(0), ctypes.c_int64(0)
+    check(lib.mg_orfcall_count(device_genome.handle, ids.size, ctypes.c_void_p(ids.ctypes.data), int(min_aa), table, starts,
+                               1 if partial else 0, ctypes.byref(n_orf), ctypes.byref(n_bytes), stream))
+    recs = np.zeros(n_orf.value, dtype=ORFCALL_DTYPE)
+    aa = np.empty(max(n_bytes.value, 1), dtype=np.uint8)
+    check(lib.mg_orfcall_emit(device_genome.handle, ctypes.c_void_p(aa.ctypes.data),
+                              ctypes.c_void_p(recs.ctypes.data) if n_orf.value else None, stream))
     check(lib.mg_stream_sync(device_genome.device, stream))
     return recs, aa[:n_bytes.value].tobytes()
 
