@@ -64,7 +64,11 @@ int mg_genome_pack_fasta(mg_genome *g, int64_t contig, const uint8_t *raw, int64
  * the contig lengths (body bytes minus line ends, genome.py:875) are known before mg_genome_create without a Python pass over
  * the sequence bytes.  Threaded; no GPU work.                                                                             */
 int mg_count_line_ends(const uint8_t *data, int64_t n, int64_t n_ranges, const int64_t *lo, const int64_t *hi, int64_t *out);
-/* Sort the exception list and make the genome usable by every call below.                   */
+/* Sort the exception list and make the genome usable by every call below.
+ * Every call that can change the bases -- mg_genome_pack*, mg_genome_finalize, mg_genome_mask -- makes the results of an
+ * earlier count (mg_sixframe_count*, mg_orfcall_count) or plan prepare (mg_plan_prepare*) stale: their emits then fail with
+ * MG_ESTATE until the count or prepare is repeated.  A CUDA graph replays what it captured without these host checks, so a
+ * graph captured before such a call must not be replayed after it.                                                        */
 int mg_genome_finalize(mg_genome *g, int64_t *n_exceptions_out);
 int mg_genome_destroy(mg_genome *g);
 int64_t mg_genome_bytes(const mg_genome *g);          /* device bytes held by the handle      */
@@ -78,7 +82,8 @@ int mg_genome_fetch(mg_genome *g, int64_t contig, int64_t lo, int64_t hi, int mi
  * Intervals are 0-based half-open [lo, hi) on `contig`, already clamped like the Python slice
  * [start-1:stop]; they may overlap.  hard = 0: lower-case them (soft mask); hard = 1: replace them
  * by 'N'.  upper_first != 0 upper-cases the whole genome before (overwrite_softmask, :403-404).
- * Both planes and the exception list are updated; the handle stays finalized.                 */
+ * Both planes and the exception list are updated; the handle stays finalized.  Counts and prepared plans of this genome
+ * become stale (see mg_genome_finalize).  On an argument error (MG_EINVAL) the genome is left unchanged.                */
 int mg_genome_mask(mg_genome *g, int64_t n_intervals, const int32_t *contig, const int64_t *lo, const int64_t *hi,
                    int hard, int upper_first, void *stream);
 
@@ -121,7 +126,10 @@ int mg_plan_destroy(mg_plan *p);
 
 /* Clamp, measure and scan (warp/block prefix sums on the device).  Outputs (host, may be NULL):
  * total bytes of the nucleotide text and of the protein text (literals included).
- * Must be called once before any emit; everything stays on the device.                      */
+ * Must be called once before any emit; everything stays on the device.  The record pass reads the genome (trimX of the first
+ * codon) and the emits read it again, so a prepare holds for the genome as it was: after a pack, finalize or mask of the
+ * plan's genome, mg_plan_prepare_prot_async, mg_plan_totals, mg_plan_lengths and every mg_emit_* of the plan fail with
+ * MG_ESTATE until it is prepared again.                                                                              */
 int mg_plan_prepare(mg_plan *p, int prot_flags, int64_t *nuc_total, int64_t *prot_total, void *stream);
 /* The same without the host round trip, for callers that already hold buffers: nuc_capacity / prot_capacity are the sizes
  * the caller's nucleotide / protein output buffers can take (an upper bound is sum(max(0, end-start+1)) + framing bytes,
@@ -221,7 +229,8 @@ int mg_sixframe_count_list_table(mg_genome *g, int64_t n_list, const int64_t *co
 /* Emits the result of the preceding mg_sixframe_count on this genome handle.  aa_out_host gets
  * n_bytes residues (ORFs back to back, no separators), recs_host n_orf records.  Either may
  * be NULL.  *_device variant leaves the residues in `aa_out_dev` (16-byte aligned, n_bytes
- * rounded up to 16).                                                                          */
+ * rounded up to 16).  The residues are read from the genome at emit time: after a pack, finalize
+ * or mask of the genome since the count, the emit fails with MG_ESTATE (count again).         */
 int mg_sixframe_emit(mg_genome *g, uint8_t *aa_out_host, mg_orf *recs_host, void *stream);
 int mg_sixframe_emit_device(mg_genome *g, uint8_t *aa_out_dev, mg_orf *recs_dev, void *stream);
 
@@ -251,7 +260,7 @@ typedef struct {
  * (NULL = ATG only); at least one codon must be flagged and none may be a stop of codon64.  partial: report 3' partials.  */
 int mg_orfcall_count(mg_genome *g, int64_t n_list, const int64_t *contig_ids, int64_t min_aa, const uint8_t *codon64,
                      const uint8_t *start64, int partial, int64_t *n_orf, int64_t *n_bytes, void *stream);
-/* As mg_sixframe_emit / mg_sixframe_emit_device, for the preceding mg_orfcall_count.                                      */
+/* As mg_sixframe_emit / mg_sixframe_emit_device, for the preceding mg_orfcall_count (MG_ESTATE after a genome change too). */
 int mg_orfcall_emit(mg_genome *g, uint8_t *aa_out_host, mg_orfcall *recs_host, void *stream);
 int mg_orfcall_emit_device(mg_genome *g, uint8_t *aa_out_dev, mg_orfcall *recs_dev, void *stream);
 

@@ -80,6 +80,8 @@ struct mg_genome {
     std::vector<int64_t> h_exc_pos;           // collected per chunk
     std::vector<uint8_t> h_exc_byte;
     bool finalized = false;
+    uint64_t generation = 0;                  // bumped by every call that can change the bases (pack*, finalize, mask): a count or
+                                              // plan prepared at another generation cannot be emitted (MG_ESTATE)
     uint8_t *d_stage = nullptr;               // H2D staging for pack / fetch
     int64_t stage_cap = 0;
     uint8_t *d_raw = nullptr;                 // raw FASTA body chunk (mg_genome_pack_fasta)
@@ -137,6 +139,7 @@ struct mg_plan {
     bool totals_known = false;                    // false between mg_plan_prepare_async and mg_plan_totals
     int prot_flags = 0;
     bool prepared = false;
+    uint64_t generation = 0;                      // g->generation at the last prepare: K1 read the bases then, the emits read them again
     bool prot_ready = false;                      // false between mg_plan_prepare_async(MG_PROT_DEFER) and mg_plan_prepare_prot_async
     unsigned long long *rec_tmp = nullptr;        // look-back words / tile table of the deferred record pass
     int64_t rec_tmp_words = 0;
@@ -165,6 +168,7 @@ struct mg_plan {
 
 // internal cross-file helpers
 void build_aa4096(uint8_t *t, const uint8_t *codon64);   // nibble-triplet -> residue table from a codon64 table (NULL = standard code)
+int mg_plan_check_prepared(const mg_plan *p);         // MG_ESTATE unless p was prepared and its genome has not changed since
 int mg_scan_i32(const int32_t *d_in, int64_t *d_out, int64_t n, int64_t *d_tmp, int64_t tmp_cap, cudaStream_t st);
 int64_t mg_scan_tmp_elems(int64_t n);
 int mg_ensure_stage(mg_genome *g, int64_t bytes);

@@ -822,7 +822,7 @@ static ProtArgs prot_args(const mg_plan *p, uint8_t *out_dev) {
 
 extern "C" int mg_emit_nuc_device(mg_plan *p, uint8_t *out_dev, void *stream) {
     MG_REQUIRE(p != nullptr, "plan handle is NULL");
-    if (!p->prepared) { mg_set_error("mg_plan_prepare has not been called"); return MG_ESTATE; }
+    if (const int rc0 = mg_plan_check_prepared(p)) return rc0;
     if (p->nuc_total == 0) return MG_OK;
     MG_REQUIRE(out_dev != nullptr && ((uintptr_t)out_dev & 31) == 0, "out_dev must be a 32-byte aligned device pointer");
     MG_CUDA(cudaSetDevice(p->device));
@@ -837,7 +837,7 @@ extern "C" int mg_emit_nuc_device(mg_plan *p, uint8_t *out_dev, void *stream) {
 
 extern "C" int mg_emit_prot_device(mg_plan *p, uint8_t *out_dev, void *stream) {
     MG_REQUIRE(p != nullptr, "plan handle is NULL");
-    if (!p->prepared) { mg_set_error("mg_plan_prepare has not been called"); return MG_ESTATE; }
+    if (const int rc0 = mg_plan_check_prepared(p)) return rc0;
     if (!p->prot_ready) { mg_set_error("the record pass was deferred (MG_PROT_DEFER): call mg_plan_prepare_prot_async first"); return MG_ESTATE; }
     if (p->prot_total == 0) return MG_OK;
     MG_REQUIRE(out_dev != nullptr && ((uintptr_t)out_dev & 15) == 0, "out_dev must be a 16-byte aligned device pointer");
@@ -855,7 +855,7 @@ static int g_fuse = 1;
 void mg_set_fuse(int v) { g_fuse = v; }
 extern "C" int mg_emit_nuc_prot_device(mg_plan *p, uint8_t *nuc_out_dev, uint8_t *prot_out_dev, void *stream) {
     MG_REQUIRE(p != nullptr, "plan handle is NULL");
-    if (!p->prepared) { mg_set_error("mg_plan_prepare has not been called"); return MG_ESTATE; }
+    if (const int rc0 = mg_plan_check_prepared(p)) return rc0;
     if (!p->prot_ready) { mg_set_error("the record pass was deferred (MG_PROT_DEFER): call mg_plan_prepare_prot_async first"); return MG_ESTATE; }
     if (p->nuc_total == 0) return mg_emit_prot_device(p, prot_out_dev, stream);       // no nucleotide tile: framing-only protein text
     if (p->prot_total == 0) return mg_emit_nuc_device(p, nuc_out_dev, stream);
@@ -950,11 +950,11 @@ __global__ void __launch_bounds__(NUC_THREADS, NUC_MINB) k_emit_multi(const __gr
 // prepared (mg_plan_prepare or mg_plan_prepare_async, the latter on this stream or joined with it) and belong to one genome.
 extern "C" int mg_emit_products_device(mg_plan *pa, uint8_t *out_a, mg_plan *pb, uint8_t *out_b_nuc, uint8_t *out_b_prot, void *stream) {
     const bool ja = pa && out_a && pa->nuc_total > 0, jb = pb && out_b_nuc && pb->nuc_total > 0, jc = pb && out_b_prot && pb->prot_total > 0;
-    if (jc && !pb->prot_ready) { mg_set_error("the record pass was deferred (MG_PROT_DEFER): call mg_plan_prepare_prot_async first"); return MG_ESTATE; }
     MG_REQUIRE(!out_a || pa, "out_a given without a plan");
     MG_REQUIRE((!out_b_nuc && !out_b_prot) || pb, "out_b given without a plan");
-    if (pa && out_a && !pa->prepared) { mg_set_error("mg_plan_prepare has not been called"); return MG_ESTATE; }
-    if (pb && (out_b_nuc || out_b_prot) && !pb->prepared) { mg_set_error("mg_plan_prepare has not been called"); return MG_ESTATE; }
+    if (pa && out_a) { if (const int rc0 = mg_plan_check_prepared(pa)) return rc0; }
+    if (pb && (out_b_nuc || out_b_prot)) { if (const int rc0 = mg_plan_check_prepared(pb)) return rc0; }
+    if (jc && !pb->prot_ready) { mg_set_error("the record pass was deferred (MG_PROT_DEFER): call mg_plan_prepare_prot_async first"); return MG_ESTATE; }
     if (!ja && !jb && !jc) return MG_OK;
     MG_REQUIRE(!ja || ((uintptr_t)out_a & 31) == 0, "out_a must be a 32-byte aligned device pointer");
     MG_REQUIRE(!jb || ((uintptr_t)out_b_nuc & 31) == 0, "out_b_nuc must be a 32-byte aligned device pointer");
@@ -1030,7 +1030,7 @@ static int copy_text_to_host(mg_plan *p, uint8_t *out_host, const uint8_t *d_src
 
 extern "C" int mg_emit_nuc_host(mg_plan *p, uint8_t *out_host, void *stream) {
     MG_REQUIRE(p != nullptr, "plan handle is NULL");
-    if (!p->prepared) { mg_set_error("mg_plan_prepare has not been called"); return MG_ESTATE; }
+    if (const int rc0 = mg_plan_check_prepared(p)) return rc0;
     if (!p->totals_known) { int rc0 = mg_plan_totals(p, nullptr, nullptr, stream); if (rc0) return rc0; }
     if (p->nuc_total == 0) return MG_OK;
     MG_REQUIRE(out_host != nullptr, "out_host is NULL");
@@ -1046,7 +1046,7 @@ extern "C" int mg_emit_nuc_host(mg_plan *p, uint8_t *out_host, void *stream) {
 // K23 into two library-owned device buffers, then both texts to the host (stream-ordered; mg_stream_sync before reading)
 extern "C" int mg_emit_nuc_prot_host(mg_plan *p, uint8_t *nuc_out_host, uint8_t *prot_out_host, void *stream) {
     MG_REQUIRE(p != nullptr, "plan handle is NULL");
-    if (!p->prepared) { mg_set_error("mg_plan_prepare has not been called"); return MG_ESTATE; }
+    if (const int rc0 = mg_plan_check_prepared(p)) return rc0;
     if (!p->totals_known) { int rc0 = mg_plan_totals(p, nullptr, nullptr, stream); if (rc0) return rc0; }
     if (p->nuc_total == 0 && p->prot_total == 0) return MG_OK;
     MG_REQUIRE((nuc_out_host != nullptr || p->nuc_total == 0) && (prot_out_host != nullptr || p->prot_total == 0), "output buffer is NULL");
@@ -1068,7 +1068,7 @@ extern "C" int mg_emit_products_host(mg_plan *pa, uint8_t *out_a_host, mg_plan *
     cudaStream_t st = (cudaStream_t)stream;
     uint8_t *da = nullptr, *dbn = nullptr, *dbp = nullptr;
     if (pa && out_a_host) {
-        if (!pa->prepared) { mg_set_error("mg_plan_prepare has not been called"); return MG_ESTATE; }
+        if (const int rc0 = mg_plan_check_prepared(pa)) return rc0;
         if (!pa->totals_known) { int rc0 = mg_plan_totals(pa, nullptr, nullptr, stream); if (rc0) return rc0; }
         MG_CUDA(cudaSetDevice(pa->device));
         int rc = ensure_out(pa, (pa->nuc_total + 31) / 32 * 32 + 32, st);
@@ -1077,7 +1077,7 @@ extern "C" int mg_emit_products_host(mg_plan *pa, uint8_t *out_a_host, mg_plan *
     }
     int64_t nn = 0;
     if (pb && (out_b_nuc_host || out_b_prot_host)) {
-        if (!pb->prepared) { mg_set_error("mg_plan_prepare has not been called"); return MG_ESTATE; }
+        if (const int rc0 = mg_plan_check_prepared(pb)) return rc0;
         if (!pb->totals_known) { int rc0 = mg_plan_totals(pb, nullptr, nullptr, stream); if (rc0) return rc0; }
         MG_CUDA(cudaSetDevice(pb->device));
         nn = out_b_nuc_host ? (pb->nuc_total + 31) / 32 * 32 : 0;
@@ -1096,7 +1096,7 @@ extern "C" int mg_emit_products_host(mg_plan *pa, uint8_t *out_a_host, mg_plan *
 
 extern "C" int mg_emit_prot_host(mg_plan *p, uint8_t *out_host, void *stream) {
     MG_REQUIRE(p != nullptr, "plan handle is NULL");
-    if (!p->prepared) { mg_set_error("mg_plan_prepare has not been called"); return MG_ESTATE; }
+    if (const int rc0 = mg_plan_check_prepared(p)) return rc0;
     if (!p->totals_known) { int rc0 = mg_plan_totals(p, nullptr, nullptr, stream); if (rc0) return rc0; }
     if (p->prot_total == 0) return MG_OK;
     MG_REQUIRE(out_host != nullptr, "out_host is NULL");

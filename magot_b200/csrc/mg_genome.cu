@@ -310,6 +310,7 @@ extern "C" int mg_genome_pack_device(mg_genome *g, int64_t contig, int64_t offse
     MG_REQUIRE(((uintptr_t)ascii_dev & 15) == 0, "device text must be 16-byte aligned");
     MG_CUDA(cudaSetDevice(g->device));
     g->finalized = false;
+    g->generation++;
     g->stops_valid = g->stops_alt_valid = false;
     if (n == 0) return MG_OK;
     return pack_device_chunk(g, g->h_contig_base[contig] + offset, ascii_dev, n, (cudaStream_t)stream);
@@ -320,6 +321,7 @@ extern "C" int mg_genome_pack(mg_genome *g, int64_t contig, int64_t offset, cons
     if (rc) return rc;
     MG_CUDA(cudaSetDevice(g->device));
     g->finalized = false;
+    g->generation++;
     g->stops_valid = g->stops_alt_valid = false;
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t STAGE = 64ll << 20;
@@ -440,6 +442,7 @@ extern "C" int mg_genome_pack_fasta(mg_genome *g, int64_t contig, const uint8_t 
     MG_REQUIRE(n_raw >= 0 && (n_raw == 0 || raw != nullptr), "bad FASTA body");
     MG_CUDA(cudaSetDevice(g->device));
     g->finalized = false;
+    g->generation++;
     g->stops_valid = g->stops_alt_valid = false;
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t RAW = 64ll << 20;                   // raw bytes per trip (multiple of the tile)
@@ -539,6 +542,7 @@ extern "C" int mg_genome_finalize(mg_genome *g, int64_t *n_exceptions_out) {
     g->h_exc_pos.swap(pos);
     g->h_exc_byte.swap(byt);
     g->finalized = true;
+    g->generation++;
     g->stops_valid = g->stops_alt_valid = false;
     if (n_exceptions_out) *n_exceptions_out = g->n_exc;
     return MG_OK;

@@ -118,6 +118,7 @@ extern "C" int mg_genome_mask(mg_genome *g, int64_t n_iv, const int32_t *contig,
         glo[i] = g->h_contig_base[contig[i]] + lo[i];
         ghi[i] = g->h_contig_base[contig[i]] + hi[i];
     }
+    g->generation++;                                                      // counts and plans from before this call are stale
     const int64_t T = g->total_bases, words = T / 8;
     int64_t *d_lo = nullptr, *d_hi = nullptr;
     if (n_iv) {

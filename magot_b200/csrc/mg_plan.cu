@@ -628,9 +628,23 @@ static int plan_launch_records(mg_plan *p, cudaStream_t st) {
     return MG_OK;
 }
 
+// Emits and the calls that report what K1 computed need a plan prepared on the genome as it is now: K1's record pass read the
+// first codons to fix trimX skips, amino-acid counts and protein offsets, and the emit kernels read the bases again.
+int mg_plan_check_prepared(const mg_plan *p) {
+    if (!p->prepared) { mg_set_error("mg_plan_prepare has not been called"); return MG_ESTATE; }
+    if (p->generation != p->g->generation) {
+        mg_set_error("the genome changed (pack, finalize or mask) since the plan was prepared: prepare it again");
+        return MG_ESTATE;
+    }
+    return MG_OK;
+}
+
+// The record pass of a deferred prepare belongs to that prepare: after a genome change it fails like an emit (with the
+// one-launch K1 the record pass has already run inside mg_plan_prepare_async).
 extern "C" int mg_plan_prepare_prot_async(mg_plan *p, void *stream) {
     MG_REQUIRE(p != nullptr, "plan handle is NULL");
     if (!p->prepared) { mg_set_error("mg_plan_prepare_async has not been called"); return MG_ESTATE; }
+    if (const int rc0 = mg_plan_check_prepared(p)) return rc0;
     if (p->prot_ready || p->n_rec == 0) return MG_OK;
     MG_CUDA(cudaSetDevice(p->device));
     p->last_stream = (cudaStream_t)stream;
@@ -692,6 +706,7 @@ extern "C" int mg_plan_prepare(mg_plan *p, int prot_flags, int64_t *nuc_total, i
     rc = plan_launch_tiles(p, p->nuc_total, p->prot_total, st);
     if (rc) return rc;
     p->prepared = true;
+    p->generation = p->g->generation;
     if (nuc_total) *nuc_total = p->nuc_total;
     if (prot_total) *prot_total = p->prot_total;
     return MG_OK;
@@ -708,12 +723,13 @@ extern "C" int mg_plan_prepare_async(mg_plan *p, int prot_flags, int64_t nuc_cap
     p->prot_total = prot_capacity;
     p->totals_known = false;
     p->prepared = true;
+    p->generation = p->g->generation;
     return MG_OK;
 }
 
 extern "C" int mg_plan_totals(mg_plan *p, int64_t *nuc_total, int64_t *prot_total, void *stream) {
     MG_REQUIRE(p != nullptr, "plan handle is NULL");
-    if (!p->prepared) { mg_set_error("mg_plan_prepare has not been called"); return MG_ESTATE; }
+    if (const int rc0 = mg_plan_check_prepared(p)) return rc0;
     MG_CUDA(cudaSetDevice(p->device));
     if (!p->totals_known) {
         int64_t totals[2];
@@ -738,7 +754,7 @@ extern "C" int mg_plan_totals(mg_plan *p, int64_t *nuc_total, int64_t *prot_tota
 
 extern "C" int mg_plan_lengths(mg_plan *p, int64_t *nuc_len, int64_t *aa_len, void *stream) {
     MG_REQUIRE(p != nullptr, "plan handle is NULL");
-    MG_REQUIRE(p->prepared, "mg_plan_prepare has not been called");
+    if (const int rc0 = mg_plan_check_prepared(p)) return rc0;
     if (p->n_rec == 0 || (!nuc_len && !aa_len)) return MG_OK;
     if (aa_len && !p->prot_ready) { mg_set_error("the record pass was deferred (MG_PROT_DEFER): call mg_plan_prepare_prot_async first"); return MG_ESTATE; }
     MG_CUDA(cudaSetDevice(p->device));

@@ -82,6 +82,7 @@ struct mg_sixframe_state {
     uint8_t *d_aa4096 = nullptr;                     // residue table of a caller's genetic code (NULL: the genome's standard table)
     uint8_t h_aa4096[4096];                          // its host copy (source of the asynchronous upload)
     bool orfcall = false;                            // counted by mg_orfcall_count (records in d_calls) instead of mg_sixframe_count*
+    uint64_t generation = 0;                         // g->generation at the count: k_six_aa reads the bases again at emit time
     mg_orfcall *d_calls = nullptr;
     uint8_t *d_start4096 = nullptr;                  // start-codon table of an ORF call (see build_start4096)
     uint8_t h_start4096[4096];
@@ -1591,6 +1592,7 @@ static int six_count(mg_genome *g, int64_t n_list, const int64_t *contig_ids, in
     s->min_aa = min_aa;
     s->force_single = g_six_force_single;
     s->orfcall = orf != nullptr;
+    s->generation = g->generation;
     const int64_t nc = n_list;
     std::vector<int32_t> &h_cid = s->h_cid;
     h_cid.resize(nc);
@@ -1798,12 +1800,24 @@ static int six_residues(mg_genome *g, uint8_t *out_dev, cudaStream_t st) {
     return MG_OK;
 }
 
-static int six_emit_device(mg_genome *g, bool orfcall, uint8_t *aa_out_dev, void *recs_dev, void *stream) {
+// MG_ESTATE unless the preceding count is of this kind and the genome is still the one it scanned
+static int six_check_counted(mg_genome *g, bool orfcall) {
     MG_REQUIRE(g != nullptr, "genome handle is NULL");
     if (!g->six || !g->six->counted || g->six->orfcall != orfcall) {
         mg_set_error(orfcall ? "mg_orfcall_count has not been called" : "mg_sixframe_count has not been called");
         return MG_ESTATE;
     }
+    if (g->six->generation != g->generation) {
+        mg_set_error("the genome changed (pack, finalize or mask) since %s: count again",
+                     orfcall ? "mg_orfcall_count" : "mg_sixframe_count");
+        return MG_ESTATE;
+    }
+    return MG_OK;
+}
+
+static int six_emit_device(mg_genome *g, bool orfcall, uint8_t *aa_out_dev, void *recs_dev, void *stream) {
+    const int rc0 = six_check_counted(g, orfcall);
+    if (rc0) return rc0;
     MG_CUDA(cudaSetDevice(g->device));
     cudaStream_t st = (cudaStream_t)stream;
     mg_sixframe_state *s = g->six;
@@ -1816,11 +1830,8 @@ static int six_emit_device(mg_genome *g, bool orfcall, uint8_t *aa_out_dev, void
 }
 
 static int six_emit_host(mg_genome *g, bool orfcall, uint8_t *aa_out_host, void *recs_host, void *stream) {
-    MG_REQUIRE(g != nullptr, "genome handle is NULL");
-    if (!g->six || !g->six->counted || g->six->orfcall != orfcall) {
-        mg_set_error(orfcall ? "mg_orfcall_count has not been called" : "mg_sixframe_count has not been called");
-        return MG_ESTATE;
-    }
+    const int rc0 = six_check_counted(g, orfcall);
+    if (rc0) return rc0;
     MG_CUDA(cudaSetDevice(g->device));
     cudaStream_t st = (cudaStream_t)stream;
     mg_sixframe_state *s = g->six;
