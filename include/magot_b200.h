@@ -302,7 +302,9 @@ int mg_copy_d2h_async(int device, void *dst_host, const void *src_dev, int64_t n
  * mg_graph_begin and mg_graph_end -- e.g. mg_plan_prepare_async + mg_emit_*_device of several plans, none of which waits for
  * the host -- and replay it with one launch.  The batch-level counterpart of the reference's per-object loop
  * `for obj in table: obj.get_fasta()` (genome.py:578-582).  Buffers and plan handles used inside must stay alive and unchanged
- * in size while the graph is in use.                                                                                    */
+ * in size while the graph is in use.  A capture needs the plan's buffers to exist already: run mg_plan_prepare_async (and
+ * mg_emit_products_device) once outside the capture with at least the captured capacities; a call that would grow a buffer
+ * inside a capture fails with MG_ESTATE before it queues anything.                                                      */
 int mg_graph_begin(int device, void *stream);
 int mg_graph_end(int device, void *stream, void **graph_exec_out);
 int mg_graph_launch(int device, void *graph_exec, void *stream);

@@ -963,14 +963,18 @@ extern "C" int mg_emit_products_device(mg_plan *pa, uint8_t *out_a, mg_plan *pb,
     mg_plan *owner = ja ? pa : pb;
     MG_CUDA(cudaSetDevice(owner->device));
     cudaStream_t st = (cudaStream_t)stream;
+    const int64_t cap = (ja ? pa->n_nuc_tile : 0) + (jb ? pb->n_nuc_tile : 0) + (jc ? pb->n_prot_tile : 0);
+    MG_REQUIRE(cap < (1ll << 28), "more than 2^28 tiles in one launch");
+    if (owner->order_cap < cap) {
+        const int rc0 = mg_refuse_growth_in_capture(st, "mg_emit_products_device (first emit led by this plan, or a larger grid)");
+        if (rc0) return rc0;
+    }
     MultiArgs m;
     memset(&m, 0, sizeof(m));
-    int64_t cap = 0;
-    if (ja) { m.a = nuc_args(pa, out_a); cap += pa->n_nuc_tile; pa->last_stream = st; }
-    if (jb) { m.b = nuc_args(pb, out_b_nuc); cap += pb->n_nuc_tile; }
-    if (jc) { m.c = prot_args(pb, out_b_prot); cap += pb->n_prot_tile; }
+    if (ja) { m.a = nuc_args(pa, out_a); pa->last_stream = st; }
+    if (jb) m.b = nuc_args(pb, out_b_nuc);
+    if (jc) m.c = prot_args(pb, out_b_prot);
     if (jb || jc) pb->last_stream = st;
-    MG_REQUIRE(cap < (1ll << 28), "more than 2^28 tiles in one launch");
     const int64_t lag = ((int64_t)g_multi_lag_ppm << MULTI_SH) / 1000000;
     m.lag[0] = 0; m.lag[1] = ja ? lag : 0; m.lag[2] = m.lag[1] + (jb ? lag : 0);
     if (owner->order_cap < cap) {

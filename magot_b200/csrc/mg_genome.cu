@@ -85,6 +85,19 @@ extern "C" int mg_graph_destroy(void *graph_exec) {
     return MG_OK;
 }
 
+// A plan buffer that has to grow is allocated with cudaMallocAsync on the caller's stream.  Inside a capture that becomes a graph
+// allocation node that nothing in the graph frees: a second launch of the graph fails, and the plan would keep a pointer with no
+// memory behind it until the first replay.  So a call that would grow a buffer while `st` is capturing fails before it queues
+// anything; the caller runs the same call once outside the capture, after which the captured call re-uses the buffer.
+int mg_refuse_growth_in_capture(cudaStream_t st, const char *what) {
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    MG_CUDA(cudaStreamIsCapturing(st, &cs));
+    if (cs == cudaStreamCaptureStatusNone) return MG_OK;
+    mg_set_error("%s would have to grow a plan buffer inside a CUDA graph capture: run it once outside the capture first "
+                 "(prepare, and for products emit, with at least the captured capacities)", what);
+    return MG_ESTATE;
+}
+
 // fork / join helpers for multi-stream steps (also what makes a second stream part of a capture)
 extern "C" int mg_stream_wait_stream(int device, void *waiter, void *signaller) {
     MG_CUDA(cudaSetDevice(device));

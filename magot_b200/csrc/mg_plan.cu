@@ -559,6 +559,10 @@ extern "C" int mg_plan_set_codon_table(mg_plan *p, const uint8_t *codon64) {
 
 // K1, first half: clamp + lengths + offsets of every piece and record; the two text sizes land in p->d_totals
 static int plan_alloc_tiles(mg_plan *p, int64_t cap_nuc, int64_t cap_prot, cudaStream_t st);
+static int64_t plan_tile_need(int64_t cap_nuc, int64_t cap_prot) {   // tile table entries for texts of up to these sizes
+    return (cap_nuc + MG_NUC_TILE - 1) / MG_NUC_TILE + 1 + (cap_prot + MG_PROT_TILE - 1) / MG_PROT_TILE + 1;
+}
+static int64_t pr_tiles(const mg_plan *p) { return (p->n_rec + PR_RECS - 1) / PR_RECS; }   // blocks of k_plan_rec
 
 // scatter_tiles: the tile tables are sized for the caller's capacities and filled by the plan kernels themselves
 static int plan_launch_records(mg_plan *p, cudaStream_t st);
@@ -575,8 +579,12 @@ static int plan_launch_scans(mg_plan *p, int prot_flags, cudaStream_t st, bool s
     // prepare may still be running on another stream when the next piece pass of the same plan starts (a bench step that
     // re-prepares a plan does exactly that), and wiping its ticket counter / status words would leave its tiles waiting for
     // predecessors for ever.  The two text sizes are written unconditionally by the last tile of each pass.
+    // The one-launch K1 zeroes its two look-back arrays and not the totals either: the previous step's K3 or products kernel
+    // may still read them on another stream to bound its tiles.  Only with no record (no kernel writes the totals) is all of
+    // the scratch zeroed.
     const bool one_launch = p->n_rec > 0 && p->max_seg_per_rec <= PR_MAXSEG && mg_k1_mode() == 1;
-    if (p->n_rec == 0 || one_launch) MG_CUDA(cudaMemsetAsync(p->d_scan_tmp, 0, p->scan_tmp_cap * sizeof(int64_t), st));
+    if (p->n_rec == 0) MG_CUDA(cudaMemsetAsync(p->d_scan_tmp, 0, p->scan_tmp_cap * sizeof(int64_t), st));
+    else if (one_launch) MG_CUDA(cudaMemsetAsync(p->d_scan_tmp, 0, 2 * (pr_tiles(p) + 1) * sizeof(unsigned long long), st));
     else MG_CUDA(cudaMemsetAsync(tmp_a, 0, (n_block + 1) * sizeof(unsigned long long), st));
     int64_t *tf_nuc = nullptr, *tf_prot = nullptr;
     if (scatter_tiles) {
@@ -586,8 +594,8 @@ static int plan_launch_scans(mg_plan *p, int prot_flags, cudaStream_t st, bool s
         tf_prot = p->d_prot_tile;
     }
     if (p->n_rec == 0) { p->prot_ready = true; return MG_OK; }
-    if (p->max_seg_per_rec <= PR_MAXSEG && mg_k1_mode() == 1) {     // K1 in one launch
-        const int64_t n_tile = (p->n_rec + PR_RECS - 1) / PR_RECS;
+    if (one_launch) {                                  // K1 in one launch
+        const int64_t n_tile = pr_tiles(p);
         unsigned long long *ta = reinterpret_cast<unsigned long long *>(p->d_scan_tmp), *tb = ta + n_tile + 1;
         p->d_totals = reinterpret_cast<int64_t *>(p->d_scan_tmp + p->scan_tmp_cap - 2);
         k_plan_rec<<<(unsigned)n_tile, PR_THREADS, 0, st>>>(
@@ -656,7 +664,7 @@ extern "C" int mg_plan_prepare_prot_async(mg_plan *p, void *stream) {
 static int plan_alloc_tiles(mg_plan *p, int64_t cap_nuc, int64_t cap_prot, cudaStream_t st) {
     p->n_nuc_tile = (cap_nuc + MG_NUC_TILE - 1) / MG_NUC_TILE;
     p->n_prot_tile = (cap_prot + MG_PROT_TILE - 1) / MG_PROT_TILE;
-    const int64_t tile_need = p->n_nuc_tile + 1 + p->n_prot_tile + 1;
+    const int64_t tile_need = plan_tile_need(cap_nuc, cap_prot);
     if (tile_need > p->tile_cap) {                   // re-used when the same plan is prepared again
         void *d = nullptr;
         MG_CUDA(cudaMallocAsync(&d, tile_need * sizeof(int64_t), st));
@@ -716,6 +724,10 @@ extern "C" int mg_plan_prepare_async(mg_plan *p, int prot_flags, int64_t nuc_cap
     MG_REQUIRE(p != nullptr, "plan handle is NULL");
     MG_REQUIRE(nuc_capacity >= 0 && prot_capacity >= 0, "capacities must be >= 0");
     MG_CUDA(cudaSetDevice(p->device));
+    if (plan_tile_need(nuc_capacity, prot_capacity) > p->tile_cap) {
+        const int rc0 = mg_refuse_growth_in_capture((cudaStream_t)stream, "mg_plan_prepare_async (first prepare, or larger capacities)");
+        if (rc0) return rc0;
+    }
     p->prepared = false;
     int rc = plan_launch_scans(p, prot_flags, (cudaStream_t)stream, true, nuc_capacity, prot_capacity);
     if (rc) return rc;
