@@ -135,6 +135,7 @@ struct mg_plan {
     int64_t *d_scan_tmp = nullptr;            // block sums for scans
     int64_t scan_tmp_cap = 0;
     int64_t nuc_total = -1, prot_total = -1;      // text sizes on the host; with mg_plan_prepare_async: the caller's upper bounds
+    int64_t prot_cap = 0;                         // the protein capacity given to mg_plan_prepare_async
     int64_t *d_totals = nullptr;                  // [2] the same on the device (written by the plan kernels)
     bool totals_known = false;                    // false between mg_plan_prepare_async and mg_plan_totals
     int prot_flags = 0;

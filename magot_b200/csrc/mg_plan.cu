@@ -22,8 +22,13 @@
 
 // ---- kernels ----------------------------------------------------------------------------------------
 
-#define PLAN_ITEMS 4                                 // pieces per thread of k_plan_pieces
-#define PLAN_TILE (256 * PLAN_ITEMS)                 // pieces per block: large enough that the look-back never serialises
+#define PLAN_THREADS 256
+#ifndef PLAN_ITEMS
+#define PLAN_ITEMS 8                                 // pieces per thread of k_plan_pieces (a power of two >= 4)
+#endif
+#define PLAN_TILE (PLAN_THREADS * PLAN_ITEMS)        // pieces per block; 4096 (34 KB of shared memory) was faster alone but
+                                                     // slowed the step by 0.06 ms: its blocks found no room next to K2
+#define PLAN_WORDS (PLAN_TILE / 32)                  // words of the block's record-head bitmap
 
 // thread per record: record r owns pieces [F(r), F(r+1)), F(r) = rec_seg_off[r] + 2r; it writes itself into every
 // PLAN_TILE-piece block whose first piece it owns (coalesced and search-free; a binary search per block was 10 us of dependent loads)
@@ -35,12 +40,28 @@ __global__ void __launch_bounds__(256) k_plan_block_rec(int64_t n_block, int64_t
     for (int64_t b = (f0 + PLAN_TILE - 1) / PLAN_TILE; b * PLAN_TILE < f1 && b < n_block; b++) blk_r0[b] = r;
 }
 
-// thread per piece: find its record, clamp like a Python slice, write src and -- through a block scan of the lengths plus a
-// decoupled look-back across blocks (mg_lookback.cuh) -- the piece's offset in the nucleotide text, all in one launch
+// tile -> first piece by scatter (mg_plan_prepare_async: the table exists before the text size is known): the piece that holds
+// byte t * MG_NUC_TILE writes itself into slot t; the same at 1 KB granularity (one warp of k_emit_nuc_stream = one 1 KB block)
+// when the streaming K2 asks for it.  Empty pieces hold no byte.
+__device__ __forceinline__ void plan_scatter_nuc(int64_t off, int64_t len, int64_t p, int64_t *__restrict__ tile_first,
+                                                 int64_t tile_cap, int32_t *__restrict__ blk1k, int64_t blk1k_cap) {
+    if (len <= 0) return;
+    if (tile_first)
+        for (int64_t t = (off + MG_NUC_TILE - 1) / MG_NUC_TILE; t * MG_NUC_TILE < off + len && t < tile_cap; t++) tile_first[t] = p;
+    for (int64_t t = (off + 1023) >> 10; (t << 10) < off + len && t < blk1k_cap; t++) blk1k[t] = (int32_t)p;
+}
+
+// K1 piece pass: clamp like a Python slice, write piece_src and -- through a block scan of the lengths plus a decoupled
+// look-back across blocks (mg_lookback.cuh) -- every piece's offset in the nucleotide text, in one launch.
+//   1. thread per record of the block: the two literal pieces (src, length) and a bit per record head in s_head;
+//   2. thread per piece, strided so the segment tables are read coalesced: record = popcount of the heads up to the piece,
+//      segment = piece - 2 * record - 1; literal pieces were written in 1, so the loop has one body;
+//   3. a thread sums PLAN_ITEMS consecutive lengths, one block scan, one look-back;
+//   4. the offsets go through shared memory (swizzled) back to the strided order: piece_off is written coalesced.
 #ifndef PLAN_MINB
-#define PLAN_MINB 8                                  // 32 registers: one plan block fits next to the 7 CTAs of k_emit_prot on an SM (step 0.5075 -> 0.4995 ms)
+#define PLAN_MINB 6                                  // 40 registers, 17 KB of shared memory: no spill at 8 items (32 registers spill)
 #endif
-__global__ void __launch_bounds__(256, PLAN_MINB) k_plan_pieces(int64_t n_piece, int64_t n_rec, const int64_t *__restrict__ rec_seg_off,
+__global__ void __launch_bounds__(PLAN_THREADS, PLAN_MINB) k_plan_pieces(int64_t n_piece, int64_t n_rec, const int64_t *__restrict__ rec_seg_off,
                                                      const int64_t *__restrict__ blk_r0,
                                                      const int32_t *__restrict__ seg_contig, const int64_t *__restrict__ seg_start,
                                                      const int64_t *__restrict__ seg_end, const int8_t *__restrict__ seg_strand,
@@ -51,94 +72,127 @@ __global__ void __launch_bounds__(256, PLAN_MINB) k_plan_pieces(int64_t n_piece,
                                                      int64_t *__restrict__ piece_src, int64_t *__restrict__ total_out,
                                                      int64_t *__restrict__ tile_first, int64_t tile_cap,
                                                      int32_t *__restrict__ blk1k, int64_t blk1k_cap) {
-    // The PLAN_TILE pieces of a block belong to at most PLAN_TILE/2 + 1 consecutive records starting at blk_r0[block]
-    // (k_plan_block_rec): F(r) = rec_seg_off[r] + 2r of those records is staged in shared memory and every thread
-    // searches there.
-    __shared__ int64_t s_F[PLAN_TILE / 2 + 2];
+    // s_len (piece lengths: a piece is < 2^31 bytes) until step 3, then s_off (block-relative offsets, 64 bits)
+    __shared__ __align__(16) int64_t s_buf[PLAN_TILE];
+    uint32_t *s_len = reinterpret_cast<uint32_t *>(s_buf);
+    __shared__ uint32_t s_head[PLAN_WORDS + 1];       // bit j: piece pb + j is a literal prefix (bit PLAN_TILE: the piece after the block)
+    __shared__ uint32_t s_cnt[PLAN_WORDS];            // heads in the words before
     __shared__ int64_t s_warp[8];
     __shared__ int64_t s_prefix;
     __shared__ unsigned int s_tile;
+    for (int i = threadIdx.x; i <= PLAN_WORDS; i += PLAN_THREADS) s_head[i] = 0;
     const int64_t tile = mg_next_tile(tmp, &s_tile);
     const int64_t pb = tile * PLAN_TILE;
-    const int64_t r0 = blk_r0[tile];
-    for (int i = threadIdx.x; i < PLAN_TILE / 2 + 2; i += blockDim.x) {
-        const int64_t r = r0 + i;
-        s_F[i] = r <= n_rec ? __ldg(rec_seg_off + r) + 2 * r : INT64_MAX;
+    const int nt = (int)min((int64_t)PLAN_TILE, n_piece - pb);   // pieces of this block
+    const int64_t pe = pb + nt;
+    const int64_t r0 = blk_r0[tile];                 // the record that owns piece pb (k_plan_block_rec)
+
+    // 1. Record r writes its prefix F(r) and suffix F(r+1)-1 where they fall in the block and marks F(r+1), the next record's
+    // head; r0 marks its own head when it starts the block.  Rounds of PLAN_THREADS records until one ends at or past pe.
+    for (int64_t r = r0 + threadIdx.x;; r += PLAN_THREADS) {
+        bool more = false;
+        if (r < n_rec) {
+            const int64_t f0 = __ldg(rec_seg_off + r) + 2 * r;
+            if (f0 < pe) {
+                const int64_t f1 = __ldg(rec_seg_off + r + 1) + 2 * (r + 1);
+                const int64_t lit = __ldg(rec_lit_off + r);
+                const int32_t pre = __ldg(rec_pre + r), suf = __ldg(rec_suf + r);
+                if (f0 >= pb) {
+                    s_len[f0 - pb] = (uint32_t)pre;
+                    piece_src[f0] = lit | (int64_t)(MG_KIND_LIT << MG_KIND_SHIFT);
+                    if (f0 == pb) atomicOr(&s_head[0], 1u);
+                }
+                if (f1 - 1 < pe) {
+                    s_len[f1 - 1 - pb] = (uint32_t)suf;
+                    piece_src[f1 - 1] = (lit + pre) | (int64_t)(MG_KIND_LIT << MG_KIND_SHIFT);
+                }
+                if (f1 - pb <= PLAN_TILE) atomicOr(&s_head[(f1 - pb) >> 5], 1u << ((f1 - pb) & 31));
+                more = f1 < pe;
+            }
+        }
+        if (!__syncthreads_and(more)) break;         // records grow with the thread index: the round's last one decides
+    }
+    if (threadIdx.x < 32) {                          // heads before each word: one warp, PLAN_WORDS / 32 words a lane
+        uint32_t c[PLAN_WORDS / 32], sum = 0;
+#pragma unroll
+        for (int k = 0; k < PLAN_WORDS / 32; k++) { c[k] = __popc(s_head[threadIdx.x * (PLAN_WORDS / 32) + k]); sum += c[k]; }
+        uint32_t incl = sum;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const uint32_t t = __shfl_up_sync(0xffffffffu, incl, d);
+            if ((int)threadIdx.x >= d) incl += t;
+        }
+        uint32_t run = incl - sum;
+#pragma unroll
+        for (int k = 0; k < PLAN_WORDS / 32; k++) { s_cnt[threadIdx.x * (PLAN_WORDS / 32) + k] = run; run += c[k]; }
     }
     __syncthreads();
-    // blocked arrangement: a thread owns PLAN_ITEMS consecutive pieces, so the block needs ONE scan and nothing between
-    // the pieces' (dependent) table loads makes them wait for each other
-    int64_t len[PLAN_ITEMS];
-    const int64_t p0 = pb + (int64_t)threadIdx.x * PLAN_ITEMS;
-    int lo = 0;                                        // record of the current piece, relative to r0
-#pragma unroll
+
+    // 2. Genome segments.  A warp's 32 pieces of one round are one word of s_head, so lane l's record is r0 plus the heads in
+    // bits 0..l (less one when the block starts with r0's own prefix).
+    const int lane = threadIdx.x & 31;
+    const uint32_t upto = 0xffffffffu >> (31 - lane);
+    const int64_t rb = r0 - (int64_t)(s_head[0] & 1u);
+#pragma unroll 4
     for (int it = 0; it < PLAN_ITEMS; it++) {
-        const int64_t p = p0 + it;
-        len[it] = 0;
-        if (p < n_piece) {
-            if (it == 0) {                              // the thread's first piece: search; its next ones: walk on
-                int hi = PLAN_TILE / 2 + 1;            // F(r0) <= p < F(r0 + PLAN_TILE/2 + 1): F grows by >= 2 per record
-                while (hi - lo > 1) {
-                    const int mid = (lo + hi) >> 1;
-                    if (s_F[mid] <= p) lo = mid; else hi = mid;
-                }
-            } else {
-                while (s_F[lo + 1] <= p) lo++;
-            }
-            const int64_t r = r0 + lo;
-            const int64_t s0 = s_F[lo] - 2 * r, s1 = s_F[lo + 1] - 2 * (r + 1);
-            const int64_t local = p - (s0 + 2 * r);
-            if (local == 0) {                           // literal prefix
-                len[it] = rec_pre[r];
-                piece_src[p] = rec_lit_off[r] | (int64_t)(MG_KIND_LIT << MG_KIND_SHIFT);
-            } else if (local == s1 - s0 + 1) {          // literal suffix
-                len[it] = rec_suf[r];
-                piece_src[p] = (rec_lit_off[r] + rec_pre[r]) | (int64_t)(MG_KIND_LIT << MG_KIND_SHIFT);
-            } else {                                    // genome segment
-                const int64_t e = s0 + local - 1;
-                const int32_t c = seg_contig[e];
-                int64_t src = MG_FRONT_PAD, n = 0;
-                if (c >= 0 && c < n_contigs) {
-                    const int64_t L = contig_len[c];
-                    // contig[start-1:end] with Python slice semantics (genome.py:606)
-                    int64_t i = seg_start[e] - 1, j = seg_end[e];
-                    if (i < 0) { i += L; if (i < 0) i = 0; } else if (i > L) i = L;
-                    if (j < 0) { j += L; if (j < 0) j = 0; } else if (j > L) j = L;
-                    n = j > i ? j - i : 0;
-                    if (n > 0x7fffffff) n = 0x7fffffff;
-                    src = contig_base[c] + i;
-                }
-                len[it] = n;
-                // '-' strand: forward bases [src, src+len) are bases [2T-src-len, 2T-src) of the reverse-complement plane,
-                // in exactly the order Sequence.reverse_compliment emits them (genome.py:784-793)
-                piece_src[p] = seg_strand[e] ? two_T - src - n : src;
-            }
+        const int j = it * PLAN_THREADS + threadIdx.x, w = j >> 5;
+        if (j >= nt) { s_len[j] = 0; continue; }
+        const uint32_t h = s_head[w];
+        const uint32_t lit = h | (h >> 1) | (s_head[w + 1] << 31);   // a head (prefix) or the piece before one (suffix)
+        if ((lit >> lane) & 1u) continue;
+        const int64_t p = pb + j;
+        const int64_t e = p - 2 * (rb + s_cnt[w] + __popc(h & upto)) - 1;
+        const int32_t c = __ldg(seg_contig + e);
+        const int64_t s = __ldg(seg_start + e), en = __ldg(seg_end + e);
+        const int8_t minus = __ldg(seg_strand + e);
+        int64_t src = MG_FRONT_PAD, n = 0;
+        if (c >= 0 && c < n_contigs) {
+            const int64_t L = __ldg(contig_len + c);
+            // contig[start-1:end] with Python slice semantics (genome.py:606)
+            int64_t i = s - 1, k = en;
+            if (i < 0) { i += L; if (i < 0) i = 0; } else if (i > L) i = L;
+            if (k < 0) { k += L; if (k < 0) k = 0; } else if (k > L) k = L;
+            n = k > i ? k - i : 0;
+            if (n > 0x7fffffff) n = 0x7fffffff;
+            src = __ldg(contig_base + c) + i;
         }
+        s_len[j] = (uint32_t)n;
+        // '-' strand: forward bases [src, src+len) are bases [2T-src-len, 2T-src) of the reverse-complement plane,
+        // in exactly the order Sequence.reverse_compliment emits them (genome.py:784-793)
+        piece_src[p] = minus ? two_T - src - n : src;
     }
+    __syncthreads();
+
+    // 3. blocked: a thread owns PLAN_ITEMS consecutive pieces, so the block needs ONE scan
+    uint32_t len[PLAN_ITEMS];
     int64_t mine = 0;
 #pragma unroll
-    for (int it = 0; it < PLAN_ITEMS; it++) mine += len[it];
+    for (int q = 0; q < PLAN_ITEMS / 4; q++) {
+        const uint4 u = reinterpret_cast<const uint4 *>(s_len + threadIdx.x * PLAN_ITEMS)[q];
+        len[4 * q] = u.x; len[4 * q + 1] = u.y; len[4 * q + 2] = u.z; len[4 * q + 3] = u.w;
+        mine += (int64_t)u.x + (int64_t)u.y + (int64_t)u.z + (int64_t)u.w;
+    }
     int64_t total;
-    const int64_t incl = mg_block_incl_scan(mine, s_warp, &total);
-    const int64_t prefix = mg_lookback(tmp, tile, total, &s_prefix);
-    int64_t run = prefix + incl - mine;
+    const int64_t incl = mg_block_incl_scan(mine, s_warp, &total);   // its barriers also end every read of s_len
+    int64_t run = incl - mine;
 #pragma unroll
+    for (int i = 0; i < PLAN_ITEMS; i++) {           // slot rotated by the thread index: two wavefronts a warp store
+        s_buf[threadIdx.x * PLAN_ITEMS + ((i + threadIdx.x) & (PLAN_ITEMS - 1))] = run;
+        run += len[i];
+    }
+    const int64_t prefix = mg_lookback(tmp, tile, total, &s_prefix);   // ends with a barrier
+
+    // 4. strided again: coalesced piece_off, and the tile tables
+#pragma unroll 4
     for (int it = 0; it < PLAN_ITEMS; it++) {
-        if (p0 + it < n_piece) {
-            piece_off[p0 + it] = run;
-            // tile -> first piece by scatter (mg_plan_prepare_async: the table exists before the text size is known): the
-            // piece that holds byte t * MG_NUC_TILE writes itself into slot t; empty pieces hold no byte
-            if (tile_first && len[it] > 0) {
-                for (int64_t t = (run + MG_NUC_TILE - 1) / MG_NUC_TILE; t * MG_NUC_TILE < run + len[it] && t < tile_cap; t++)
-                    tile_first[t] = p0 + it;
-            }
-            // the same at 1 KB granularity (one warp of k_emit_nuc_stream = one 1 KB block): a piece of ~190 bytes holds the first
-            // byte of a block once in five times
-            if (blk1k_cap > 0 && len[it] > 0) {
-                for (int64_t t = (run + 1023) >> 10; (t << 10) < run + len[it] && t < blk1k_cap; t++) blk1k[t] = (int32_t)(p0 + it);
-            }
-        }
-        run += len[it];
+        const int j = it * PLAN_THREADS + threadIdx.x;
+        if (j >= nt) break;
+        const int t0 = j / PLAN_ITEMS, t1 = (j + 1) / PLAN_ITEMS;
+        const int64_t o0 = s_buf[t0 * PLAN_ITEMS + ((j + t0) & (PLAN_ITEMS - 1))];
+        const int64_t o1 = j + 1 < nt ? s_buf[t1 * PLAN_ITEMS + ((j + 1 + t1) & (PLAN_ITEMS - 1))] : total;
+        const int64_t off = prefix + o0;
+        piece_off[pb + j] = off;
+        plan_scatter_nuc(off, o1 - o0, pb + j, tile_first, tile_cap, blk1k, blk1k_cap);
     }
     if (tile == gridDim.x - 1 && threadIdx.x == 0) {
         const int64_t all = prefix + total;
@@ -153,9 +207,16 @@ __global__ void __launch_bounds__(256, PLAN_MINB) k_plan_pieces(int64_t n_piece,
     }
 }
 
-// thread per record: spliced length -> amino-acid count (Sequence.translate, genome.py:810-821) and, with the same
-// scan + look-back, the record's offset in the protein text
-__global__ void __launch_bounds__(256) k_plan_records(int64_t n_rec, const int64_t *__restrict__ rec_seg_off,
+// K1 record pass: spliced length -> amino-acid count (Sequence.translate, genome.py:810-821) and, with a block scan + look-back,
+// the record's offset in the protein text.  A thread owns REC_ITEMS consecutive records, and a record costs three dependent
+// trips in the common case: its rec_seg_off words; the offsets of its prefix, first two segment pieces, suffix and the first
+// segment's source; the first codon, read straight from that segment when it holds skip + 3 bases.
+#define REC_THREADS 256
+#ifndef REC_ITEMS
+#define REC_ITEMS 2                                  // 4 was slower at 1/8 of config 4 (fewer blocks in flight)
+#endif
+#define REC_TILE (REC_THREADS * REC_ITEMS)
+__global__ void __launch_bounds__(REC_THREADS) k_plan_records(int64_t n_rec, const int64_t *__restrict__ rec_seg_off,
                                                       const int64_t *__restrict__ piece_off, const int64_t *__restrict__ piece_src,
                                                       const uint32_t *__restrict__ packed, const int8_t *__restrict__ rec_phase,
                                                       int flags, int32_t *__restrict__ rec_aa, int8_t *__restrict__ rec_skip,
@@ -166,49 +227,69 @@ __global__ void __launch_bounds__(256) k_plan_records(int64_t n_rec, const int64
     __shared__ int64_t s_prefix;
     __shared__ unsigned int s_tile;
     const int64_t tile = mg_next_tile(tmp, &s_tile);
-    const int64_t r = tile * (int64_t)blockDim.x + threadIdx.x;
-    int64_t plen = 0;
-    if (r < n_rec) {
-    const int64_t f0 = rec_seg_off[r] + 2 * r, f1 = rec_seg_off[r + 1] + 2 * (r + 1);
-    const int64_t pay0 = piece_off[f0 + 1], pay1 = piece_off[f1 - 1];
-    const int64_t pre = pay0 - piece_off[f0], suf = piece_off[f1] - pay1;
-    int64_t L = pay1 - pay0;
-    int skip = 0;
-    if ((flags & MG_PROT_USE_PHASE) && rec_phase) { skip = rec_phase[r]; if (skip < 0 || skip > 2) skip = 0; }
-    L -= skip;
-    int64_t naa;
-    if (L <= 2) {
-        naa = -1;                                        // reference returns None (genome.py:810)
-    } else {
-        naa = L / 3;
-        if (flags & MG_PROT_TRIMX) {                     // drop exactly one leading X (genome.py:819-821)
-            uint64_t acc[3];
-            const int64_t S = pay0 + skip;
-            // the piece that holds S: nearly always the record's first segment piece (a walk over the same cache line;
-            // a binary search over the record's pieces was three dependent global loads)
-            int64_t j = f0 + 1;
-            while (j + 1 < f1 - 1 && __ldg(piece_off + j + 1) <= S) j++;
-            mg_gather_nib(packed, piece_off, piece_src, j, S, 3, acc);
-            const uint32_t n3 = (uint32_t)acc[0] & 0xFFFu;
-            if (n3 & 0x888u) { naa -= 1; skip += 3; }
+    const int64_t r0 = tile * REC_TILE + (int64_t)threadIdx.x * REC_ITEMS;
+    const bool phase = (flags & MG_PROT_USE_PHASE) && rec_phase;
+    int64_t so[REC_ITEMS + 1];
+    int ph[REC_ITEMS];
+#pragma unroll
+    for (int k = 0; k <= REC_ITEMS; k++) so[k] = r0 + k <= n_rec ? __ldg(rec_seg_off + r0 + k) : 0;
+#pragma unroll
+    for (int k = 0; k < REC_ITEMS; k++) ph[k] = phase && r0 + k < n_rec ? rec_phase[r0 + k] : 0;
+    int64_t plen[REC_ITEMS], mine = 0;
+#pragma unroll
+    for (int k = 0; k < REC_ITEMS; k++) {
+        const int64_t r = r0 + k;
+        plen[k] = 0;
+        if (r >= n_rec) continue;
+        const int64_t f0 = so[k] + 2 * r, f1 = so[k + 1] + 2 * (r + 1);
+        // f0 + 2 <= f1 <= n_piece: all five offsets exist; piece f0 + 1 is the first segment whenever the payload is not empty
+        const int64_t o_pre = __ldg(piece_off + f0), pay0 = __ldg(piece_off + f0 + 1), o_2 = __ldg(piece_off + f0 + 2);
+        const int64_t pay1 = __ldg(piece_off + f1 - 1), o_end = __ldg(piece_off + f1);
+        const int64_t src1 = __ldg(piece_src + f0 + 1) & (int64_t)MG_SRC_MASK;
+        int skip = ph[k];
+        if (skip < 0 || skip > 2) skip = 0;
+        const int64_t L = pay1 - pay0 - skip;
+        int64_t naa;
+        if (L <= 2) {
+            naa = -1;                                    // reference returns None (genome.py:810)
+        } else {
+            naa = L / 3;
+            if (flags & MG_PROT_TRIMX) {                 // drop exactly one leading X (genome.py:819-821)
+                const int64_t S = pay0 + skip;
+                uint32_t n3;
+                if (S + 3 <= o_2) {
+                    n3 = (uint32_t)mg_ld_nib16(packed, src1 + skip);
+                } else {                                 // the codon starts past, or runs out of, the first segment: walk
+                    uint64_t acc[3];
+                    int64_t j = f0 + 1;
+                    while (j + 1 < f1 - 1 && __ldg(piece_off + j + 1) <= S) j++;
+                    mg_gather_nib(packed, piece_off, piece_src, j, S, 3, acc);
+                    n3 = (uint32_t)acc[0];
+                }
+                if (n3 & 0x888u) { naa -= 1; skip += 3; }
+            }
         }
-    }
-    if (naa > 0x7fffffff) naa = 0x7fffffff;
-    rec_aa[r] = (int32_t)naa;
-    rec_skip[r] = (int8_t)skip;
-    plen = pre + (naa > 0 ? naa : 0) + suf;
+        if (naa > 0x7fffffff) naa = 0x7fffffff;
+        rec_aa[r] = (int32_t)naa;
+        rec_skip[r] = (int8_t)skip;
+        plen[k] = (pay0 - o_pre) + (naa > 0 ? naa : 0) + (o_end - pay1);
+        mine += plen[k];
     }
     int64_t total;
-    const int64_t incl = mg_block_incl_scan(plen, s_warp, &total);
+    const int64_t incl = mg_block_incl_scan(mine, s_warp, &total);
     const int64_t prefix = mg_lookback(tmp, tile, total, &s_prefix);
-    if (r < n_rec) {
-        const int64_t off = prefix + incl - plen;
+    int64_t off = prefix + incl - mine;
+#pragma unroll
+    for (int k = 0; k < REC_ITEMS; k++) {
+        const int64_t r = r0 + k;
+        if (r >= n_rec) break;
         prot_off[r] = off;
-        if (tile_first && plen > 0) {                  // tile -> first record by scatter, see k_plan_pieces
-            for (int64_t t = (off + MG_PROT_TILE - 1) / MG_PROT_TILE; t * MG_PROT_TILE < off + plen && t < tile_cap; t++) tile_first[t] = r;
+        if (tile_first && plen[k] > 0) {               // tile -> first record by scatter, see plan_scatter_nuc
+            for (int64_t t = (off + MG_PROT_TILE - 1) / MG_PROT_TILE; t * MG_PROT_TILE < off + plen[k] && t < tile_cap; t++) tile_first[t] = r;
         }
+        off += plen[k];
     }
-    if (tile == gridDim.x - 1 && threadIdx.x == blockDim.x - 1) {
+    if (tile == gridDim.x - 1 && threadIdx.x == 0) {
         const int64_t all = prefix + total;
         prot_off[n_rec] = all;
         *total_out = all;
@@ -509,7 +590,8 @@ extern "C" int mg_plan_create(mg_genome *g, int64_t n_rec, const int64_t *rec_se
     TRY(dalloc(p, &p->d_prot_off, n_rec + 1, st));
     TRY(dalloc(p, &p->d_rec_aa, n_rec, st));
     TRY(dalloc(p, &p->d_rec_skip, n_rec, st));
-    // look-back scratch: [ticket, status per 256-piece block] [ticket, status per 256-record block] [nuc total, prot total]
+    // look-back scratch: [ticket, status per PLAN_TILE-piece block] [ticket, status per REC_TILE-record block] [nuc total, prot total];
+    // the one-launch K1 uses two [ticket, status per PR_RECS-record block] arrays and the last two words
     p->scan_tmp_cap = (p->n_piece + PLAN_TILE - 1) / PLAN_TILE + 1 + 2 * ((n_rec + 127) / 128 + 1) + 2;
     for (int64_t r = 0; r < n_rec; r++) p->max_seg_per_rec = std::max(p->max_seg_per_rec, rec_seg_off[r + 1] - rec_seg_off[r]);
     TRY(dalloc(p, &p->d_scan_tmp, p->scan_tmp_cap, st));
@@ -572,7 +654,7 @@ static int plan_launch_scans(mg_plan *p, int prot_flags, cudaStream_t st, bool s
     p->prot_flags = prot_flags;
     p->last_stream = st;
     p->prot_ready = false;
-    const int64_t n_block = (p->n_piece + PLAN_TILE - 1) / PLAN_TILE, n_rblock = (p->n_rec + 255) / 256;
+    const int64_t n_block = (p->n_piece + PLAN_TILE - 1) / PLAN_TILE, n_rblock = (p->n_rec + REC_TILE - 1) / REC_TILE;
     unsigned long long *tmp_a = reinterpret_cast<unsigned long long *>(p->d_scan_tmp), *tmp_b = tmp_a + n_block + 1;
     p->d_totals = reinterpret_cast<int64_t *>(tmp_b + n_rblock + 1);
     // Each pass zeroes ITS OWN look-back words, in its own stream, right before its kernel: the record pass of a deferred
@@ -611,7 +693,7 @@ static int plan_launch_scans(mg_plan *p, int prot_flags, cudaStream_t st, bool s
     // (d_blk_r0 was filled by mg_plan_create.)  The 1 KB block table is read by the streaming K2 variant only.
     const bool want_blk1k = mg_emit_mode() == 2;
     p->blk1k_ready = want_blk1k;
-    k_plan_pieces<<<(unsigned)n_block, 256, 0, st>>>(
+    k_plan_pieces<<<(unsigned)n_block, PLAN_THREADS, 0, st>>>(
         p->n_piece, p->n_rec, p->d_rec_seg_off, p->d_blk_r0, p->d_seg_contig, p->d_seg_start, p->d_seg_end, p->d_seg_strand,
         p->d_rec_lit_off, p->d_rec_pre, p->d_rec_suf, g->d_contig_len, g->d_contig_base, g->n_contigs, 2 * g->total_bases,
         tmp_a, p->d_piece_off, p->d_piece_src, p->d_totals, tf_nuc, p->n_nuc_tile, p->d_blk1k, want_blk1k ? p->blk1k_cap : 0);
@@ -626,9 +708,9 @@ static int plan_launch_scans(mg_plan *p, int prot_flags, cudaStream_t st, bool s
 // K1, record half: amino-acid counts, first-codon trims and the offsets in the protein text (needed by the protein kernels only)
 static int plan_launch_records(mg_plan *p, cudaStream_t st) {
     mg_genome *g = p->g;
-    const int64_t n_rblock = (p->n_rec + 255) / 256;
+    const int64_t n_rblock = (p->n_rec + REC_TILE - 1) / REC_TILE;
     MG_CUDA(cudaMemsetAsync(p->rec_tmp, 0, p->rec_tmp_words * sizeof(unsigned long long), st));
-    k_plan_records<<<(unsigned)n_rblock, 256, 0, st>>>(
+    k_plan_records<<<(unsigned)n_rblock, REC_THREADS, 0, st>>>(
         p->n_rec, p->d_rec_seg_off, p->d_piece_off, p->d_piece_src, g->d_packed, p->d_rec_phase, p->prot_flags,
         p->d_rec_aa, p->d_rec_skip, p->rec_tmp, p->d_prot_off, p->d_totals + 1, p->rec_tile, p->n_prot_tile);
     MG_LAUNCH_CHECK();
@@ -656,6 +738,10 @@ extern "C" int mg_plan_prepare_prot_async(mg_plan *p, void *stream) {
     if (p->prot_ready || p->n_rec == 0) return MG_OK;
     MG_CUDA(cudaSetDevice(p->device));
     p->last_stream = (cudaStream_t)stream;
+    if (p->totals_known) {                             // mg_plan_totals ran before this pass: its protein size (0) is stale
+        p->prot_total = p->prot_cap;
+        p->totals_known = false;
+    }
     return plan_launch_records(p, (cudaStream_t)stream);
 }
 
@@ -733,6 +819,7 @@ extern "C" int mg_plan_prepare_async(mg_plan *p, int prot_flags, int64_t nuc_cap
     if (rc) return rc;
     p->nuc_total = nuc_capacity;                     // until mg_plan_totals: what the caller's buffers can take
     p->prot_total = prot_capacity;
+    p->prot_cap = prot_capacity;
     p->totals_known = false;
     p->prepared = true;
     p->generation = p->g->generation;
