@@ -106,6 +106,9 @@ int mg_window_sums(int device, const void *values_host, int elem_size, int64_t n
  * (prefix bytes immediately followed by suffix bytes).
  * Segment coordinates are the raw, sorted GFF pair (start,end), 1-based inclusive; the device
  * applies Python slice semantics contig[start-1:end] including negative / out-of-range values.
+ * A segment may be of any length (a whole chromosome of more than 2^31 bases too).  A record's
+ * payload (its clamped segments together) is limited to 3 * (2^31 - 1) + 2 bases, so that its
+ * protein has at most 2^31 - 1 residues: a longer record fails with MG_EINVAL.
  * seg_strand: 0 = '+' or '.', 1 = '-' (reverse-complement that segment).
  * rec_phase (may be NULL): phase of the first segment in emission order, used only with
  * MG_PROT_USE_PHASE.                                                                          */

@@ -153,7 +153,7 @@ __global__ void __launch_bounds__(PLAN_THREADS, PLAN_MINB) k_plan_pieces(int64_t
             if (i < 0) { i += L; if (i < 0) i = 0; } else if (i > L) i = L;
             if (k < 0) { k += L; if (k < 0) k = 0; } else if (k > L) k = L;
             n = k > i ? k - i : 0;
-            if (n > 0x7fffffff) n = 0x7fffffff;
+            if (n > 0x7fffffff) n = 0x7fffffff;   // not reached: mg_plan_create splits longer segments
             src = __ldg(contig_base + c) + i;
         }
         s_len[j] = (uint32_t)n;
@@ -330,7 +330,7 @@ __device__ __forceinline__ pr_seg pr_clamp(int64_t e, const int32_t *__restrict_
         if (i < 0) { i += L; if (i < 0) i = 0; } else if (i > L) i = L;
         if (j < 0) { j += L; if (j < 0) j = 0; } else if (j > L) j = L;
         n = j > i ? j - i : 0;
-        if (n > 0x7fffffff) n = 0x7fffffff;
+        if (n > 0x7fffffff) n = 0x7fffffff;       // not reached: mg_plan_create splits longer segments
         src = __ldg(contig_base + c) + i;
     }
     // '-' strand: forward bases [src, src+n) are bases [2T-src-n, 2T-src) of the reverse-complement plane, in the order
@@ -539,6 +539,73 @@ extern "C" int mg_plan_create(mg_genome *g, int64_t n_rec, const int64_t *rec_se
     MG_REQUIRE(n_seg == 0 || (seg_contig && seg_start && seg_end && seg_strand), "segment arrays are NULL");
     MG_REQUIRE(n_rec == 0 || (rec_lit_off && rec_pre_len && rec_suf_len), "record arrays are NULL");
     MG_REQUIRE(rec_seg_off[0] == 0 && rec_seg_off[n_rec] == n_seg, "rec_seg_off must start at 0 and end at n_seg");
+    // The Python-slice clamp of every segment (the rule of the plan kernels, genome.py:606), exactly, on the host: the nucleotide
+    // text size, the protein limit of each record, and the segments the kernels cannot take as one piece.
+    const int64_t SPLIT_AT = 1ll << 31, CHUNK = 1ll << 30;
+    const int64_t REC_MAX = 3 * 0x7fffffffll + 2;     // rec_aa is int32: at most 2^31 - 1 amino acids of 3 bases each
+    auto clamp = [&](int64_t e, int64_t *lo) -> int64_t {   // clamped length of segment e; *lo = its first base in the contig
+        const int32_t c = seg_contig[e];
+        *lo = 0;
+        if (c < 0 || c >= g->n_contigs) return 0;
+        const int64_t L = g->h_contig_len[c];
+        int64_t i = seg_start[e] - 1, k = seg_end[e];
+        if (i < 0) { i += L; if (i < 0) i = 0; } else if (i > L) i = L;
+        if (k < 0) { k += L; if (k < 0) k = 0; } else if (k > L) k = L;
+        *lo = i;
+        return k > i ? k - i : 0;
+    };
+    int64_t nuc_bytes = 0;
+    bool any_long = false;
+    for (int64_t r = 0; r < n_rec; r++) {
+        int64_t pay = 0, lo;
+        for (int64_t e = rec_seg_off[r]; e < rec_seg_off[r + 1]; e++) {
+            const int64_t n = clamp(e, &lo);
+            any_long |= n >= SPLIT_AT;
+            pay += n;
+        }
+        if (pay > REC_MAX) {
+            mg_set_error("record %lld holds %lld bases: a record's payload is limited to 3 * (2^31 - 1) + 2 = %lld bases "
+                         "(its protein length is an int32)", (long long)r, (long long)pay, (long long)REC_MAX);
+            return MG_EINVAL;
+        }
+        nuc_bytes += pay + rec_pre_len[r] + rec_suf_len[r];
+    }
+    // Pieces are int32-long in the plan and emit kernels (piece lengths in shared memory, tile-relative offsets), so a segment of
+    // 2^31 bases or more is split into consecutive chunks of at most 2^30 bases.  Each chunk lies inside its contig, so the
+    // kernels' clamp leaves it alone; on '-' the chunks run from the slice's end to its start, because rc(s) = rc(last chunk) +
+    // ... + rc(first chunk).  A table without such a segment is uploaded as it is.
+    std::vector<int64_t> x_rec_seg_off, x_start, x_end;
+    std::vector<int32_t> x_contig;
+    std::vector<int8_t> x_strand;
+    if (any_long) {
+        x_rec_seg_off.reserve(n_rec + 1);
+        x_rec_seg_off.push_back(0);
+        for (int64_t r = 0; r < n_rec; r++) {
+            for (int64_t e = rec_seg_off[r]; e < rec_seg_off[r + 1]; e++) {
+                int64_t lo0;
+                const int64_t n = clamp(e, &lo0);
+                if (n < SPLIT_AT) {
+                    x_contig.push_back(seg_contig[e]); x_start.push_back(seg_start[e]); x_end.push_back(seg_end[e]);
+                    x_strand.push_back(seg_strand[e]);
+                    continue;
+                }
+                const int64_t k = (n + CHUNK - 1) / CHUNK;
+                for (int64_t q = 0; q < k; q++) {
+                    const int64_t j = seg_strand[e] ? k - 1 - q : q;
+                    const int64_t lo = lo0 + j * CHUNK, hi = std::min(lo0 + n, lo + CHUNK);
+                    x_contig.push_back(seg_contig[e]); x_start.push_back(lo + 1); x_end.push_back(hi);
+                    x_strand.push_back(seg_strand[e]);
+                }
+            }
+            x_rec_seg_off.push_back((int64_t)x_contig.size());
+        }
+        n_seg = (int64_t)x_contig.size();
+        rec_seg_off = x_rec_seg_off.data();
+        seg_contig = x_contig.data();
+        seg_start = x_start.data();
+        seg_end = x_end.data();
+        seg_strand = x_strand.data();
+    }
     MG_REQUIRE(n_seg + 2 * n_rec < 0x7fffffff, "more than 2^31 pieces in one plan: split the table");
     MG_CUDA(cudaSetDevice(g->device));
     cudaStream_t st = (cudaStream_t)stream;
@@ -571,16 +638,8 @@ extern "C" int mg_plan_create(mg_genome *g, int64_t n_rec, const int64_t *rec_se
     }
     if (rec_phase) TRY(upload(p, &p->d_rec_phase, rec_phase, n_rec, st));
     TRY(dalloc(p, &p->d_blk_r0, (p->n_piece + PLAN_TILE - 1) / PLAN_TILE + 1, st));
-    {   // upper bound of the nucleotide text size from the host tables (clamping on the device can only shorten a segment)
-        int64_t up = 0;
-        for (int64_t e = 0; e < n_seg; e++) {
-            int64_t d = seg_end[e] - seg_start[e] + 1;
-            const int32_t c = seg_contig[e];
-            const int64_t L = (c >= 0 && c < g->n_contigs) ? g->h_contig_len[c] : 0;
-            if (seg_start[e] > seg_end[e] || d > L) d = L;          // unsorted pairs can wrap around (Python slice rules): bound by the contig
-            if (d > 0) up += d < 0x7fffffff ? d : 0x7fffffff;
-        }
-        for (int64_t r = 0; r < n_rec; r++) up += (int64_t)rec_pre_len[r] + rec_suf_len[r];
+    {   // the nucleotide text size, from the clamped lengths above
+        const int64_t up = nuc_bytes;
         p->nuc_upper = up;
         p->blk1k_cap = (up >> 10) + 3;
         TRY(dalloc(p, &p->d_blk1k, p->blk1k_cap, st));
