@@ -267,6 +267,56 @@ int mg_orfcall_count(mg_genome *g, int64_t n_list, const int64_t *contig_ids, in
 int mg_orfcall_emit(mg_genome *g, uint8_t *aa_out_host, mg_orfcall *recs_host, void *stream);
 int mg_orfcall_emit_device(mg_genome *g, uint8_t *aa_out_dev, mg_orfcall *recs_dev, void *stream);
 
+/* ---- gene-model check of a prepared plan (start / stop codons, in-frame stops, reading frame, splice sites, codon usage).
+ * Record r's payload S is its clamped segments in emission order, each reverse-complemented by its strand: the bytes the
+ * nucleotide emit writes without framing.  skip = rec_phase[r] when MG_PROT_USE_PHASE is given and it is 0..2, else 0 (never
+ * trimX).  Codon i is S[skip+3i, skip+3i+3) for i < n_codons = max(0, (len(S) - skip) / 3); rem = (len(S) - skip) mod 3, or 0
+ * when len(S) <= skip.  A codon with a base outside A/C/G/T (either case) is ambiguous: never a start or a stop, not counted in
+ * codon usage or GC.  A stop is a codon the plan's codon table (mg_plan_set_codon_table, default table 1) maps to '*'; a start is
+ * a codon flagged in start64 (as in mg_orfcall_count).
+ * Junction between segments k and k+1 of a record (caller's segment indices, emission order, both clamped like the plan and not
+ * empty, same contig and strand): '+' intron [b_k, a_{k+1}), donor = bases b_k, b_k+1, acceptor = a_{k+1}-2, a_{k+1}-1; '-' intron
+ * [b_{k+1}, a_k), donor = reverse complement of a_k-2, a_k-1, acceptor = reverse complement of b_{k+1}, b_{k+1}+1.  The intron
+ * must hold at least 4 bases.  Class 1 = GT-AG, 2 = GC-AG, 3 = AT-AC, 4 = any other pair (case ignored, a base outside ACGT
+ * gives 4), 0 = no junction (last segment, empty segment, contig or strand change, gap under 4 bases, overlap, wrong order).
+ * The chunks mg_plan_create makes of a segment of 2^31 bases or more are not junctions.                                     */
+typedef struct {
+    int64_t nuc_len;              /* len(S)                                                                  */
+    int64_t gc;                   /* G/C bases in unambiguous codons                                         */
+    int32_t n_codons;
+    int32_t n_ambig;              /* ambiguous codons                                                        */
+    int32_t n_stop;               /* stop codons, the terminal one included                                  */
+    int32_t first_stop;           /* codon index of the first stop, -1 = none                                */
+    int32_t gc3;                  /* unambiguous codons whose third base is G or C                           */
+    int32_t n_junction;           /* junctions of class 1..4                                                 */
+    int32_t n_noncanonical;       /* junctions of class 4                                                    */
+    int32_t flags;                /* MG_CHK_*                                                                */
+    int8_t  skip;
+    int8_t  rem;
+    uint8_t start_codon;          /* 16*b0 + 4*b1 + b2 of codon 0, 0xFF = absent or ambiguous                 */
+    uint8_t stop_codon;           /* the same for the last complete codon                                    */
+    int32_t pad;
+} mg_cds_check;                   /* 56 bytes                                                                */
+#define MG_CHK_NO_START            1   /* codon 0 absent, ambiguous or not a start                                */
+#define MG_CHK_NO_STOP             2   /* no complete codon, or the last one is not a stop                        */
+#define MG_CHK_INTERNAL_STOP       4   /* a stop before the last codon (n_stop - terminal > 0)                     */
+#define MG_CHK_PARTIAL_CODON       8   /* rem != 0                                                                 */
+#define MG_CHK_NONCANONICAL_SPLICE 16  /* a junction of class 4                                                    */
+#define MG_CHK_AMBIGUOUS           32  /* an ambiguous codon                                                       */
+#define MG_CHK_EMPTY               64  /* n_codons == 0                                                            */
+/* rec_out[n_rec]; codon_counts[64 * r + 16*b0 + 4*b1 + b2] (n_rec x 64, may be NULL: not computed); junction[e] = class of the
+ * junction after caller segment e (n_seg entries of the table given to mg_plan_create, may be NULL).  flags: 0 or
+ * MG_PROT_USE_PHASE.  start64 is a host table as in mg_orfcall_count (NULL = ATG), checked against the plan's code and passed to
+ * the kernels by value.  Needs a plan prepared on the genome as it is (MG_ESTATE otherwise); MG_PROT_DEFER is enough.
+ * mg_plan_check_device takes device pointers for the three outputs and queues everything on `stream` without a host round trip
+ * (a CUDA graph can capture it); mg_plan_check takes host pointers and copies in stream order (sync before reading).
+ * The stop set of the plan's code and the start set are passed to the kernels by value: a captured check keeps the genetic
+ * code and the start codons it was captured with, whatever mg_plan_set_codon_table is called later (capture it again).                                                                                                              */
+int mg_plan_check(mg_plan *p, int flags, const uint8_t *start64, mg_cds_check *rec_out, uint32_t *codon_counts, int8_t *junction,
+                  void *stream);
+int mg_plan_check_device(mg_plan *p, int flags, const uint8_t *start64, mg_cds_check *rec_out, uint32_t *codon_counts,
+                         int8_t *junction, void *stream);
+
 /* ---- host side: native GFF3 / GTF reader + flattener (no GPU work; csrc/mg_gff.cu) ------------------------------------------
  * mg_gff_parse replaces read_gff (genome.py:242-415: line filter, version detection, attribute parsing, ID naming, de-dup,
  * implicit parents, child lists) on interned integer ids; `opts` is the option blob magot_b200/gffnative.py packs (format

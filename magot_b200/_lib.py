@@ -33,6 +33,18 @@ class MgOrfCall(ctypes.Structure):
                 ("hi", ctypes.c_int64), ("len", ctypes.c_int64), ("aa_off", ctypes.c_int64)]
 
 
+class MgCdsCheck(ctypes.Structure):
+    """mg_cds_check (include/magot_b200.h)."""
+    _fields_ = [("nuc_len", ctypes.c_int64), ("gc", ctypes.c_int64), ("n_codons", ctypes.c_int32),
+                ("n_ambig", ctypes.c_int32), ("n_stop", ctypes.c_int32), ("first_stop", ctypes.c_int32),
+                ("gc3", ctypes.c_int32), ("n_junction", ctypes.c_int32), ("n_noncanonical", ctypes.c_int32),
+                ("flags", ctypes.c_int32), ("skip", ctypes.c_int8), ("rem", ctypes.c_int8), ("start_codon", ctypes.c_uint8),
+                ("stop_codon", ctypes.c_uint8), ("pad", ctypes.c_int32)]
+
+
+#: MG_CHK_* flag bits of mg_cds_check.flags, in bit order (the names genome_tools check_cds prints)
+CHK_FLAGS = ("NO_START", "NO_STOP", "INTERNAL_STOP", "PARTIAL_CODON", "NONCANONICAL_SPLICE", "AMBIGUOUS", "EMPTY")
+
 if not os.path.isfile(LIB_PATH):
     raise ImportError(
         "magot_b200: %s is missing -- build it with `python -c 'import __graft_entry__ as g; g.build()'` "
@@ -91,6 +103,8 @@ SIGNATURES = {
     "mg_orfcall_count": (_i32, [_vp, _i64, _vp, _i64, _vp, _vp, _i32, _pi64, _pi64, _vp]),
     "mg_orfcall_emit": (_i32, [_vp, _vp, _vp, _vp]),
     "mg_orfcall_emit_device": (_i32, [_vp, _vp, _vp, _vp]),
+    "mg_plan_check": (_i32, [_vp, _i32, _vp, _vp, _vp, _vp, _vp]),
+    "mg_plan_check_device": (_i32, [_vp, _i32, _vp, _vp, _vp, _vp, _vp]),
     "mg_stream_sync": (_i32, [_i32, _vp]),
     "mg_copy_d2h_async": (_i32, [_i32, _vp, _vp, _i64, _vp]),
     "mg_tune": (_i32, [ctypes.c_char_p, _i32]),

@@ -151,8 +151,21 @@ struct mg_plan {
     int64_t out_cap = 0;
     uint8_t *d_aa8192 = nullptr;              // the plan's own translation tables (mg_plan_set_codon_table): plain | mg_aa_slot order
     bool own_code = false;                    // true: K3 / K23 / the one-launch emit read d_aa8192 instead of the genome's tables
+    uint64_t stop_mask = 0;                   // stop codons of the plan's code, bit 16*b0 + 4*b1 + b2 (mg_plan_check)
+    // the caller's segment table as given to mg_plan_create (mg_plan_check reports junctions per caller segment); the same
+    // pointers as the plan's own table unless a segment of 2^31 bases or more was split into chunks
+    int64_t n_cseg = 0;
+    int64_t *d_crec_seg_off = nullptr;
+    int32_t *d_cseg_contig = nullptr;
+    int64_t *d_cseg_start = nullptr, *d_cseg_end = nullptr;
+    int8_t *d_cseg_strand = nullptr;
+    mg_cds_check *d_chk = nullptr;            // device outputs of the host-buffer mg_plan_check
+    uint32_t *d_chk_counts = nullptr;
+    int8_t *d_chk_junction = nullptr;
     std::vector<void *> owned;                // everything to free
 };
+
+#define MG_STD_STOPS ((1ull << 48) | (1ull << 50) | (1ull << 56))   // TAA TAG TGA, bit 16*b0 + 4*b1 + b2 (A=0 C=1 G=2 T=3)
 
 #define MG_KIND_FWD 0ull
 #define MG_KIND_RC 1ull

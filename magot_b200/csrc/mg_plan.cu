@@ -577,6 +577,10 @@ extern "C" int mg_plan_create(mg_genome *g, int64_t n_rec, const int64_t *rec_se
     std::vector<int64_t> x_rec_seg_off, x_start, x_end;
     std::vector<int32_t> x_contig;
     std::vector<int8_t> x_strand;
+    const int64_t n_cseg = n_seg;                     // the caller's table (mg_plan_check reports junctions per caller segment)
+    const int64_t *c_rec_seg_off = rec_seg_off, *c_start = seg_start, *c_end = seg_end;
+    const int32_t *c_contig = seg_contig;
+    const int8_t *c_strand = seg_strand;
     if (any_long) {
         x_rec_seg_off.reserve(n_rec + 1);
         x_rec_seg_off.push_back(0);
@@ -637,6 +641,18 @@ extern "C" int mg_plan_create(mg_genome *g, int64_t n_rec, const int64_t *rec_se
         p->d_lit = d + 64;
     }
     if (rec_phase) TRY(upload(p, &p->d_rec_phase, rec_phase, n_rec, st));
+    p->n_cseg = n_cseg;
+    if (any_long) {
+        TRY(upload(p, &p->d_crec_seg_off, c_rec_seg_off, n_rec + 1, st));
+        TRY(upload(p, &p->d_cseg_contig, c_contig, n_cseg, st));
+        TRY(upload(p, &p->d_cseg_start, c_start, n_cseg, st));
+        TRY(upload(p, &p->d_cseg_end, c_end, n_cseg, st));
+        TRY(upload(p, &p->d_cseg_strand, c_strand, n_cseg, st));
+    } else {
+        p->d_crec_seg_off = p->d_rec_seg_off; p->d_cseg_contig = p->d_seg_contig; p->d_cseg_start = p->d_seg_start;
+        p->d_cseg_end = p->d_seg_end; p->d_cseg_strand = p->d_seg_strand;
+    }
+    p->stop_mask = MG_STD_STOPS;
     TRY(dalloc(p, &p->d_blk_r0, (p->n_piece + PLAN_TILE - 1) / PLAN_TILE + 1, st));
     {   // the nucleotide text size, from the clamped lengths above
         const int64_t up = nuc_bytes;
@@ -680,9 +696,11 @@ extern "C" int mg_plan_destroy(mg_plan *p) {
 // captured in a graph later reads a table that is already on the device; codon64 == NULL goes back to the genome's table.
 extern "C" int mg_plan_set_codon_table(mg_plan *p, const uint8_t *codon64) {
     MG_REQUIRE(p != nullptr, "plan handle is NULL");
-    if (!codon64) { p->own_code = false; return MG_OK; }
+    if (!codon64) { p->own_code = false; p->stop_mask = MG_STD_STOPS; return MG_OK; }
     // the record pass drops a leading codon for trimX when it holds a base outside ACGT, i.e. where the table gives 'X'
     for (int c = 0; c < 64; c++) MG_REQUIRE(codon64[c] != 'X', "codon64 maps an A/C/G/T codon to 'X'");
+    uint64_t stops = 0;
+    for (int c = 0; c < 64; c++) if (codon64[c] == '*') stops |= 1ull << c;
     MG_CUDA(cudaSetDevice(p->device));
     uint8_t t[8192];
     build_aa4096(t, codon64);
@@ -695,6 +713,7 @@ extern "C" int mg_plan_set_codon_table(mg_plan *p, const uint8_t *codon64) {
     MG_CUDA(cudaMemcpyAsync(p->d_aa8192, t, 8192, cudaMemcpyHostToDevice, st));
     MG_CUDA(cudaStreamSynchronize(st));
     p->own_code = true;
+    p->stop_mask = stops;
     return MG_OK;
 }
 

@@ -22,6 +22,13 @@ from .tables import RecordTable  # noqa: F401  (re-exported: engine.RecordTable)
 
 _CHUNK = 64 << 20          # bases per mg_genome_pack call (multiple of 32)
 
+#: mg_cds_check (include/magot_b200.h) as a numpy record: the per-record result of Plan.check
+CHECK_DTYPE = np.dtype([("nuc_len", np.int64), ("gc", np.int64), ("n_codons", np.int32), ("n_ambig", np.int32),
+                        ("n_stop", np.int32), ("first_stop", np.int32), ("gc3", np.int32), ("n_junction", np.int32),
+                        ("n_noncanonical", np.int32), ("flags", np.int32), ("skip", np.int8), ("rem", np.int8),
+                        ("start_codon", np.uint8), ("stop_codon", np.uint8), ("pad", np.int32)])
+assert CHECK_DTYPE.itemsize == ctypes.sizeof(_lib.MgCdsCheck)
+
 
 def _ptr(a):
     return ctypes.c_void_p(a.ctypes.data) if a is not None else None
@@ -199,6 +206,23 @@ class Plan(object):
         aa = np.empty(n, dtype=np.int64)
         check(lib.mg_plan_lengths(self.handle, _ptr(nuc), _ptr(aa), self.stream))
         return nuc, aa
+
+    def check(self, start_codons=None, use_phase=False, codon_usage=False, junctions=False):
+        """Gene-model check of every record (mg_plan_check) under the plan's genetic code.  start_codons: 64 flags as
+        gencode.start64 gives them, None = ATG.  Returns (CHECK_DTYPE records, uint32 [n_rec, 64] codon counts or None,
+        int8 junction class per segment of the table or None).  Needs prepare() or prepare_async() first."""
+        n = self.table.n_rec
+        recs = np.zeros(n, dtype=CHECK_DTYPE)
+        counts = np.zeros((n, 64), dtype=np.uint32) if codon_usage else None
+        junc = np.zeros(self.table.n_seg, dtype=np.int8) if junctions else None
+        if start_codons is not None:
+            start_codons = bytes(start_codons)
+            if len(start_codons) != 64:
+                raise ValueError("start_codons must hold 64 flags")
+        check(lib.mg_plan_check(self.handle, _lib.MG_PROT_USE_PHASE if use_phase else 0, start_codons, _ptr(recs),
+                                _ptr(counts), _ptr(junc), self.stream))
+        check(lib.mg_stream_sync(self.genome.device, self.stream))
+        return recs, counts, junc
 
     def emit_host(self, protein=False, out=None):
         total = self.prot_total if protein else self.nuc_total

@@ -165,12 +165,25 @@ class Flattener(object):
                                   suf_len, lit, np.where(valid, ph[safe] if ph.size else 0, 0).astype(np.int8))
 
     def run(self, seq_type, codon64=None):
+        tbl, rec_ids, protein = self.records(seq_type)
+        if tbl is None:
+            return ""
+        eng = self.gs._engine()
+        text, l2 = eng.run_table(tbl, protein=protein, want_lengths=protein, codon64=codon64)
+        if protein and l2 is not None and (l2[1] < 0)[np.asarray(rec_ids) >= 0].any():
+            # Sequence.translate returned None (spliced length <= 2): '>' + name + '\n' + None (genome.py:710)
+            raise TypeError("cannot concatenate 'str' and 'NoneType' objects")
+        return engine.decode_text(text, strip_last=1)
+
+    def records(self, seq_type):
+        """(RecordTable, leaf id per record (-1 = blank line), protein) of what run(seq_type) prints, or (None, [], False)
+        without tops.  The `longest` selection runs here (one length pass on the device)."""
         if seq_type not in ("nucleotide", "protein"):
             if any(t.entries for t in self.tops if not t.genomic):
                 print(seq_type + ' is not valid seq_type. Please specify "protein" or "nucleotide".')
                 raise UnboundLocalError("local variable 'new_seq' referenced before assignment")
         if not self.tops:
-            return ""
+            return None, [], False
         eng = self.gs._engine()
         any_longest = any(t.longest for t in self.tops)
         # genomic records are always nucleotide text (genome.py:680-682 ignores seq_type); they cannot be
@@ -208,9 +221,4 @@ class Flattener(object):
                 rec_ids.append(rid)
                 pre.append(b">" + self.names[rid].encode("latin-1") + b"\n")
                 suf.append(b"\n\n" if top.genomic else b"\n")
-        tbl = self._table(rec_ids, pre, suf)
-        text, l2 = eng.run_table(tbl, protein=protein, want_lengths=protein, codon64=codon64)
-        if protein and l2 is not None and (l2[1] < 0)[np.asarray(rec_ids) >= 0].any():
-            # Sequence.translate returned None (spliced length <= 2): '>' + name + '\n' + None (genome.py:710)
-            raise TypeError("cannot concatenate 'str' and 'NoneType' objects")
-        return engine.decode_text(text, strip_last=1)
+        return self._table(rec_ids, pre, suf), rec_ids, protein

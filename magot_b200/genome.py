@@ -18,6 +18,7 @@ Reference API kept (file:line in /root/reference/genome.py):
 Record order: the reference iterates Python-2.7 dicts; `RECORD_ORDER = "py2"` (default) replays
 that order (magot_b200.py2dict) so whole files are byte-identical; "insertion" keeps file order.
 """
+import collections
 import io
 import os
 
@@ -728,6 +729,54 @@ class AnnotationSet(object):
         return fl.run(seq_type, codon64=codon64)
 
 
+    def check_cds(self, feature, genetic_code=1, start_codons=("ATG",), use_phase=False, codon_usage=True, junctions=True):
+        """Gene-model check (mg_plan_check) of exactly the records get_fasta(feature, seq_type="protein") prints, in its
+        order: start / stop codons, in-frame stops, reading frame, ambiguous codons, GC, splice sites and codon usage under
+        NCBI table `genetic_code`.  start_codons: codons a CDS may start with; use_phase: start at the GFF phase of the first
+        CDS.  Returns CdsCheck(names, records (engine.CHECK_DTYPE), codon_counts (uint32 [n, 64] or None), junctions (int8
+        class after each segment, or None), seg_off (segments of record i: junctions[seg_off[i]:seg_off[i+1]])).  The names
+        are the records' FASTA headers without '>'."""
+        code = gencode.check(genetic_code)
+        starts = gencode.start64(start_codons, code)      # ValueError before any device work
+        model = _PENDING.get(self) if _PENDING else None
+        flat = _native_table(self, model, feature) if model is not None else None
+        if flat is not None:
+            gs, tbl = flat[0], flat[1]
+        else:
+            table = getattr(self, feature)
+            from .flatten import Flattener
+            fl = Flattener(self)
+            for key in table:
+                obj = table[key]
+                if not hasattr(obj, "get_fasta"):
+                    raise AttributeError("%s instance has no attribute 'get_fasta'" % obj.__class__.__name__)
+                fl.add_top(obj, seq_type="protein", longest=False, genomic=False, name_from='ID')
+            gs = fl.gs
+            tbl = fl.records("protein")[0]
+        if tbl is None or tbl.n_rec == 0:
+            return CdsCheck([], np.zeros(0, dtype=engine.CHECK_DTYPE), np.zeros((0, 64), np.uint32) if codon_usage else None,
+                            np.zeros(0, np.int8) if junctions else None, np.zeros(1, np.int64))
+        plan = engine.Plan(gs._engine().primary, tbl)
+        try:
+            if code != 1:
+                plan.set_codon_table(gencode.codon64(code))
+            plan.prepare_async(trimx=False, defer_records=True)     # the check needs the piece pass only
+            recs, counts, junc = plan.check(starts, use_phase=use_phase, codon_usage=codon_usage, junctions=junctions)
+        finally:
+            plan.close()
+        keep = np.flatnonzero(tbl.rec_pre_len > 0)        # FASTA records; the blank entries of empty tops have no header
+        lit = tbl.lit.tobytes()
+        names = [lit[o + 1:o + n - 1].decode("latin-1") for o, n in zip(tbl.rec_lit_off[keep].tolist(), tbl.rec_pre_len[keep].tolist())]
+        nseg = np.diff(tbl.rec_seg_off)[keep]
+        seg_off = np.concatenate(([0], np.cumsum(nseg))).astype(np.int64)
+        if junc is not None:
+            rows = np.concatenate([np.arange(tbl.rec_seg_off[r], tbl.rec_seg_off[r + 1]) for r in keep.tolist()]) if keep.size else np.zeros(0, np.int64)
+            junc = junc[rows.astype(np.int64)]
+        return CdsCheck(names, recs[keep], counts[keep] if counts is not None else None, junc, seg_off)
+
+
+CdsCheck = collections.namedtuple("CdsCheck", "names records codon_counts junctions seg_off")
+
 _ASET_CLASS_NAMES = frozenset(dir(AnnotationSet))
 
 
@@ -753,12 +802,33 @@ def _native_get_fasta(annotation_set, model, feature, seq_type, longest, genomic
     longest=, an unknown table, a model the flattener refuses: the object path then prints / raises like the reference)."""
     if genomic is True or longest is True or seq_type not in ("nucleotide", "protein") or not isinstance(feature, str):
         return None
+    import time as _time
+    t0 = _time.perf_counter()
+    flat = _native_table(annotation_set, model, feature)
+    if flat is None:
+        return None
+    gs, tbl, rec_name = flat
+    protein = seq_type == "protein"
+    t1 = _time.perf_counter()
+    text, lens = gs._engine().run_table(tbl, protein=protein, want_lengths=protein, codon64=codon64)
+    t2 = _time.perf_counter()
+    if protein and lens is not None and ((lens[1] < 0) & (rec_name >= 0)).any():
+        # Sequence.translate returned None (spliced length <= 2): '>' + name + '\n' + None (genome.py:710)
+        raise TypeError("cannot concatenate 'str' and 'NoneType' objects")
+    out = engine.decode_text(text, strip_last=1)
+    if TIMINGS is not None:
+        TIMINGS.update({"flatten_s": t1 - t0, "device_and_copy_s": t2 - t1, "decode_s": _time.perf_counter() - t2,
+                        "records": int(tbl.n_rec), "segments": int(tbl.n_seg), "text_bytes": len(text)})
+    return out
+
+
+def _native_table(annotation_set, model, feature):
+    """(genome sequence, RecordTable, rec_name ids) of AnnotationSet.get_fasta(feature) on the native model, framed as the
+    FASTA text; None when the call needs the object model."""
     genome = object.__getattribute__(annotation_set, "__dict__").get("genome")
     gs = getattr(genome, "genome_sequence", None) if genome is not None else None
     if gs is None:
         return None
-    import time as _time
-    t0 = _time.perf_counter()
     rows = model.table_rows(feature)
     if rows is None or rows.size == 0:
         return None
@@ -776,18 +846,7 @@ def _native_get_fasta(annotation_set, model, feature, seq_type, longest, genomic
     tbl, top_rec_off, rec_name = model.flatten(tops, contig_of, framing=True)
     if tbl is None:
         return None
-    protein = seq_type == "protein"
-    t1 = _time.perf_counter()
-    text, lens = gs._engine().run_table(tbl, protein=protein, want_lengths=protein, codon64=codon64)
-    t2 = _time.perf_counter()
-    if protein and lens is not None and ((lens[1] < 0) & (rec_name >= 0)).any():
-        # Sequence.translate returned None (spliced length <= 2): '>' + name + '\n' + None (genome.py:710)
-        raise TypeError("cannot concatenate 'str' and 'NoneType' objects")
-    out = engine.decode_text(text, strip_last=1)
-    if TIMINGS is not None:
-        TIMINGS.update({"flatten_s": t1 - t0, "device_and_copy_s": t2 - t1, "decode_s": _time.perf_counter() - t2,
-                        "records": int(tbl.n_rec), "segments": int(tbl.n_seg), "text_bytes": len(text)})
-    return out
+    return gs, tbl, rec_name
 
 
 def write_gff(annotation_set, gff_format="simple gff3"):

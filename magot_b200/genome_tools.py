@@ -11,7 +11,8 @@ get_seq_from_fasta :483, exclude_from_fasta :377, extract_upstream_downstream :4
 blast_csv2fasta :265, exonerate2fasta :274, mask_from_gff :394, convert_gff :527,
 dna2orfs :145 (the reference's version cannot run -- it calls str.translate with keyword
 arguments -- this one does what it intended, on the device).  New: call_orfs, start-to-stop
-ORF calling with genome coordinates (GFF3, protein or CDS nucleotide output).  The dispatcher (main :25-45)
+ORF calling with genome coordinates (GFF3, protein or CDS nucleotide output), and check_cds, a gene-model check (start /
+stop codons, in-frame stops, frame, splice sites, codon usage).  The dispatcher (main :25-45)
 keeps the grammar but looks the function up in a table instead of eval()-ing a string.
 """
 import sys
@@ -361,9 +362,95 @@ def call_orfs(fasta, min_orf="100", genetic_code="1", start_codons="ATG", partia
     sys.stdout.write("\n".join(lines) + "\n" if lines else "")
 
 
+CHECK_FORMATS = ("tsv", "codon_usage")
+CHECK_HEADER = "\t".join(("#ID", "nuc_len", "codons", "skip", "rem", "start", "stop", "internal_stops", "first_internal_stop",
+                          "ambiguous", "gc", "gc3", "junctions", "noncanonical", "status"))
+CODON_USAGE_HEADER = "\t".join(("#codon", "residue", "count", "per_thousand", "fraction"))
+
+
+def _codon_text(idx):
+    """Codon 16*b0 + 4*b1 + b2 (A=0 C=1 G=2 T=3) as text; '.' for 0xFF (absent or ambiguous)."""
+    idx = int(idx)
+    return "." if idx == 0xFF else "ACGT"[idx >> 4] + "ACGT"[(idx >> 2) & 3] + "ACGT"[idx & 3]
+
+
+def _check_status(flags):
+    """'ok', or the names of the set MG_CHK_* bits joined by commas, in bit order."""
+    flags = int(flags)
+    names = [n for k, n in enumerate(engine._lib.CHK_FLAGS) if flags >> k & 1]
+    return ",".join(names) if names else "ok"
+
+
+def _check_tsv_lines(names, recs):
+    """check_cds out_format=tsv: the header, then one line per record (engine.CHECK_DTYPE) with the columns of CHECK_HEADER.
+    internal_stops = n_stop less the terminal stop; first_internal_stop is the codon index of the first stop when there is an
+    internal one, else '.'; gc = G/C bases over the bases of unambiguous codons, gc3 = G/C third bases over unambiguous codons,
+    both with 4 decimals ('.' without an unambiguous codon)."""
+    lines = [CHECK_HEADER]
+    for name, r in zip(names, recs):
+        terminal = 0 if int(r["flags"]) & 2 else 1
+        internal = int(r["n_stop"]) - terminal
+        unamb = int(r["n_codons"]) - int(r["n_ambig"])
+        gc = "%.4f" % (int(r["gc"]) / (3.0 * unamb)) if unamb else "."
+        gc3 = "%.4f" % (int(r["gc3"]) / float(unamb)) if unamb else "."
+        lines.append("\t".join((name, str(int(r["nuc_len"])), str(int(r["n_codons"])), str(int(r["skip"])), str(int(r["rem"])),
+                                _codon_text(r["start_codon"]), _codon_text(r["stop_codon"]), str(internal),
+                                str(int(r["first_stop"])) if internal > 0 else ".", str(int(r["n_ambig"])), gc, gc3,
+                                str(int(r["n_junction"])), str(int(r["n_noncanonical"])), _check_status(r["flags"]))))
+    return lines
+
+
+def _codon_usage_lines(counts, genetic_code):
+    """check_cds out_format=codon_usage: the header, then the 64 codons in NCBI order (TTT, TTC, TTA, TTG, TCT, ...): codon,
+    residue under the code ('*' = stop), count, per thousand codons counted (2 decimals) and fraction of the codons of the same
+    residue (4 decimals); '.' where the denominator is 0.  counts: 64 totals indexed 16*b0 + 4*b1 + b2 (A=0 C=1 G=2 T=3)."""
+    counts = [int(c) for c in counts]
+    table = gencode.TABLES[gencode.check(genetic_code)]
+    total = sum(counts)
+    family = {}
+    for i, aa in enumerate(table):
+        c = "TCAG"[i >> 4] + "TCAG"[(i >> 2) & 3] + "TCAG"[i & 3]
+        family[aa] = family.get(aa, 0) + counts["ACGT".index(c[0]) * 16 + "ACGT".index(c[1]) * 4 + "ACGT".index(c[2])]
+    lines = [CODON_USAGE_HEADER]
+    for i, aa in enumerate(table):
+        c = "TCAG"[i >> 4] + "TCAG"[(i >> 2) & 3] + "TCAG"[i & 3]
+        n = counts["ACGT".index(c[0]) * 16 + "ACGT".index(c[1]) * 4 + "ACGT".index(c[2])]
+        lines.append("\t".join((c, aa, str(n), "%.2f" % (1000.0 * n / total) if total else ".",
+                                "%.4f" % (float(n) / family[aa]) if family[aa] else ".")))
+    return lines
+
+
+def check_cds(genome_sequence, gff, feature="gene", genetic_code="1", start_codons="ATG", use_phase="False", out_format="tsv",
+              only_ok="False"):
+    """Gene-model check of every record `gff2fasta ... seq_type=protein` would print (new): start and stop codon, in-frame
+    stops, reading frame, ambiguous codons, GC, splice-site consensus and codon usage, on the device.  start_codons:
+    comma-separated codons a CDS may start with (default ATG); use_phase=True starts at the GFF phase of the first CDS;
+    genetic_code: NCBI table id.  out_format=tsv prints a header line and one tab-separated line per record (see
+    _check_tsv_lines): ID, nuc_len, codons, skip, rem, start, stop, internal_stops, first_internal_stop, ambiguous, gc, gc3,
+    junctions, noncanonical, status ('ok' or the comma-joined flags NO_START, NO_STOP, INTERNAL_STOP, PARTIAL_CODON,
+    NONCANONICAL_SPLICE, AMBIGUOUS, EMPTY).  out_format=codon_usage prints a header line and the 64 codons in NCBI order (see
+    _codon_usage_lines), summed over the records.  only_ok=True keeps only the records without a flag, in both formats."""
+    code = gencode.check(genetic_code)
+    if out_format not in CHECK_FORMATS:
+        raise ValueError("out_format %r is not one of %s" % (out_format, ", ".join(CHECK_FORMATS)))
+    codons = start_codons.split(",") if isinstance(start_codons, str) else list(start_codons)
+    gencode.start64(codons, code)                            # ValueError before any device work
+    phase, ok_only = _truth(use_phase), _truth(only_ok)
+    my_genome = genome.Genome(genome_sequence)
+    my_genome.read_gff(gff)
+    res = my_genome.annotations.check_cds(feature, genetic_code=code, start_codons=codons, use_phase=phase,
+                                          codon_usage=out_format == "codon_usage", junctions=False)
+    keep = np.flatnonzero(res.records["flags"] == 0) if ok_only else np.arange(len(res.names))
+    if out_format == "tsv":
+        lines = _check_tsv_lines([res.names[i] for i in keep.tolist()], res.records[keep])
+    else:
+        lines = _codon_usage_lines(res.codon_counts[keep].sum(axis=0, dtype=np.int64), code)
+    sys.stdout.write("\n".join(lines) + "\n")
+
+
 FUNCTIONS = {f.__name__: f for f in (gff2fasta, cds2pep, coords2fasta, get_seq_from_fasta, exclude_from_fasta,
                                      extract_upstream_downstream, dna2orfs, blast_csv2fasta, exonerate2fasta, mask_from_gff,
-                                     convert_gff, call_orfs)}
+                                     convert_gff, call_orfs, check_cds)}
 
 
 def help_func():
