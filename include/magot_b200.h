@@ -317,6 +317,47 @@ int mg_plan_check(mg_plan *p, int flags, const uint8_t *start64, mg_cds_check *r
 int mg_plan_check_device(mg_plan *p, int flags, const uint8_t *start64, mg_cds_check *rec_out, uint32_t *codon_counts,
                          int8_t *junction, void *stream);
 
+/* ---- CDS prediction of a prepared plan: the longest ORF of every record's spliced payload, mapped back to genome CDS segments
+ * (TransDecoder.LongOrfs style, one ORF per record).  Record r's payload S is the one of mg_plan_check; n = len(S).
+ * A codon starts at every position i with i + 3 <= n; its frame is i mod 3.  Case is ignored and a codon with a base outside
+ * A/C/G/T is neither a start nor a stop.  A stop is a codon the plan's code (mg_plan_set_codon_table) maps to '*'; a start is a
+ * codon flagged in start64 (NULL = ATG; at least one codon, no stop, as mg_orfcall_count checks it).
+ * Stretches: in frame f the stops cut the codons f, f+3, ... into stretches.  A stretch ends at a stop (included) or at the
+ * frame's last complete codon (an open 3' end); the first stretch of a frame begins at codon f (an open 5' end), every later
+ * one right after a stop.  A stretch's ORF starts at its first start codon b -- with MG_PRED_5PARTIAL the first stretch of a
+ * frame starts at its first codon instead, start codon or not -- and ends after the stop, or after the frame's last complete
+ * codon for an open 3' end, which is kept only with MG_PRED_3PARTIAL.  n_aa counts the codons from the start up to, not
+ * including, the stop; a candidate needs n_aa >= max(1, min_aa).  Type bit 0 (5' partial): the first codon is not a start
+ * codon; bit 1 (3' partial): there is no stop.  Each record gets the candidate with the largest n_aa, ties broken by the
+ * smallest start; a record without a candidate reports none (lo = hi = -1, n_aa = 0, frame = -1, type = 0, codons 0xFF).
+ * Mapping: caller segment e of the record (the table given to mg_plan_create; the chunks it makes of a segment of 2^31 bases
+ * or more are never visible), clamped as the plan clamps it to [cl, ch), covers payload range [o_e, o_e + len_e).  With
+ * [x, y) its intersection with the ORF's [lo, hi): on '+' its forward interval is [cl + x - o_e, cl + y - o_e), on '-'
+ * [ch - (y - o_e), ch - (x - o_e)); its GFF3 phase is (3 - (x - lo) mod 3) mod 3.  Segments the ORF does not touch (and
+ * every segment of a record without an ORF) are reported empty: lo = hi = phase = -1.                                   */
+#define MG_PRED_5PARTIAL 1
+#define MG_PRED_3PARTIAL 2
+typedef struct {
+    int64_t lo, hi;               /* ORF in S, [lo, hi), stop included; -1, -1 = none                        */
+    int32_t n_aa;                 /* residues, stop excluded; 0 = none                                       */
+    int8_t  frame;                /* lo mod 3                                                                */
+    int8_t  type;                 /* bit 0: 5' partial, bit 1: 3' partial                                    */
+    uint8_t start_codon;          /* codon at lo, 16*b0+4*b1+b2; 0xFF = none or ambiguous                    */
+    uint8_t stop_codon;           /* codon at hi-3 when there is a stop, else 0xFF                           */
+    int32_t n_cds_seg;            /* caller segments the ORF touches                                         */
+    int32_t pad;
+} mg_cds_pred;                    /* 32 bytes */
+typedef struct { int64_t lo, hi; int8_t phase; int8_t pad[7]; } mg_cds_seg;   /* 0-based half-open forward coords; -1,-1,-1 = empty */
+/* rec_out[n_rec]; seg_out[n_seg] (one entry per caller segment, may be NULL).  flags: MG_PRED_5PARTIAL | MG_PRED_3PARTIAL.
+ * Rules of mg_plan_check: a prepared plan on the genome as it is (MG_ESTATE otherwise; MG_PROT_DEFER is enough), the stop set
+ * and the start set passed to the kernels by value.  mg_plan_predict_cds takes host outputs and copies them in stream order
+ * (sync before reading; its device scratch grows outside a capture only); mg_plan_predict_cds_device takes device outputs and
+ * queues two launches on `stream` with no host round trip, so a CUDA graph can capture it.                                */
+int mg_plan_predict_cds(mg_plan *p, int64_t min_aa, const uint8_t *start64, int flags,
+                        mg_cds_pred *rec_out, mg_cds_seg *seg_out, void *stream);
+int mg_plan_predict_cds_device(mg_plan *p, int64_t min_aa, const uint8_t *start64, int flags,
+                               mg_cds_pred *rec_out, mg_cds_seg *seg_out, void *stream);
+
 /* ---- host side: native GFF3 / GTF reader + flattener (no GPU work; csrc/mg_gff.cu) ------------------------------------------
  * mg_gff_parse replaces read_gff (genome.py:242-415: line filter, version detection, attribute parsing, ID naming, de-dup,
  * implicit parents, child lists) on interned integer ids; `opts` is the option blob magot_b200/gffnative.py packs (format

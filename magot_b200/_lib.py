@@ -13,6 +13,8 @@ LIB_PATH = os.environ.get("MAGOT_B200_LIB") or os.path.join(_HERE, "libmagot_b20
 MG_PROT_TRIMX = 1
 MG_PROT_USE_PHASE = 2
 MG_PROT_DEFER = 4
+MG_PRED_5PARTIAL = 1
+MG_PRED_3PARTIAL = 2
 
 
 class MagotError(RuntimeError):
@@ -41,6 +43,21 @@ class MgCdsCheck(ctypes.Structure):
                 ("flags", ctypes.c_int32), ("skip", ctypes.c_int8), ("rem", ctypes.c_int8), ("start_codon", ctypes.c_uint8),
                 ("stop_codon", ctypes.c_uint8), ("pad", ctypes.c_int32)]
 
+
+class MgCdsPred(ctypes.Structure):
+    """mg_cds_pred (include/magot_b200.h)."""
+    _fields_ = [("lo", ctypes.c_int64), ("hi", ctypes.c_int64), ("n_aa", ctypes.c_int32), ("frame", ctypes.c_int8),
+                ("type", ctypes.c_int8), ("start_codon", ctypes.c_uint8), ("stop_codon", ctypes.c_uint8),
+                ("n_cds_seg", ctypes.c_int32), ("pad", ctypes.c_int32)]
+
+
+class MgCdsSeg(ctypes.Structure):
+    """mg_cds_seg (include/magot_b200.h)."""
+    _fields_ = [("lo", ctypes.c_int64), ("hi", ctypes.c_int64), ("phase", ctypes.c_int8), ("pad", ctypes.c_int8 * 7)]
+
+
+#: orf_type text of mg_cds_pred.type (bit 0: 5' partial, bit 1: 3' partial)
+ORF_TYPES = ("complete", "5prime_partial", "3prime_partial", "internal")
 
 #: MG_CHK_* flag bits of mg_cds_check.flags, in bit order (the names genome_tools check_cds prints)
 CHK_FLAGS = ("NO_START", "NO_STOP", "INTERNAL_STOP", "PARTIAL_CODON", "NONCANONICAL_SPLICE", "AMBIGUOUS", "EMPTY")
@@ -105,6 +122,8 @@ SIGNATURES = {
     "mg_orfcall_emit_device": (_i32, [_vp, _vp, _vp, _vp]),
     "mg_plan_check": (_i32, [_vp, _i32, _vp, _vp, _vp, _vp, _vp]),
     "mg_plan_check_device": (_i32, [_vp, _i32, _vp, _vp, _vp, _vp, _vp]),
+    "mg_plan_predict_cds": (_i32, [_vp, _i64, _vp, _i32, _vp, _vp, _vp]),
+    "mg_plan_predict_cds_device": (_i32, [_vp, _i64, _vp, _i32, _vp, _vp, _vp]),
     "mg_stream_sync": (_i32, [_i32, _vp]),
     "mg_copy_d2h_async": (_i32, [_i32, _vp, _vp, _i64, _vp]),
     "mg_tune": (_i32, [ctypes.c_char_p, _i32]),

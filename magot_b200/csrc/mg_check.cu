@@ -390,9 +390,7 @@ __global__ void __launch_bounds__(256) k_check_final(int64_t n_rec, uint64_t sto
 
 // ---- host API -----------------------------------------------------------------------------------------------
 
-static int check_args(mg_plan *p, int flags, const uint8_t *start64, uint64_t *start_mask) {
-    MG_REQUIRE(p != nullptr, "plan handle is NULL");
-    MG_REQUIRE((flags & ~MG_PROT_USE_PHASE) == 0, "flags: only MG_PROT_USE_PHASE is accepted");
+int mg_start_mask(const mg_plan *p, const uint8_t *start64, uint64_t *start_mask) {
     uint64_t m = 0;
     if (!start64) {
         m = 1ull << 14;                                // ATG: 16*0 + 4*3 + 2 (A=0 C=1 G=2 T=3)
@@ -408,6 +406,13 @@ static int check_args(mg_plan *p, int flags, const uint8_t *start64, uint64_t *s
         MG_REQUIRE(m != 0, "start64 flags no start codon");
     }
     *start_mask = m;
+    return MG_OK;
+}
+
+static int check_args(mg_plan *p, int flags, const uint8_t *start64, uint64_t *start_mask) {
+    MG_REQUIRE(p != nullptr, "plan handle is NULL");
+    MG_REQUIRE((flags & ~MG_PROT_USE_PHASE) == 0, "flags: only MG_PROT_USE_PHASE is accepted");
+    if (const int rc = mg_start_mask(p, start64, start_mask)) return rc;
     return mg_plan_check_prepared(p);
 }
 

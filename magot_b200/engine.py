@@ -29,6 +29,15 @@ CHECK_DTYPE = np.dtype([("nuc_len", np.int64), ("gc", np.int64), ("n_codons", np
                         ("start_codon", np.uint8), ("stop_codon", np.uint8), ("pad", np.int32)])
 assert CHECK_DTYPE.itemsize == ctypes.sizeof(_lib.MgCdsCheck)
 
+#: mg_cds_pred (include/magot_b200.h): the per-record result of Plan.predict_cds
+PRED_DTYPE = np.dtype([("lo", np.int64), ("hi", np.int64), ("n_aa", np.int32), ("frame", np.int8), ("type", np.int8),
+                       ("start_codon", np.uint8), ("stop_codon", np.uint8), ("n_cds_seg", np.int32), ("pad", np.int32)])
+assert PRED_DTYPE.itemsize == ctypes.sizeof(_lib.MgCdsPred)
+
+#: mg_cds_seg: each caller segment's share of its record's predicted CDS (-1, -1, -1 = empty)
+CDSSEG_DTYPE = np.dtype([("lo", np.int64), ("hi", np.int64), ("phase", np.int8), ("pad", np.int8, (7,))])
+assert CDSSEG_DTYPE.itemsize == ctypes.sizeof(_lib.MgCdsSeg)
+
 
 def _ptr(a):
     return ctypes.c_void_p(a.ctypes.data) if a is not None else None
@@ -223,6 +232,21 @@ class Plan(object):
                                 _ptr(counts), _ptr(junc), self.stream))
         check(lib.mg_stream_sync(self.genome.device, self.stream))
         return recs, counts, junc
+
+    def predict_cds(self, min_aa, start_codons=None, partial5=False, partial3=False):
+        """Longest ORF of every record (mg_plan_predict_cds) under the plan's genetic code.  start_codons: 64 flags as
+        gencode.start64 gives them, None = ATG; partial5 / partial3: also ORFs open at the frame's 5' end / without a stop.
+        Returns (PRED_DTYPE records, CDSSEG_DTYPE entry per segment of the table).  Needs prepare() or prepare_async() first."""
+        recs = np.zeros(self.table.n_rec, dtype=PRED_DTYPE)
+        segs = np.zeros(self.table.n_seg, dtype=CDSSEG_DTYPE)
+        if start_codons is not None:
+            start_codons = bytes(start_codons)
+            if len(start_codons) != 64:
+                raise ValueError("start_codons must hold 64 flags")
+        flags = (_lib.MG_PRED_5PARTIAL if partial5 else 0) | (_lib.MG_PRED_3PARTIAL if partial3 else 0)
+        check(lib.mg_plan_predict_cds(self.handle, int(min_aa), start_codons, flags, _ptr(recs), _ptr(segs), self.stream))
+        check(lib.mg_stream_sync(self.genome.device, self.stream))
+        return recs, segs
 
     def emit_host(self, protein=False, out=None):
         total = self.prot_total if protein else self.nuc_total

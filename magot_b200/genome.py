@@ -738,21 +738,7 @@ class AnnotationSet(object):
         are the records' FASTA headers without '>'."""
         code = gencode.check(genetic_code)
         starts = gencode.start64(start_codons, code)      # ValueError before any device work
-        model = _PENDING.get(self) if _PENDING else None
-        flat = _native_table(self, model, feature) if model is not None else None
-        if flat is not None:
-            gs, tbl = flat[0], flat[1]
-        else:
-            table = getattr(self, feature)
-            from .flatten import Flattener
-            fl = Flattener(self)
-            for key in table:
-                obj = table[key]
-                if not hasattr(obj, "get_fasta"):
-                    raise AttributeError("%s instance has no attribute 'get_fasta'" % obj.__class__.__name__)
-                fl.add_top(obj, seq_type="protein", longest=False, genomic=False, name_from='ID')
-            gs = fl.gs
-            tbl = fl.records("protein")[0]
+        gs, tbl = _feature_table(self, feature, "protein")
         if tbl is None or tbl.n_rec == 0:
             return CdsCheck([], np.zeros(0, dtype=engine.CHECK_DTYPE), np.zeros((0, 64), np.uint32) if codon_usage else None,
                             np.zeros(0, np.int8) if junctions else None, np.zeros(1, np.int64))
@@ -765,8 +751,7 @@ class AnnotationSet(object):
         finally:
             plan.close()
         keep = np.flatnonzero(tbl.rec_pre_len > 0)        # FASTA records; the blank entries of empty tops have no header
-        lit = tbl.lit.tobytes()
-        names = [lit[o + 1:o + n - 1].decode("latin-1") for o, n in zip(tbl.rec_lit_off[keep].tolist(), tbl.rec_pre_len[keep].tolist())]
+        names = _record_names(tbl, keep)
         nseg = np.diff(tbl.rec_seg_off)[keep]
         seg_off = np.concatenate(([0], np.cumsum(nseg))).astype(np.int64)
         if junc is not None:
@@ -774,8 +759,100 @@ class AnnotationSet(object):
             junc = junc[rows.astype(np.int64)]
         return CdsCheck(names, recs[keep], counts[keep] if counts is not None else None, junc, seg_off)
 
+    def predict_cds(self, feature="gene", min_aa=100, genetic_code=1, start_codons=("ATG",), partial5=False, partial3=False,
+                    strand="sense"):
+        """CDS prediction (mg_plan_predict_cds) for exactly the records get_fasta(feature, seq_type="nucleotide") prints, in its
+        order, e.g. exon-only transcript models: the longest ORF of each spliced transcript in its three frames, at least
+        min_aa residues, from a codon in start_codons to a stop of NCBI table `genetic_code`; partial5 / partial3 also accept
+        ORFs open at the 5' end of a frame / without a stop.  strand="both" also scores the antisense (the reverse complement of
+        the transcript): per record the longer ORF wins, the sense one on a tie.  Returns CdsPrediction(names, records
+        (engine.PRED_DTYPE, coordinates in the chosen strand's transcript), antisense (int8, 1 where the antisense ORF was
+        chosen), seg_contig, seg_lo, seg_hi (0-based half-open forward coordinates), seg_strand (0 '+', 1 '-'), seg_phase: the
+        CDS segments of record i in transcript order are seg_*[seg_off[i]:seg_off[i+1]], none for a record without an ORF)."""
+        code = gencode.check(genetic_code)
+        starts = gencode.start64(start_codons, code)      # ValueError before any device work
+        if strand not in ("sense", "both"):
+            raise ValueError("strand %r is not 'sense' or 'both'" % (strand,))
+        if isinstance(min_aa, bool) or int(min_aa) != min_aa or int(min_aa) < 0:
+            raise ValueError("min_aa %r is not a count of residues" % (min_aa,))
+        gs, tbl = _feature_table(self, feature, "nucleotide")
+        if tbl is None or tbl.n_rec == 0:
+            return _empty_prediction()
+        flags = dict(min_aa=int(min_aa), start_codons=starts, partial5=bool(partial5), partial3=bool(partial3))
+        recs, segs = _predict_table(gs, tbl, code, **flags)
+        contig, seg_strand = tbl.seg_contig, tbl.seg_strand
+        anti = np.zeros(tbl.n_rec, dtype=np.int8)
+        if strand == "both":
+            at = antisense_table(tbl)
+            recs2, segs2 = _predict_table(gs, at, code, **flags)
+            anti = (recs2["n_aa"] > recs["n_aa"]).astype(np.int8)
+            rep = np.repeat(anti, np.diff(tbl.rec_seg_off)).astype(bool)
+            recs = np.where(anti.astype(bool), recs2, recs)
+            segs = np.where(rep, segs2, segs)
+            contig = np.where(rep, at.seg_contig, tbl.seg_contig)
+            seg_strand = np.where(rep, at.seg_strand, tbl.seg_strand)
+        keep = np.flatnonzero(tbl.rec_pre_len > 0)        # FASTA records; the blank entries of empty tops have no header
+        keep_seg = np.repeat(tbl.rec_pre_len > 0, np.diff(tbl.rec_seg_off)) & (segs["lo"] >= 0)
+        seg_off = np.concatenate(([0], np.cumsum(recs["n_cds_seg"][keep]))).astype(np.int64)
+        return CdsPrediction(_record_names(tbl, keep), recs[keep], anti[keep], contig[keep_seg].astype(np.int32),
+                             segs["lo"][keep_seg], segs["hi"][keep_seg], seg_strand[keep_seg].astype(np.int8),
+                             segs["phase"][keep_seg], seg_off)
+
 
 CdsCheck = collections.namedtuple("CdsCheck", "names records codon_counts junctions seg_off")
+CdsPrediction = collections.namedtuple("CdsPrediction", "names records antisense seg_contig seg_lo seg_hi seg_strand seg_phase "
+                                                        "seg_off")
+
+
+def _empty_prediction():
+    z = np.zeros(0, np.int64)
+    return CdsPrediction([], np.zeros(0, dtype=engine.PRED_DTYPE), np.zeros(0, np.int8), np.zeros(0, np.int32), z, z,
+                         np.zeros(0, np.int8), np.zeros(0, np.int8), np.zeros(1, np.int64))
+
+
+def _feature_table(annotation_set, feature, seq_type):
+    """(genome sequence, RecordTable) of what annotation_set.get_fasta(feature, seq_type) prints: the native model's table
+    when the set still holds one, else the Flattener's; the table is None without records."""
+    model = _PENDING.get(annotation_set) if _PENDING else None
+    flat = _native_table(annotation_set, model, feature) if model is not None else None
+    if flat is not None:
+        return flat[0], flat[1]
+    table = getattr(annotation_set, feature)
+    from .flatten import Flattener
+    fl = Flattener(annotation_set)
+    for key in table:
+        obj = table[key]
+        if not hasattr(obj, "get_fasta"):
+            raise AttributeError("%s instance has no attribute 'get_fasta'" % obj.__class__.__name__)
+        fl.add_top(obj, seq_type=seq_type, longest=False, genomic=False, name_from='ID')
+    return fl.gs, fl.records(seq_type)[0]
+
+
+def _record_names(tbl, rows):
+    """FASTA headers without '>' of the records `rows` of a framed table."""
+    lit = tbl.lit.tobytes()
+    return [lit[o + 1:o + n - 1].decode("latin-1") for o, n in zip(tbl.rec_lit_off[rows].tolist(), tbl.rec_pre_len[rows].tolist())]
+
+
+def antisense_table(tbl):
+    """The table whose record r is the reverse complement of record r of tbl: its segments in reverse order, strands flipped
+    (literals and phases kept)."""
+    cnt = np.diff(tbl.rec_seg_off)
+    rep = np.repeat(np.arange(tbl.n_rec), cnt)
+    idx = tbl.rec_seg_off[rep + 1] - 1 - (np.arange(tbl.n_seg) - tbl.rec_seg_off[rep])
+    return engine.RecordTable(tbl.rec_seg_off, tbl.seg_contig[idx], tbl.seg_start[idx], tbl.seg_end[idx], tbl.seg_strand[idx] == 0,
+                              tbl.rec_lit_off, tbl.rec_pre_len, tbl.rec_suf_len, tbl.lit, tbl.rec_phase)
+
+
+def _predict_table(gs, tbl, code, min_aa, start_codons, partial5, partial3):
+    plan = engine.Plan(gs._engine().primary, tbl)
+    try:
+        if code != 1:
+            plan.set_codon_table(gencode.codon64(code))
+        plan.prepare_async(trimx=False, defer_records=True)     # the prediction needs the piece pass only
+        return plan.predict_cds(min_aa, start_codons, partial5, partial3)
+    finally:
+        plan.close()
 
 _ASET_CLASS_NAMES = frozenset(dir(AnnotationSet))
 

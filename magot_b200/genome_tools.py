@@ -11,8 +11,9 @@ get_seq_from_fasta :483, exclude_from_fasta :377, extract_upstream_downstream :4
 blast_csv2fasta :265, exonerate2fasta :274, mask_from_gff :394, convert_gff :527,
 dna2orfs :145 (the reference's version cannot run -- it calls str.translate with keyword
 arguments -- this one does what it intended, on the device).  New: call_orfs, start-to-stop
-ORF calling with genome coordinates (GFF3, protein or CDS nucleotide output), and check_cds, a gene-model check (start /
-stop codons, in-frame stops, frame, splice sites, codon usage).  The dispatcher (main :25-45)
+ORF calling with genome coordinates (GFF3, protein or CDS nucleotide output), check_cds, a gene-model check (start /
+stop codons, in-frame stops, frame, splice sites, codon usage), and predict_cds, the longest ORF of each exon-only transcript
+model as GFF3 CDS rows, protein or CDS text.  The dispatcher (main :25-45)
 keeps the grammar but looks the function up in a table instead of eval()-ing a string.
 """
 import sys
@@ -448,9 +449,107 @@ def check_cds(genome_sequence, gff, feature="gene", genetic_code="1", start_codo
     sys.stdout.write("\n".join(lines) + "\n")
 
 
+PREDICT_FORMATS = ("gff3", "protein", "cds")
+#: partial= -> (partial5, partial3) of AnnotationSet.predict_cds
+PREDICT_PARTIAL = {"none": (False, False), "5prime": (True, False), "3prime": (False, True), "both": (True, True)}
+PREDICT_STRANDS = ("sense", "both")
+
+
+def _predict_header(name, rec, antisense):
+    """FASTA header (without '>') of a predicted ORF: <tid>.p1 orf_type=<type> len=<n> <tid>:<lo+1>-<hi>(<+|->), where lo / hi
+    are the ORF's coordinates in the transcript ('-': in its reverse complement)."""
+    return "%s.p1 orf_type=%s len=%d %s:%d-%d(%s)" % (name, engine._lib.ORF_TYPES[int(rec["type"]) & 3], int(rec["n_aa"]), name,
+                                                      int(rec["lo"]) + 1, int(rec["hi"]), "-" if antisense else "+")
+
+
+def _predict_lines(pred, contig_names, out_format, seqs=None):
+    """Output lines of predict_cds for a genome.CdsPrediction.  contig_names[c] = seqid of contig index c; seqs[i] = the protein
+    or CDS text of the i-th record that has an ORF (not read for gff3).  gff3: the version line, then per record with an ORF (in
+    record order) its CDS segments in ascending start order; protein / cds: a header line and the text on one line."""
+    lines = ["##gff-version 3"] if out_format == "gff3" else []
+    k = 0
+    for i, name in enumerate(pred.names):
+        rec = pred.records[i]
+        if int(rec["n_aa"]) <= 0:
+            continue
+        if out_format == "gff3":
+            attrs = "ID=%s.cds;Parent=%s;orf_type=%s;length_aa=%d" % (name, name, engine._lib.ORF_TYPES[int(rec["type"]) & 3],
+                                                                       int(rec["n_aa"]))
+            s0, s1 = int(pred.seg_off[i]), int(pred.seg_off[i + 1])
+            for e in sorted(range(s0, s1), key=lambda e: (int(pred.seg_lo[e]), int(pred.seg_hi[e]))):
+                lines.append("\t".join((contig_names[int(pred.seg_contig[e])], "magot_b200", "CDS", str(int(pred.seg_lo[e]) + 1),
+                                        str(int(pred.seg_hi[e])), ".", "-" if pred.seg_strand[e] else "+",
+                                        str(int(pred.seg_phase[e])), attrs)))
+        else:
+            lines.append(">" + _predict_header(name, rec, pred.antisense[i]))
+            lines.append(seqs[k])
+        k += 1
+    return lines
+
+
+def _predict_texts(eng, pred, genetic_code, protein):
+    """The CDS text (K2) or its translation (K3, trimX off, the first residue 'M' when the ORF starts at a start codon, a
+    terminal '*' kept) of every record of `pred` that has an ORF, from one RecordTable of its CDS segments."""
+    has = np.flatnonzero(pred.records["n_aa"] > 0)
+    if has.size == 0:
+        return []
+    R = len(pred.names)
+    zero = np.zeros(R, dtype=np.int32)
+    tbl = engine.RecordTable(pred.seg_off, pred.seg_contig, pred.seg_lo + 1, pred.seg_hi, pred.seg_strand,
+                             np.zeros(R, dtype=np.int64), zero, zero, np.zeros(0, dtype=np.uint8))
+    text, (nuc_len, aa_len) = eng.run_table(tbl, protein=protein, trimx=False, want_lengths=True,
+                                            codon64=gencode.codon64(genetic_code) if protein and genetic_code != 1 else None)
+    lens = np.maximum(aa_len, 0) if protein else nuc_len
+    off = np.concatenate(([0], np.cumsum(lens)))
+    out = []
+    for i in has.tolist():
+        t = text[off[i]:off[i + 1]].decode("latin-1")
+        if protein and not int(pred.records["type"][i]) & 1:
+            t = "M" + t[1:]
+        out.append(t)
+    return out
+
+
+def predict_cds(genome_sequence, gff, min_orf="100", genetic_code="1", start_codons="ATG", partial="none", strand="sense",
+                out_format="gff3"):
+    """CDS prediction for exon-only transcript models (new; TransDecoder.LongOrfs / gffread style, one ORF per transcript): the
+    longest ORF of each spliced transcript in its three frames, at least `min_orf` residues, from a codon in start_codons
+    (comma-separated, default ATG) to a stop of NCBI table `genetic_code`, mapped back to genome CDS segments on the device.
+    The GFF is read with exons as the transcripts' base features and CDS rows ignored.  partial=5prime / 3prime / both also
+    accept ORFs open at a frame's 5' end / without a stop; strand=both also scores the antisense (the longer ORF wins, the
+    sense one on a tie).  out_format: gff3 (CDS rows ID=<tid>.cds;Parent=<tid>;orf_type=..;length_aa=.., segments in
+    ascending start order), protein ('>'<tid>.p1 header, the first residue M at a start codon, a terminal '*' kept) or cds
+    (the CDS nucleotides under the same header)."""
+    code = gencode.check(genetic_code)
+    if out_format not in PREDICT_FORMATS:
+        raise ValueError("out_format %r is not one of %s" % (out_format, ", ".join(PREDICT_FORMATS)))
+    if partial not in PREDICT_PARTIAL:
+        raise ValueError("partial %r is not one of %s" % (partial, ", ".join(PREDICT_PARTIAL)))
+    if strand not in PREDICT_STRANDS:
+        raise ValueError("strand %r is not one of %s" % (strand, ", ".join(PREDICT_STRANDS)))
+    try:
+        min_aa = int(min_orf)
+    except (TypeError, ValueError):
+        min_aa = -1
+    if min_aa < 0:
+        raise ValueError("min_orf %r is not a count of residues" % (min_orf,))
+    codons = start_codons.split(",") if isinstance(start_codons, str) else list(start_codons)
+    gencode.start64(codons, code)                            # ValueError before any device work
+    my_genome = genome.Genome(genome_sequence)
+    my_genome.read_gff(gff, base_features=["exon"], features_to_ignore=["CDS"])
+    p5, p3 = PREDICT_PARTIAL[partial]
+    pred = my_genome.annotations.predict_cds("gene", min_aa=min_aa, genetic_code=code, start_codons=codons, partial5=p5,
+                                             partial3=p3, strand=strand)
+    gs = my_genome.genome_sequence
+    names = {gs.contig_index(seq): seq for seq in gs}
+    seqs = None if out_format == "gff3" else _predict_texts(gs._engine(), pred, code, out_format == "protein")
+    lines = _predict_lines(pred, names, out_format, seqs)
+    sys.stdout.write("\n".join(lines) + "\n" if lines else "")
+
+
 FUNCTIONS = {f.__name__: f for f in (gff2fasta, cds2pep, coords2fasta, get_seq_from_fasta, exclude_from_fasta,
                                      extract_upstream_downstream, dna2orfs, blast_csv2fasta, exonerate2fasta, mask_from_gff,
-                                     convert_gff, call_orfs, check_cds)}
+                                     convert_gff, call_orfs, check_cds, predict_cds)}
 
 
 def help_func():
