@@ -358,6 +358,84 @@ int mg_plan_predict_cds(mg_plan *p, int64_t min_aa, const uint8_t *start64, int 
 int mg_plan_predict_cds_device(mg_plan *p, int64_t min_aa, const uint8_t *start64, int flags,
                                mg_cds_pred *rec_out, mg_cds_seg *seg_out, void *stream);
 
+/* ---- coding consequences of variant alleles on a prepared plan (bcftools csq / SnpEff / VEP style, no HGVS).
+ * Inputs: allele i is on genome contig contig[i] at 0-based pos[i] (REF's first base); REF = bytes[allele_off[2i],
+ * allele_off[2i+1]), ALT = bytes[allele_off[2i+1], allele_off[2i+2]).  The alleles must be sorted by (contig, pos) (checked on
+ * the host: MG_EINVAL), and allele_off must be non-decreasing inside [0, n_bytes].  The count uploads the arrays: the caller's
+ * buffers are free again when it returns.
+ * Status (status_host[i], written for every allele; an allele with a non-zero status gets no rows), the first that applies:
+ *   1 contig not in the genome, pos < 0 or REF past the contig end;  2 REF differs from the genome (case ignored; a genome byte
+ *   held in the exception list never matches);  3 REF or ALT empty, or REF equals ALT (case ignored).
+ * Normalisation: strip the longest common suffix of REF and ALT (case ignored), then the longest common prefix of what remains,
+ * adding its length to pos: REF' is the forward span [s, t), A' the remaining ALT bytes.  A substitution has len(REF') ==
+ * len(A'); an insertion has an empty REF' and sits at point s (between forward bases s-1 and s); anything else is a deletion
+ * or a complex allele.
+ * Terms: payload S, skip, n_codons and codon i as in mg_plan_check.  Caller segment e (the table given to mg_plan_create; the
+ * chunks of segments of 2^31 bases or more are never visible), clamped as the plan clamps it to [cl_e, ch_e), covers payload
+ * [o_e, o_e + ch_e - cl_e); forward base x of it is payload o_e + x - cl_e on '+', o_e + ch_e - 1 - x on '-'.  Every junction
+ * of class 1..4 after segment e (mg_plan_check's definition; the class depends on the geometry alone) has a donor site D and an
+ * acceptor site A, 2-base forward intervals: '+' D = [ch_e, ch_e+2), A = [cl_{e+1}-2, cl_{e+1}); '-' D = [cl_e-2, cl_e),
+ * A = [ch_{e+1}, ch_{e+1}+2).  Junction class 0 has no sites.
+ * Touch (same contig only): a non-empty span touches [u, w) when they intersect.  An insertion at s touches a segment when
+ * cl < s < ch, and a site [u, u+2) when s == u+1 or s is the point the site shares with its own segment (ch_e for '+' D,
+ * cl_{e+1} for '+' A, cl_e for '-' D, ch_{e+1} for '-' A).  An insertion at a record end touches nothing.
+ * Rows: one per (allele, record) for which the allele touches a segment or a site of the record.  seg = the first caller
+ * segment e of the record in emission order that the allele touches directly or through junction e's sites (the owner).
+ * Rows are ordered by record, then allele index.
+ * nuc_lo, nuc_hi: the part of [s, t) inside the owner segment, as a payload range; for an insertion inside it [x, x), where
+ * the bases go before payload x (x = o_e + s - cl_e on '+', o_e + ch_e - s on '-'); -1, -1 when the allele touches the owner
+ * only through a site.  codon: for a substitution the first codon i < n_codons overlapping [nuc_lo, nuc_hi), for the others
+ * the codon holding nuc_lo when skip <= nuc_lo < skip + 3 n_codons; -1 otherwise.
+ * Class: the smallest code that applies.  1 SPLICE_ACCEPTOR: touches an acceptor site of the record;  2 SPLICE_DONOR: a donor
+ * site;  3 BOUNDARY: [s, t) is not inside one segment of the record (an insertion: no segment with cl < s < ch);
+ * 4 FRAMESHIFT: len(A') - len(REF') of a non-substitution is not a multiple of 3;  5 INFRAME_INSERTION / 6 INFRAME_DELETION:
+ * it gains / loses a multiple of 3 bases (4..6 by length alone, wherever the indel sits in the payload).  Codes 7..13 are for
+ * substitutions; their affected codons are the codons i < n_codons overlapping [nuc_lo, nuc_hi), and each alternative codon
+ * is the reference codon (read through the plan's pieces, so a codon across a junction takes bases from the neighbouring
+ * segment) with payload nuc_lo + k replaced by A'[k] on '+', by the complement of A'[len-1-k] on '-'.  A codon with a base
+ * outside A/C/G/T (either case) is ambiguous: never a start or a stop.  7 START_LOST: codon 0 is affected, its reference is a
+ * start (start64) and its alternative is not;  8 STOP_GAINED: an affected codon goes from an unambiguous non-stop to a stop;
+ * 9 STOP_LOST: codon n_codons-1 is affected, its reference is a stop and its alternative is not;  10 AMBIGUOUS: an affected
+ * codon is ambiguous in its reference or alternative;  11 MISSENSE: an affected codon's residue changes under the plan's code;
+ * 12 SYNONYMOUS: otherwise, with at least one affected codon;  13 NONCODING_PAYLOAD: a substitution with no affected codon.
+ * n_aff, ref_codon, alt_codon, ref_aa, alt_aa are filled for classes 7..12 only (else 0, 0xFF, 0xFF, empty): the number of
+ * affected codons (capped at 127), the first one's codon indices (0xFF when ambiguous) and the residues of the first 8
+ * ('X' for an ambiguous codon), NUL-padded.
+ * The count holds its state on the plan: mg_plan_variant_emit* emits the plan's last count and fails with MG_ESTATE without
+ * one, or after a re-prepare of the plan or a pack, finalize or mask of its genome.  The emit classifies under the plan's code
+ * at emit time and the start set given to the count.  Neither call can be captured in a CUDA graph (the count returns a row
+ * count to the host).  flags: 0 or MG_PROT_USE_PHASE; start64 as in mg_orfcall_count (NULL = ATG).  mg_plan_variant_emit
+ * copies the rows to host memory in stream order (sync before reading).                                                    */
+#define MG_VEF_SPLICE_ACCEPTOR 1
+#define MG_VEF_SPLICE_DONOR 2
+#define MG_VEF_BOUNDARY 3
+#define MG_VEF_FRAMESHIFT 4
+#define MG_VEF_INFRAME_INSERTION 5
+#define MG_VEF_INFRAME_DELETION 6
+#define MG_VEF_START_LOST 7
+#define MG_VEF_STOP_GAINED 8
+#define MG_VEF_STOP_LOST 9
+#define MG_VEF_AMBIGUOUS 10
+#define MG_VEF_MISSENSE 11
+#define MG_VEF_SYNONYMOUS 12
+#define MG_VEF_NONCODING_PAYLOAD 13
+typedef struct {
+    int64_t var;                  /* allele index (input order)                                              */
+    int64_t rec;                  /* plan record                                                             */
+    int64_t seg;                  /* caller segment that owns the hit                                        */
+    int64_t nuc_lo, nuc_hi;       /* payload range REF' replaces; [x, x) for an insertion; -1, -1 if none    */
+    int32_t codon;                /* first affected codon index, -1 = none                                   */
+    int8_t  cls;                  /* MG_VEF_*                                                                */
+    int8_t  n_aff;                /* affected codons of a substitution, capped at 127                        */
+    uint8_t ref_codon, alt_codon; /* first affected codon, 16*b0 + 4*b1 + b2; 0xFF = none or ambiguous      */
+    char    ref_aa[8], alt_aa[8]; /* residues of the first 8 affected codons, NUL-padded                     */
+} mg_var_effect;                  /* 64 bytes */
+int mg_plan_variant_count(mg_plan *p, int64_t n_var, const int32_t *contig, const int64_t *pos, const int64_t *allele_off,
+                          const uint8_t *bytes, int64_t n_bytes, int flags, const uint8_t *start64, int8_t *status_host,
+                          int64_t *n_rows, void *stream);
+int mg_plan_variant_emit(mg_plan *p, mg_var_effect *rows_host, void *stream);
+int mg_plan_variant_emit_device(mg_plan *p, mg_var_effect *rows_dev, void *stream);
+
 /* ---- host side: native GFF3 / GTF reader + flattener (no GPU work; csrc/mg_gff.cu) ------------------------------------------
  * mg_gff_parse replaces read_gff (genome.py:242-415: line filter, version detection, attribute parsing, ID naming, de-dup,
  * implicit parents, child lists) on interned integer ids; `opts` is the option blob magot_b200/gffnative.py packs (format

@@ -56,6 +56,18 @@ class MgCdsSeg(ctypes.Structure):
     _fields_ = [("lo", ctypes.c_int64), ("hi", ctypes.c_int64), ("phase", ctypes.c_int8), ("pad", ctypes.c_int8 * 7)]
 
 
+class MgVarEffect(ctypes.Structure):
+    """mg_var_effect (include/magot_b200.h)."""
+    _fields_ = [("var", ctypes.c_int64), ("rec", ctypes.c_int64), ("seg", ctypes.c_int64), ("nuc_lo", ctypes.c_int64),
+                ("nuc_hi", ctypes.c_int64), ("codon", ctypes.c_int32), ("cls", ctypes.c_int8), ("n_aff", ctypes.c_int8),
+                ("ref_codon", ctypes.c_uint8), ("alt_codon", ctypes.c_uint8), ("ref_aa", ctypes.c_char * 8),
+                ("alt_aa", ctypes.c_char * 8)]
+
+
+#: MG_VEF_* consequence classes of mg_var_effect.cls: VEF_CLASSES[cls - 1] is the name of class cls
+VEF_CLASSES = ("SPLICE_ACCEPTOR", "SPLICE_DONOR", "BOUNDARY", "FRAMESHIFT", "INFRAME_INSERTION", "INFRAME_DELETION",
+               "START_LOST", "STOP_GAINED", "STOP_LOST", "AMBIGUOUS", "MISSENSE", "SYNONYMOUS", "NONCODING_PAYLOAD")
+
 #: orf_type text of mg_cds_pred.type (bit 0: 5' partial, bit 1: 3' partial)
 ORF_TYPES = ("complete", "5prime_partial", "3prime_partial", "internal")
 
@@ -124,6 +136,9 @@ SIGNATURES = {
     "mg_plan_check_device": (_i32, [_vp, _i32, _vp, _vp, _vp, _vp, _vp]),
     "mg_plan_predict_cds": (_i32, [_vp, _i64, _vp, _i32, _vp, _vp, _vp]),
     "mg_plan_predict_cds_device": (_i32, [_vp, _i64, _vp, _i32, _vp, _vp, _vp]),
+    "mg_plan_variant_count": (_i32, [_vp, _i64, _vp, _vp, _vp, _vp, _i64, _i32, _vp, _vp, _pi64, _vp]),
+    "mg_plan_variant_emit": (_i32, [_vp, _vp, _vp]),
+    "mg_plan_variant_emit_device": (_i32, [_vp, _vp, _vp]),
     "mg_stream_sync": (_i32, [_i32, _vp]),
     "mg_copy_d2h_async": (_i32, [_i32, _vp, _vp, _i64, _vp]),
     "mg_tune": (_i32, [ctypes.c_char_p, _i32]),

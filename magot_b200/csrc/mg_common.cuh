@@ -63,6 +63,7 @@ extern std::atomic<int64_t> g_mg_launches;        // kernels launched by this li
 
 // ---- handles -------------------------------------------------------------------------------------
 struct mg_sixframe_state;
+struct mg_var_state;
 
 struct mg_genome {
     int device = 0;
@@ -164,6 +165,8 @@ struct mg_plan {
     int8_t *d_chk_junction = nullptr;
     mg_cds_pred *d_pred = nullptr;            // device outputs of the host-buffer mg_plan_predict_cds
     mg_cds_seg *d_pred_seg = nullptr;
+    uint64_t prepares = 0;                    // mg_plan_prepare* calls so far: a variant count belongs to one prepare
+    mg_var_state *var = nullptr;              // state of the last mg_plan_variant_count (mg_variant.cu)
     std::vector<void *> owned;                // everything to free
 };
 
@@ -186,6 +189,7 @@ struct mg_plan {
 void build_aa4096(uint8_t *t, const uint8_t *codon64);   // nibble-triplet -> residue table from a codon64 table (NULL = standard code)
 int mg_plan_check_prepared(const mg_plan *p);         // MG_ESTATE unless p was prepared and its genome has not changed since
 int mg_refuse_growth_in_capture(cudaStream_t st, const char *what);   // MG_ESTATE when st is being captured (a buffer would have to grow)
+void mg_var_free(mg_plan *p);                         // releases p->var (mg_plan_destroy)
 int mg_start_mask(const mg_plan *p, const uint8_t *start64, uint64_t *mask);   // start64 flags (NULL = ATG) as a bit set, checked against the plan's stops
 int mg_scan_i32(const int32_t *d_in, int64_t *d_out, int64_t n, int64_t *d_tmp, int64_t tmp_cap, cudaStream_t st);
 int64_t mg_scan_tmp_elems(int64_t n);

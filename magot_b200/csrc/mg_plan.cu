@@ -686,6 +686,7 @@ extern "C" int mg_plan_create(mg_genome *g, int64_t n_rec, const int64_t *rec_se
 extern "C" int mg_plan_destroy(mg_plan *p) {
     if (!p) return MG_OK;
     cudaSetDevice(p->device);
+    mg_var_free(p);
     for (void *d : p->owned) cudaFreeAsync(d, p->last_stream);
     if (p->d_out) cudaFreeAsync(p->d_out, p->last_stream);
     delete p;
@@ -867,6 +868,7 @@ extern "C" int mg_plan_prepare(mg_plan *p, int prot_flags, int64_t *nuc_total, i
     MG_CUDA(cudaSetDevice(p->device));
     cudaStream_t st = (cudaStream_t)stream;
     p->prepared = false;
+    p->prepares++;
     int rc = plan_launch_scans(p, prot_flags & ~MG_PROT_DEFER, st);
     if (rc) return rc;
     int64_t totals[2];
@@ -893,6 +895,7 @@ extern "C" int mg_plan_prepare_async(mg_plan *p, int prot_flags, int64_t nuc_cap
         if (rc0) return rc0;
     }
     p->prepared = false;
+    p->prepares++;
     int rc = plan_launch_scans(p, prot_flags, (cudaStream_t)stream, true, nuc_capacity, prot_capacity);
     if (rc) return rc;
     p->nuc_total = nuc_capacity;                     // until mg_plan_totals: what the caller's buffers can take

@@ -38,6 +38,12 @@ assert PRED_DTYPE.itemsize == ctypes.sizeof(_lib.MgCdsPred)
 CDSSEG_DTYPE = np.dtype([("lo", np.int64), ("hi", np.int64), ("phase", np.int8), ("pad", np.int8, (7,))])
 assert CDSSEG_DTYPE.itemsize == ctypes.sizeof(_lib.MgCdsSeg)
 
+#: mg_var_effect (include/magot_b200.h): one row of Plan.variant_effects
+VEF_DTYPE = np.dtype([("var", np.int64), ("rec", np.int64), ("seg", np.int64), ("nuc_lo", np.int64), ("nuc_hi", np.int64),
+                      ("codon", np.int32), ("cls", np.int8), ("n_aff", np.int8), ("ref_codon", np.uint8),
+                      ("alt_codon", np.uint8), ("ref_aa", "S8"), ("alt_aa", "S8")])
+assert VEF_DTYPE.itemsize == ctypes.sizeof(_lib.MgVarEffect)
+
 
 def _ptr(a):
     return ctypes.c_void_p(a.ctypes.data) if a is not None else None
@@ -247,6 +253,34 @@ class Plan(object):
         check(lib.mg_plan_predict_cds(self.handle, int(min_aa), start_codons, flags, _ptr(recs), _ptr(segs), self.stream))
         check(lib.mg_stream_sync(self.genome.device, self.stream))
         return recs, segs
+
+    def variant_effects(self, contig, pos, allele_off, allele_bytes, start_codons=None, use_phase=False):
+        """Coding consequences of sorted alleles on every record (mg_plan_variant_count + mg_plan_variant_emit) under the plan's
+        genetic code.  contig (int32), pos (int64, 0-based) per allele, sorted by (contig, pos); REF of allele i is
+        allele_bytes[allele_off[2i]:allele_off[2i+1]], ALT the bytes up to allele_off[2i+2].  start_codons: 64 flags as
+        gencode.start64 gives them, None = ATG.  Returns (int8 status per allele, VEF_DTYPE rows ordered by record, then
+        allele).  Needs prepare() or prepare_async() first."""
+        contig = np.ascontiguousarray(contig, dtype=np.int32)
+        pos = np.ascontiguousarray(pos, dtype=np.int64)
+        allele_off = np.ascontiguousarray(allele_off, dtype=np.int64)
+        buf = np.frombuffer(bytes(allele_bytes), dtype=np.uint8) if not isinstance(allele_bytes, np.ndarray) else \
+            np.ascontiguousarray(allele_bytes, dtype=np.uint8)
+        n = contig.size
+        if pos.size != n or allele_off.size != 2 * n + 1:
+            raise ValueError("contig and pos need one entry per allele, allele_off 2 * n + 1")
+        if start_codons is not None:
+            start_codons = bytes(start_codons)
+            if len(start_codons) != 64:
+                raise ValueError("start_codons must hold 64 flags")
+        status = np.zeros(n, dtype=np.int8)
+        n_rows = ctypes.c_int64(0)
+        check(lib.mg_plan_variant_count(self.handle, n, _ptr(contig), _ptr(pos), _ptr(allele_off), _ptr(buf), buf.size,
+                                        _lib.MG_PROT_USE_PHASE if use_phase else 0, start_codons, _ptr(status),
+                                        ctypes.byref(n_rows), self.stream))
+        rows = np.zeros(n_rows.value, dtype=VEF_DTYPE)
+        check(lib.mg_plan_variant_emit(self.handle, _ptr(rows), self.stream))
+        check(lib.mg_stream_sync(self.genome.device, self.stream))
+        return status, rows
 
     def emit_host(self, protein=False, out=None):
         total = self.prot_total if protein else self.nuc_total

@@ -798,8 +798,55 @@ class AnnotationSet(object):
                              segs["lo"][keep_seg], segs["hi"][keep_seg], seg_strand[keep_seg].astype(np.int8),
                              segs["phase"][keep_seg], seg_off)
 
+    def variant_effects(self, feature, variants, genetic_code=1, start_codons=("ATG",), use_phase=False):
+        """Coding consequences (mg_plan_variant_count / _emit) of VCF alleles on exactly the records check_cds(feature) checks:
+        which records each SNV, MNV or indel touches, and whether it hits a splice site, crosses a segment boundary, shifts the
+        frame, or is synonymous, missense, a stop gain or loss, a start loss, ambiguous or outside the codons.  variants: a
+        variants.VcfAlleles, or a VCF path or bytes for variants.read_vcf.  A CHROM the genome does not hold gets status 1.
+        Returns VariantEffects(names, rows, status, variants, strand): rows (engine.VEF_DTYPE) in VCF line order, then ALT
+        order, then record order, with `var` the allele's index in `variants` and `rec` an index into `names`; status (int8
+        per allele, 0 = ok; see include/magot_b200.h); strand[k] = 0 '+', 1 '-' of row k's owning segment."""
+        from . import variants as _variants
+        code = gencode.check(genetic_code)
+        starts = gencode.start64(start_codons, code)      # ValueError before any device work
+        if not isinstance(variants, _variants.VcfAlleles):
+            variants = _variants.read_vcf(variants)
+        gs, tbl = _feature_table(self, feature, "protein")
+        n = len(variants)
+        if tbl is None or tbl.n_rec == 0:
+            return VariantEffects([], np.zeros(0, dtype=engine.VEF_DTYPE), np.zeros(n, np.int8), variants, np.zeros(0, np.int8))
+        contig = np.empty(n, dtype=np.int32)
+        for i, name in enumerate(variants.chrom):
+            try:
+                contig[i] = gs.contig_index(name)
+            except KeyError:
+                contig[i] = -1
+        pos0 = variants.pos - 1
+        order = np.lexsort((pos0, contig))                # stable: equal keys keep their VCF order
+        parts = [x for i in order.tolist() for x in (variants.ref[i], variants.alt[i])]
+        off = np.concatenate(([0], np.cumsum([len(x) for x in parts]))).astype(np.int64)
+        plan = engine.Plan(gs._engine().primary, tbl)
+        try:
+            if code != 1:
+                plan.set_codon_table(gencode.codon64(code))
+            plan.prepare_async(trimx=False, defer_records=True)     # the call needs the piece pass only
+            st, rows = plan.variant_effects(contig[order], pos0[order], off, b"".join(parts), starts, use_phase)
+        finally:
+            plan.close()
+        status = np.empty(n, dtype=np.int8)
+        status[order] = st
+        keep = np.flatnonzero(tbl.rec_pre_len > 0)        # FASTA records; the blank entries of empty tops have no header
+        rec_of = np.full(tbl.n_rec, -1, dtype=np.int64)
+        rec_of[keep] = np.arange(keep.size)
+        rows = rows[rec_of[rows["rec"]] >= 0]
+        rows["var"] = order[rows["var"]]
+        rows["rec"] = rec_of[rows["rec"]]
+        rows = rows[np.lexsort((rows["rec"], rows["var"]))]
+        return VariantEffects(_record_names(tbl, keep), rows, status, variants, tbl.seg_strand[rows["seg"]].astype(np.int8))
+
 
 CdsCheck = collections.namedtuple("CdsCheck", "names records codon_counts junctions seg_off")
+VariantEffects = collections.namedtuple("VariantEffects", "names rows status variants strand")
 CdsPrediction = collections.namedtuple("CdsPrediction", "names records antisense seg_contig seg_lo seg_hi seg_strand seg_phase "
                                                         "seg_off")
 

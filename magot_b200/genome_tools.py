@@ -547,9 +547,94 @@ def predict_cds(genome_sequence, gff, min_orf="100", genetic_code="1", start_cod
     sys.stdout.write("\n".join(lines) + "\n" if lines else "")
 
 
+VARIANT_FORMATS = ("tsv", "vcf")
+VARIANT_TSV_HEADER = "\t".join(("CHROM", "POS", "ID", "REF", "ALT", "record", "strand", "consequence", "nuc_pos", "codon",
+                                "codons", "residues"))
+VARIANT_INFO_HEADER = ('##INFO=<ID=MGCSQ,Number=.,Type=String,Description="Coding consequence per allele and record: '
+                       'class|allele|record|strand|ref_aa/alt_aa|1-based payload position">')
+
+
+def _codon_text(c):
+    return "." if c == 0xFF else "ACGT"[c >> 4] + "ACGT"[(c >> 2) & 3] + "ACGT"[c & 3]
+
+
+def _variant_fields(res, k):
+    """(consequence, strand, 1-based payload position, 1-based codon, codons, residues) of row k of a genome.VariantEffects;
+    '.' for an absent value."""
+    row = res.rows[k]
+    cls = engine._lib.VEF_CLASSES[int(row["cls"]) - 1]
+    nuc = "." if int(row["nuc_lo"]) < 0 else str(int(row["nuc_lo"]) + 1)
+    codon = "." if int(row["codon"]) < 0 else str(int(row["codon"]) + 1)
+    n_aff = int(row["n_aff"])
+    codons = "." if n_aff == 0 else "%s/%s" % (_codon_text(int(row["ref_codon"])), _codon_text(int(row["alt_codon"])))
+    aa = "." if n_aff == 0 else "%s/%s" % (bytes(row["ref_aa"]).decode("latin-1"), bytes(row["alt_aa"]).decode("latin-1"))
+    return cls, "-" if res.strand[k] else "+", nuc, codon, codons, aa
+
+
+def variant_effects(genome_sequence, gff, vcf, feature="gene", genetic_code="1", start_codons="ATG", use_phase="False",
+                    out_format="tsv"):
+    """Coding consequences of the alleles of a VCF (plain or gzip) on every record `check_cds` checks (new; bcftools csq /
+    SnpEff style, on the device): splice acceptor or donor site, segment boundary, frameshift, in-frame insertion or deletion,
+    start lost, stop gained, stop lost, ambiguous, missense, synonymous, or a substitution outside the codons.  Multi-allelic
+    lines give one allele per ALT; symbolic, '*', '.' and breakend ALTs are skipped.  out_format=tsv prints a header line and
+    one line per (allele, record): CHROM, POS, ID, REF, ALT, record, strand of the owning segment, consequence, 1-based
+    payload position, 1-based codon, codons (GCT/GTT) and residues (A/V) of a substitution's first affected codon(s), '.' when
+    absent.  out_format=vcf prints the VCF unchanged except for an ##INFO=<ID=MGCSQ> header line and, on lines with rows,
+    MGCSQ=class|allele|record|strand|aa_change|nuc_pos entries added to INFO.  The status counts (0 ok, 1 unknown contig or
+    out of range, 2 REF mismatch, 3 empty or REF == ALT) and the skipped ALTs go to stderr."""
+    code = gencode.check(genetic_code)
+    if out_format not in VARIANT_FORMATS:
+        raise ValueError("out_format %r is not one of %s" % (out_format, ", ".join(VARIANT_FORMATS)))
+    codons = start_codons.split(",") if isinstance(start_codons, str) else list(start_codons)
+    gencode.start64(codons, code)                            # ValueError before any device work
+    phase = _truth(use_phase)
+    from . import variants as _variants
+    calls = _variants.read_vcf(vcf)
+    my_genome = genome.Genome(genome_sequence)
+    my_genome.read_gff(gff)
+    res = my_genome.annotations.variant_effects(feature, calls, genetic_code=code, start_codons=codons, use_phase=phase)
+    out = []
+    if out_format == "tsv":
+        out.append(VARIANT_TSV_HEADER)
+        for k in range(res.rows.size):
+            i = int(res.rows["var"][k])
+            f = _variant_fields(res, k)
+            out.append("\t".join((calls.chrom[i], str(int(calls.pos[i])), calls.ids[i], calls.ref[i].decode("latin-1"),
+                                  calls.alt[i].decode("latin-1"), res.names[int(res.rows["rec"][k])], f[1], f[0], f[2], f[3],
+                                  f[4], f[5])))
+    else:
+        per_line = {}
+        for k in range(res.rows.size):
+            i = int(res.rows["var"][k])
+            cls, strand, nuc, _, _, aa = _variant_fields(res, k)
+            per_line.setdefault(int(calls.line[i]), []).append(
+                "|".join((cls, calls.alt[i].decode("latin-1"), res.names[int(res.rows["rec"][k])], strand,
+                          "" if aa == "." else aa, "" if nuc == "." else nuc)))
+        header_done = False
+        for n, text in enumerate(calls.lines):
+            line = text.decode("latin-1")
+            if line.startswith("#CHROM") and not header_done:
+                out.append(VARIANT_INFO_HEADER)
+                header_done = True
+            if n in per_line:
+                cols = line.split("\t")
+                while len(cols) < 8:
+                    cols.append(".")
+                entry = "MGCSQ=" + ",".join(per_line[n])
+                cols[7] = entry if cols[7] in ("", ".") else cols[7] + ";" + entry
+                line = "\t".join(cols)
+            out.append(line)
+    sys.stdout.write("\n".join(out) + "\n")
+    counts = np.bincount(res.status.astype(np.int64), minlength=4) if res.status.size else np.zeros(4, np.int64)
+    sys.stderr.write("variant_effects: %d alleles, status ok %d, unknown contig or out of range %d, REF mismatch %d, "
+                     "empty or unchanged %d; skipped ALTs: %s; %d rows\n"
+                     % (len(calls), counts[0], counts[1], counts[2], counts[3],
+                        ", ".join("%s %d" % kv for kv in calls.skipped.items()), res.rows.size))
+
+
 FUNCTIONS = {f.__name__: f for f in (gff2fasta, cds2pep, coords2fasta, get_seq_from_fasta, exclude_from_fasta,
                                      extract_upstream_downstream, dna2orfs, blast_csv2fasta, exonerate2fasta, mask_from_gff,
-                                     convert_gff, call_orfs, check_cds, predict_cds)}
+                                     convert_gff, call_orfs, check_cds, predict_cds, variant_effects)}
 
 
 def help_func():
